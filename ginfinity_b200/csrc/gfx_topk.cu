@@ -12,12 +12,24 @@
 //           queries of the item stay in shared memory; accumulators are
 //           double-buffered in TMEM (2 x 2 x 128 columns).
 //   finish  exact re-scoring of the surviving candidates (sequential fp32 FMA
-//           in dimension order: reproducible and restatable on the CPU) and
-//           selection of the k best by (score desc, index asc).
+//           in dimension order: reproducible and restatable on the CPU),
+//           selection of the k best by (score desc, index asc), and a
+//           certificate per query (below).
+//   fallback  for the queries whose certificate fails: an exact scan of the
+//           whole database (the same FMA chain for every row) and the same
+//           selection.  Launched unconditionally; its grid reads the number
+//           of flagged queries on the device.
 //   merge   k-way merge of per-rank lists after the all-gather.
 //
 // Tensor-core scores only choose the candidates (kc = k + >=4 spares per
-// segment); the returned scores and order come from the exact pass.
+// segment); the returned scores and order come from the exact pass.  The scan
+// drops a row only when its tensor-core score is <= max(seed', last entry of a
+// full list), so the largest such bound B over the segments bounds every
+// dropped row.  A query is certified when B + eps < S_k, its k-th exact score
+// in the scan's frame (+|q|^2 for L2): no dropped row can then reach the top k.
+// Otherwise (near-ties the tensor cores cannot order, e.g. many near-duplicate
+// rows, or a row of very large norm inflating eps) the query is rescored
+// exactly against every row.  The result is exact for every input.
 #include <limits.h>
 #include <math.h>
 
@@ -62,11 +74,17 @@ struct alignas(64) Maps {
   CUtensorMap q, db;
 };
 
+// Workspace header: the int64 count of queries that took the exact fallback in
+// the last call (read by EmbeddingIndex.last_fallbacks), then the largest
+// squared row norm (float bits; atomicMax on the bits orders non-negative
+// floats).  Zeroed by every call.
+constexpr size_t kOffFallbacks = 0, kOffMaxSqNorm = 8, kHeaderBytes = 256;
+
 struct Plan {
   int64_t tiles_q, tiles_db, segs, tiles_per_seg, qp;
   int kc;
   int64_t sample_tiles;       // 0 = no seeding pre-pass
-  size_t off_scores, off_index, off_d2, off_seed_scores, off_seed_index, total;
+  size_t off_flagged, off_scores, off_index, off_d2, off_seed_scores, off_seed_index, total;
 };
 
 static Plan make_plan(int64_t Q, int64_t D, int k) {
@@ -85,8 +103,9 @@ static Plan make_plan(int64_t Q, int64_t D, int k) {
   p.kc = kc > kMaxCand ? kMaxCand : kc;
   auto up = [](size_t v) { return (v + 255) & ~size_t(255); };
   const size_t cand = size_t(p.segs) * p.qp * p.kc;
-  p.off_scores = 0;
-  p.off_index = up(cand * 4);
+  p.off_flagged = kHeaderBytes;                              // [Q] int32 queries to rescan
+  p.off_scores = p.off_flagged + up(size_t(Q) * 4);
+  p.off_index = p.off_scores + up(cand * 4);
   p.off_d2 = p.off_index + up(cand * 4);
   p.total = p.off_d2 + up(size_t(p.tiles_db) * kDbTile * 4);
   // Seeding pays when the sample is a small part of the scan.
@@ -98,7 +117,7 @@ static Plan make_plan(int64_t Q, int64_t D, int k) {
 }
 
 struct Args {
-  const float *d2;            // [tiles_db * 128] squared row norms, +inf past the end (L2 only)
+  const float *d2;            // [tiles_db * 128] squared row norms, +inf past the end (read by the L2 scan)
   float *part_scores;         // [segs][qp][kc]
   int32_t *part_index;
   int64_t tiles_q, tiles_db, segs, tiles_per_seg, qp, num_rows;
@@ -126,6 +145,10 @@ __device__ __noinline__ float list_insert(float *ls, int32_t *li, int kc, float 
   li[j * kQTile] = idx;
   return ls[(kc - 1) * kQTile];
 }
+
+// Threshold a scan starts from, given the kc-th score of the seeding sample:
+// strictly below it, so rows that tie with the seed still enter.
+__device__ __forceinline__ float seed_threshold(float s) { return s - (fabsf(s) * 2.4e-7f + 1e-30f); }
 
 __device__ __forceinline__ float max3(float a, float b, float c) {
   float r;
@@ -275,10 +298,8 @@ topk_scan_kernel(const __grid_constant__ Maps maps, const Args p) {
         li[j * kQTile] = INT_MAX;
       }
       float seed = ninf;
-      if (p.seed) {                                 // kc-th best of the sample (lists are sorted)
-        seed = p.seed[(size_t(qt) * kQTile + row) * kc + kc - 1];
-        seed -= fabsf(seed) * 2.4e-7f + 1e-30f;     // strictly below: ties with the seed still enter
-      }
+      if (p.seed)                                   // kc-th best of the sample (lists are sorted)
+        seed = seed_threshold(p.seed[(size_t(qt) * kQTile + row) * kc + kc - 1]);
       float thr = seed;
       for (int64_t t = t0; t < t1; ++t, ++it) {
         const uint32_t a = it & 1, pha = (it >> 1) & 1;
@@ -345,11 +366,14 @@ topk_scan_kernel(const __grid_constant__ Maps maps, const Args p) {
   if (warp == kMmaWarp) tmem_dealloc(tmem, 512);
 }
 
-// ---- |d|^2 per database row (L2 metric); +inf for the padding rows -----------------
+// ---- |d|^2 per database row (L2 metric); +inf for the padding rows; and the ----------
+// largest |d|^2 of the real rows into *max_sqnorm (float bits, zeroed by the caller)
 __global__ void __launch_bounds__(256)
-row_sqnorm_kernel(const __half *__restrict__ db, int64_t rows, int64_t padded, float *__restrict__ out) {
+row_sqnorm_kernel(const __half *__restrict__ db, int64_t rows, int64_t padded, float *__restrict__ out,
+                  unsigned int *__restrict__ max_sqnorm) {
   const int sub = threadIdx.x & 15;
   const int64_t per_pass = int64_t(gridDim.x) * (blockDim.x >> 4);
+  float top = 0.f;
   for (int64_t i = int64_t(blockIdx.x) * (blockDim.x >> 4) + (threadIdx.x >> 4); i < padded;
        i += per_pass) {
     float s = 0.f;
@@ -366,7 +390,11 @@ row_sqnorm_kernel(const __half *__restrict__ db, int64_t rows, int64_t padded, f
 #pragma unroll
     for (int d = 8; d > 0; d >>= 1) s += __shfl_xor_sync(0xffffffffu, s, d, 16);
     if (sub == 0) out[i] = i < rows ? s : INFINITY;
+    if (i < rows) top = fmaxf(top, s);
   }
+#pragma unroll
+  for (int d = 16; d > 0; d >>= 1) top = fmaxf(top, __shfl_xor_sync(0xffffffffu, top, d));
+  if ((threadIdx.x & 31) == 0) atomicMax(max_sqnorm, __float_as_uint(top));
 }
 
 // ---- ordering -----------------------------------------------------------------------
@@ -389,6 +417,15 @@ __device__ __forceinline__ void warp_best(float &s, I &i) {
   }
 }
 
+// One step of the exact score's chain: the finish and the fallback passes share
+// it, so they produce the same bits.
+template <int METRIC>
+__device__ __forceinline__ float exact_step(float acc, float q, float x) {
+  if (METRIC == 0) return fmaf(q, x, acc);
+  const float d = q - x;
+  return fmaf(d, d, acc);
+}
+
 // Exact score of (query in shared memory as fp32, database row): a sequential
 // fp32 FMA chain in dimension order.
 template <int METRIC>
@@ -399,44 +436,35 @@ __device__ __forceinline__ float exact_score(const float *q, const __half *row) 
     const uint4 raw = __ldg(reinterpret_cast<const uint4 *>(row) + c);
     const __half *h = reinterpret_cast<const __half *>(&raw);
 #pragma unroll
-    for (int j = 0; j < 8; ++j) {
-      const float x = __half2float(h[j]);
-      if (METRIC == 0) {
-        acc = fmaf(q[c * 8 + j], x, acc);
-      } else {
-        const float d = q[c * 8 + j] - x;
-        acc = fmaf(d, d, acc);
-      }
-    }
+    for (int j = 0; j < 8; ++j) acc = exact_step<METRIC>(acc, q[c * 8 + j], __half2float(h[j]));
   }
   return METRIC == 0 ? acc : -acc;
 }
 
 constexpr int kFinishWarps = 4;
 
-template <int METRIC>
-__global__ void __launch_bounds__(kFinishWarps * 32)
-topk_finish_kernel(const __half *__restrict__ queries, const __half *__restrict__ db,
-                   float *__restrict__ part_scores, const int32_t *__restrict__ part_index,
-                   int64_t segs, int64_t qp, int kc, int64_t Q, int k, int64_t index_base,
-                   float *__restrict__ out_scores, int64_t *__restrict__ out_index) {
-  __shared__ float qsm[kFinishWarps][kHidden];
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int64_t qi = int64_t(blockIdx.x) * kFinishWarps + warp;
-  if (qi >= Q) return;
-  float *q = qsm[warp];
-#pragma unroll
-  for (int j = 0; j < 4; ++j) q[lane * 4 + j] = __half2float(queries[qi * kHidden + lane * 4 + j]);
-  __syncwarp();
+// Certificate margin, relative: eps = 2^-14 |q| N_max (cosine) or
+// 2^-14 (2 |q| N_max + N_max^2 + |q|^2) (L2, the scan's frame), N_max the
+// largest row norm.  It has to cover the exact chain's error plus the tensor
+// cores' error on the same dot product.  The sequential chain of 128 FMAs is
+// within 128 * 2^-24 * sum|q_i x_i| = 2^-17 sum|q_i x_i| of the real value.
+// Published measurements of fp16-input, fp32-accumulate tensor cores on earlier
+// NVIDIA generations show an accumulator that truncates, about 2^-23 per
+// addition, which over 128 products is 2^-16 sum|q_i x_i|; and
+// sum|q_i x_i| <= |q| N_max (for L2 the terms of 2 q.d - |d|^2 and |q|^2 add
+// the other two parts).  2^-14 leaves a margin of at least 4x over the sum.
+// The B200's accumulator has not been measured: this constant rests on that
+// argument, not on a measurement.
+constexpr float kCertRel = 1.f / 16384.f;
+
+// k selection rounds over the (score desc, index asc) order of query qi's
+// segs x kc candidate slots (index INT_MAX = empty slot).  Writes the output
+// row; returns the k-th score, or -inf when fewer than k rows exist.  One warp.
+__device__ __forceinline__ float select_topk(const float *__restrict__ part_scores, const int32_t *__restrict__ part_index,
+                             int64_t segs, int64_t qp, int kc, int64_t qi, int k, int64_t index_base,
+                             float *__restrict__ out_scores, int64_t *__restrict__ out_index) {
+  const int lane = threadIdx.x & 31;
   const int64_t C = segs * kc;
-  // pass 1: exact scores, written over the tensor-core scores
-  for (int64_t c = lane; c < C; c += 32) {
-    const size_t off = (size_t(c / kc) * qp + qi) * kc + (c % kc);
-    const int32_t idx = part_index[off];
-    part_scores[off] = idx == INT_MAX ? -INFINITY : exact_score<METRIC>(q, db + int64_t(idx) * kHidden);
-  }
-  __syncwarp();
-  // pass 2: k selection rounds over the (score desc, index asc) order
   float last_s = INFINITY;
   int32_t last_i = -1;
   for (int r = 0; r < k; ++r) {
@@ -461,11 +489,170 @@ topk_finish_kernel(const __half *__restrict__ queries, const __half *__restrict_
         out_scores[qi * k + rr] = -INFINITY;
         out_index[qi * k + rr] = -1;
       }
-      break;
+      return -INFINITY;
     }
     last_s = bs;
     last_i = bi;
   }
+  return last_s;
+}
+
+// One warp per query: exact rescoring of the candidates, selection, and the
+// certificate.  `seed` is the seeding pre-pass's [qp][kc] lists or NULL;
+// uncertified queries are appended to `flagged` (count in *fallbacks).
+template <int METRIC>
+__global__ void __launch_bounds__(kFinishWarps * 32)
+topk_finish_kernel(const __half *__restrict__ queries, const __half *__restrict__ db,
+                   float *__restrict__ part_scores, const int32_t *__restrict__ part_index,
+                   const float *__restrict__ seed, const unsigned int *__restrict__ max_sqnorm,
+                   int64_t segs, int64_t qp, int kc, int64_t Q, int k, int64_t index_base,
+                   float *__restrict__ out_scores, int64_t *__restrict__ out_index,
+                   unsigned long long *__restrict__ fallbacks, int32_t *__restrict__ flagged) {
+  __shared__ float qsm[kFinishWarps][kHidden];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int64_t qi = int64_t(blockIdx.x) * kFinishWarps + warp;
+  if (qi >= Q) return;
+  float *q = qsm[warp];
+  float qq = 0.f;
+#pragma unroll
+  for (int j = 0; j < 4; ++j) {
+    const float v = __half2float(queries[qi * kHidden + lane * 4 + j]);
+    q[lane * 4 + j] = v;
+    qq = fmaf(v, v, qq);
+  }
+  // pass 0, before the tensor-core scores are overwritten: every row the scan
+  // dropped has a tensor-core score <= max(seed', last entry of a full list)
+  float bound = seed ? seed_threshold(seed[qi * kc + kc - 1]) : -INFINITY;
+  for (int64_t s = lane; s < segs; s += 32) {
+    const size_t off = (size_t(s) * qp + qi) * kc + kc - 1;
+    if (part_index[off] != INT_MAX) bound = fmaxf(bound, part_scores[off]);
+  }
+#pragma unroll
+  for (int d = 16; d > 0; d >>= 1) {
+    qq += __shfl_xor_sync(0xffffffffu, qq, d);
+    bound = fmaxf(bound, __shfl_xor_sync(0xffffffffu, bound, d));
+  }
+  __syncwarp();
+  const int64_t C = segs * kc;
+  // pass 1: exact scores, written over the tensor-core scores
+  for (int64_t c = lane; c < C; c += 32) {
+    const size_t off = (size_t(c / kc) * qp + qi) * kc + (c % kc);
+    const int32_t idx = part_index[off];
+    part_scores[off] = idx == INT_MAX ? -INFINITY : exact_score<METRIC>(q, db + int64_t(idx) * kHidden);
+  }
+  __syncwarp();
+  // pass 2: selection
+  const float sk = select_topk(part_scores, part_index, segs, qp, kc, qi, k, index_base, out_scores,
+                               out_index);
+  // certificate: no dropped row can reach the k-th exact score (kCertRel above).
+  // A query whose scan dropped nothing (B = -inf: small databases) is exact as it is.
+  const float n2 = __uint_as_float(*max_sqnorm), qn = sqrtf(qq), nmax = sqrtf(n2);
+  const float eps = METRIC == 0 ? kCertRel * qn * nmax : kCertRel * (2.f * qn * nmax + n2 + qq);
+  const float sk_scan = METRIC == 0 ? sk : sk + qq;
+  if (lane == 0 && bound > -INFINITY && !(bound + eps < sk_scan))
+    flagged[atomicAdd(fallbacks, 1ull)] = int32_t(qi);
+}
+
+// ---- exact fallback -----------------------------------------------------------------
+// Work item = (group of kFbWarps flagged queries, database segment): the CTA
+// stages 64 rows at a time in shared memory as fp32 (read from global memory
+// once for the whole group); warp w scores them for query w with the exact
+// chain (two rows per lane) and keeps the segment's k best by (score desc,
+// index asc) in registers, entry j in lane j.  The list goes to the query's
+// candidate slots of that segment (the first k of kc; the rest emptied), which
+// topk_fallback_select_kernel then reduces as the finish kernel does.
+constexpr int kFbWarps = 8, kFbRows = 64, kFbStride = kHidden + 1;   // +1: conflict-free columns
+constexpr int kFbBlocksPerSM = 4;
+
+template <int METRIC>
+__global__ void __launch_bounds__(kFbWarps * 32)
+topk_fallback_scan_kernel(const __half *__restrict__ queries, const __half *__restrict__ db,
+                          int64_t num_rows, int64_t rows_per_seg, int64_t segs, int64_t qp, int kc, int k,
+                          const unsigned long long *__restrict__ fallbacks,
+                          const int32_t *__restrict__ flagged, float *__restrict__ part_scores,
+                          int32_t *__restrict__ part_index) {
+  __shared__ float xs[kFbRows * kFbStride];
+  __shared__ float qsm[kFbWarps][kHidden];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int64_t n = int64_t(*fallbacks);
+  const int64_t groups = (n + kFbWarps - 1) / kFbWarps;
+  for (int64_t w = blockIdx.x; w < groups * segs; w += gridDim.x) {
+    const int64_t g = w % groups, seg = w / groups;     // neighbouring CTAs share a segment (L2)
+    const bool active = g * kFbWarps + warp < n;        // warp-uniform
+    const int64_t qi = active ? flagged[g * kFbWarps + warp] : 0;
+    __syncthreads();                                    // the previous item is done with qsm / xs
+    if (active) {
+#pragma unroll
+      for (int j = 0; j < 4; ++j) qsm[warp][lane * 4 + j] = __half2float(queries[qi * kHidden + lane * 4 + j]);
+    }
+    const float *q = qsm[warp];
+    float ls = -INFINITY, ts = -INFINITY;               // this lane's entry; the k-th entry
+    int32_t li = INT_MAX, ti = INT_MAX;
+    const int64_t r0 = seg * rows_per_seg;
+    const int64_t r1 = r0 + rows_per_seg < num_rows ? r0 + rows_per_seg : num_rows;
+    for (int64_t t = r0; t < r1; t += kFbRows) {
+      __syncthreads();
+      for (int e = threadIdx.x; e < kFbRows * (kHidden / 8); e += kFbWarps * 32) {
+        const int r = e / (kHidden / 8), c = e % (kHidden / 8);
+        uint4 raw = make_uint4(0u, 0u, 0u, 0u);
+        if (t + r < r1) raw = __ldg(reinterpret_cast<const uint4 *>(db + (t + r) * kHidden) + c);
+        const __half *h = reinterpret_cast<const __half *>(&raw);
+#pragma unroll
+        for (int j = 0; j < 8; ++j) xs[r * kFbStride + c * 8 + j] = __half2float(h[j]);
+      }
+      __syncthreads();
+      if (!active) continue;
+      const float *x0 = xs + lane * kFbStride, *x1 = xs + (lane + 32) * kFbStride;
+      float a0 = 0.f, a1 = 0.f;
+#pragma unroll 16
+      for (int d = 0; d < kHidden; ++d) {
+        a0 = exact_step<METRIC>(a0, q[d], x0[d]);
+        a1 = exact_step<METRIC>(a1, q[d], x1[d]);
+      }
+#pragma unroll
+      for (int h = 0; h < 2; ++h) {
+        const float s = METRIC == 0 ? (h ? a1 : a0) : -(h ? a1 : a0);
+        const int32_t i = int32_t(t + h * 32 + lane);
+        unsigned int m = __ballot_sync(0xffffffffu, t + h * 32 + lane < r1 && better<int32_t>(s, i, ts, ti));
+        while (m) {                                     // rare once the list has filled
+          const int src = __ffs(m) - 1;
+          m &= m - 1;
+          const float cs = __shfl_sync(0xffffffffu, s, src);
+          const int32_t ci = __shfl_sync(0xffffffffu, i, src);
+          if (!better<int32_t>(cs, ci, ts, ti)) continue;
+          const int pos = __popc(__ballot_sync(0xffffffffu, lane < k && better<int32_t>(ls, li, cs, ci)));
+          const float us = __shfl_up_sync(0xffffffffu, ls, 1);
+          const int32_t ui = __shfl_up_sync(0xffffffffu, li, 1);
+          if (lane > pos) {
+            ls = us;
+            li = ui;
+          } else if (lane == pos) {
+            ls = cs;
+            li = ci;
+          }
+          ts = __shfl_sync(0xffffffffu, ls, k - 1);
+          ti = __shfl_sync(0xffffffffu, li, k - 1);
+        }
+      }
+    }
+    if (active && lane < kc) {
+      const size_t off = (size_t(seg) * qp + qi) * kc + lane;
+      part_scores[off] = lane < k ? ls : -INFINITY;
+      part_index[off] = lane < k ? li : INT_MAX;
+    }
+  }
+}
+
+__global__ void __launch_bounds__(kFinishWarps * 32)
+topk_fallback_select_kernel(const float *__restrict__ part_scores, const int32_t *__restrict__ part_index,
+                            int64_t segs, int64_t qp, int kc, int k, int64_t index_base,
+                            const unsigned long long *__restrict__ fallbacks,
+                            const int32_t *__restrict__ flagged, float *__restrict__ out_scores,
+                            int64_t *__restrict__ out_index) {
+  const int warp = threadIdx.x >> 5;
+  const int64_t n = int64_t(*fallbacks);
+  for (int64_t f = int64_t(blockIdx.x) * kFinishWarps + warp; f < n; f += int64_t(gridDim.x) * kFinishWarps)
+    select_topk(part_scores, part_index, segs, qp, kc, flagged[f], k, index_base, out_scores, out_index);
 }
 
 __global__ void __launch_bounds__(kFinishWarps * 32)
@@ -518,6 +705,32 @@ static int launch_scan(const Maps &maps, const Args &a, int64_t items, cudaStrea
   return GFX_OK;
 }
 
+// scan (after the optional seeding pre-pass), finish with the certificate, and
+// the exact fallback for the flagged queries -- all stream-ordered, no host sync
+template <int METRIC>
+static int search(const Maps &maps, const Args &a, const Args &pre, const Plan &plan, const __half *q,
+                  const __half *db, int64_t Q, int64_t num_rows, int k, int64_t index_base,
+                  float *out_scores, int64_t *out_index, unsigned long long *fallbacks,
+                  const unsigned int *max_sqnorm, int32_t *flagged, cudaStream_t st) {
+  int rc = plan.sample_tiles ? launch_scan<METRIC>(maps, pre, plan.tiles_q, st) : GFX_OK;
+  if (!rc) rc = launch_scan<METRIC>(maps, a, plan.tiles_q * plan.segs, st);
+  if (rc) return rc;
+  const int finish_blocks = int((Q + kFinishWarps - 1) / kFinishWarps);
+  topk_finish_kernel<METRIC><<<finish_blocks, kFinishWarps * 32, 0, st>>>(
+      q, db, a.part_scores, a.part_index, a.seed, max_sqnorm,
+      plan.segs, plan.qp, plan.kc, Q, k, index_base, out_scores, out_index, fallbacks, flagged);
+  GFX_LAUNCH_CHECK();
+  topk_fallback_scan_kernel<METRIC><<<kNumSMs * kFbBlocksPerSM, kFbWarps * 32, 0, st>>>(
+      q, db, num_rows, plan.tiles_per_seg * kDbTile, plan.segs, plan.qp, plan.kc, k, fallbacks, flagged,
+      a.part_scores, a.part_index);
+  GFX_LAUNCH_CHECK();
+  topk_fallback_select_kernel<<<kNumSMs, kFinishWarps * 32, 0, st>>>(
+      a.part_scores, a.part_index, plan.segs, plan.qp, plan.kc, k, index_base, fallbacks, flagged,
+      out_scores, out_index);
+  GFX_LAUNCH_CHECK();
+  return GFX_OK;
+}
+
 }  // namespace topk
 }  // namespace gfx
 
@@ -555,6 +768,8 @@ extern "C" int gfx_topk(const void *queries, int64_t num_queries, const void *da
   a.tiles_per_seg = plan.tiles_per_seg; a.qp = plan.qp; a.num_rows = num_rows; a.kc = plan.kc;
   const __half *q = static_cast<const __half *>(queries), *db = static_cast<const __half *>(database);
   const int finish_blocks = int((num_queries + topk::kFinishWarps - 1) / topk::kFinishWarps);
+  // fallback count and largest squared row norm start at 0
+  GFX_CUDA(cudaMemsetAsync(ws, 0, topk::kHeaderBytes, st));
   if (num_rows == 0) {
     // empty database: a merge of zero lists writes (-inf, -1) everywhere
     StageScope scope(GFX_STAGE_TOPK, st, 1);
@@ -567,8 +782,8 @@ extern "C" int gfx_topk(const void *queries, int64_t num_queries, const void *da
   int rc = tma::make_rows128_map(&maps.q, q, num_queries, 128);
   if (!rc) rc = tma::make_rows128_map(&maps.db, db, num_rows, 128);
   if (rc) return rc;
-  StageScope scope(GFX_STAGE_TOPK, st, (metric == 1 ? 3 : 2) + (plan.sample_tiles ? 1 : 0));
-  const int64_t items = plan.tiles_q * plan.segs;
+  // sqnorm, [pre-pass,] scan, finish, fallback scan, fallback select
+  StageScope scope(GFX_STAGE_TOPK, st, 5 + (plan.sample_tiles ? 1 : 0));
   topk::Args pre = a;                      // seeding pre-pass over the first rows, one segment
   static const bool seeding = [] {         // developer switch: GFX_TOPK_SEED=0 scans unseeded
     const char *v = getenv("GFX_TOPK_SEED");
@@ -583,28 +798,22 @@ extern "C" int gfx_topk(const void *queries, int64_t num_queries, const void *da
     pre.num_rows = plan.sample_tiles * topk::kDbTile;
     a.seed = pre.part_scores;
   }
-  if (metric == 1) {
+  auto *fallbacks = reinterpret_cast<unsigned long long *>(ws + topk::kOffFallbacks);
+  auto *max_sqnorm = reinterpret_cast<unsigned int *>(ws + topk::kOffMaxSqNorm);
+  auto *flagged = reinterpret_cast<int32_t *>(ws + plan.off_flagged);
+  {
     const int64_t padded = plan.tiles_db * topk::kDbTile;
     int64_t blocks = (padded + 15) / 16;
     if (blocks > int64_t(kNumSMs) * 8) blocks = int64_t(kNumSMs) * 8;
-    topk::row_sqnorm_kernel<<<int(blocks), 256, 0, st>>>(db, num_rows, padded, const_cast<float *>(a.d2));
+    topk::row_sqnorm_kernel<<<int(blocks), 256, 0, st>>>(db, num_rows, padded, const_cast<float *>(a.d2),
+                                                        max_sqnorm);
     GFX_LAUNCH_CHECK();
-    if (plan.sample_tiles && (rc = topk::launch_scan<1>(maps, pre, plan.tiles_q, st))) return rc;
-    rc = topk::launch_scan<1>(maps, a, items, st);
-    if (rc) return rc;
-    topk::topk_finish_kernel<1><<<finish_blocks, topk::kFinishWarps * 32, 0, st>>>(
-        q, db, a.part_scores, a.part_index, plan.segs, plan.qp, plan.kc, num_queries, k, index_base,
-        out_scores, out_index);
-  } else {
-    if (plan.sample_tiles && (rc = topk::launch_scan<0>(maps, pre, plan.tiles_q, st))) return rc;
-    rc = topk::launch_scan<0>(maps, a, items, st);
-    if (rc) return rc;
-    topk::topk_finish_kernel<0><<<finish_blocks, topk::kFinishWarps * 32, 0, st>>>(
-        q, db, a.part_scores, a.part_index, plan.segs, plan.qp, plan.kc, num_queries, k, index_base,
-        out_scores, out_index);
   }
-  GFX_LAUNCH_CHECK();
-  return GFX_OK;
+  return metric == 1
+      ? topk::search<1>(maps, a, pre, plan, q, db, num_queries, num_rows, k, index_base, out_scores,
+                        out_index, fallbacks, max_sqnorm, flagged, st)
+      : topk::search<0>(maps, a, pre, plan, q, db, num_queries, num_rows, k, index_base, out_scores,
+                        out_index, fallbacks, max_sqnorm, flagged, st);
 }
 
 extern "C" int gfx_topk_merge(const float *in_scores, const int64_t *in_index, int parts,

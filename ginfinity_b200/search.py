@@ -10,6 +10,15 @@ so the contract here is this package's own:
   * results are ordered by (score descending, database index ascending);
     scores are the sequential fp32 FMA chain over dimensions 0..127 of the
     fp16 inputs, so they are reproducible bit for bit on any rank layout;
+  * the result is exact for every input.  A tensor-core scan keeps a few
+    candidates per database segment, which are rescored exactly; a query is
+    certified when the highest tensor-core score the scan dropped, plus a
+    margin (2^-14 |q| N_max for cosine, N_max the largest row norm; see
+    csrc/gfx_topk.cu), is below its k-th exact score, so no dropped row can
+    reach the top k.  Queries that fail are rescored exactly against every
+    row on the device in the same call.  A database with one very large-norm
+    row, or with many near-duplicates of a query's best rows, pays for that
+    fallback; `EmbeddingIndex.last_fallbacks()` counts the queries that took it;
   * multi-GPU: every rank holds a contiguous row range of the database
     (`EmbeddingIndex.shard`), queries are replicated, each rank takes its
     local top-k on its own GPU (gfx_topk: tcgen05 GEMM with the running top-k
@@ -91,6 +100,8 @@ class EmbeddingIndex:
         scores = torch.empty((Q, k), dtype=torch.float32, device=self.device)
         index = torch.empty((Q, k), dtype=torch.int64, device=self.device)
         if Q == 0:
+            if self._ws is not None:
+                self._ws[:8].zero_()       # no query took the fallback
             return scores, index
         with torch.cuda.device(self.device):
             need = nat.lib.gfx_topk_workspace_bytes(Q, D, int(k))
@@ -102,6 +113,15 @@ class EmbeddingIndex:
                 index.data_ptr(), self._ws.data_ptr(), self._ws.numel(),
                 torch.cuda.current_stream().cuda_stream))
         return scores, index
+
+    def last_fallbacks(self) -> int:
+        """Number of queries of the last `search` on this index that took the
+        exact fallback (their candidates could not be certified).  gfx_topk
+        keeps this count as an int64 in the first 8 bytes of its workspace;
+        reading it waits for the search to finish."""
+        if self._ws is None:
+            return 0
+        return int(self._ws[:8].view(torch.int64).item())
 
     # -- sharded search -----------------------------------------------------------
     def search_sharded(self, queries, k: int = 10, metric: str = "cosine", *,

@@ -360,6 +360,17 @@ int gfx_encode_described_f32(const gfx_model *model, const float *x,
  * metric 0 = cosine (dot product), 1 = L2 (ranked by -|q-d|^2).
  * Result order: score descending, database index ascending on ties;
  * out_scores float32 [Q,k], out_index int64 [Q,k] (index + index_base).
+ * Scores are the sequential fp32 FMA chain over dimensions 0..127, and the
+ * result is exact for every input: a tensor-core scan picks kc candidates per
+ * database segment, the candidates are rescored exactly, and each query is
+ * certified when the highest tensor-core score the scan dropped, plus a
+ * margin of 2^-14 |q| N_max (L2: 2^-14 (2 |q| N_max + N_max^2 + |q|^2);
+ * N_max the largest row norm), is below its k-th exact score.  Queries that
+ * fail the certificate are rescored exactly against every row, on the
+ * device, within the same call.  A database with one very large-norm row, or
+ * with many near-duplicates of a query's best rows, pays for that fallback.
+ * The first 8 bytes of the workspace hold, after the call, the number of
+ * queries that took it (int64).
  * ------------------------------------------------------------------------ */
 size_t gfx_topk_workspace_bytes(int64_t num_queries, int64_t num_rows, int k);
 int gfx_topk(const void *queries, int64_t num_queries, const void *database,

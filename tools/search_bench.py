@@ -54,7 +54,7 @@ def main():
             nat.profile_read("topk")
             flop = 2.0 * 128 * Q * D
             row = {"Q": Q, "D": D, "metric": metric, "seconds": t, "tflops": flop / t / 1e12,
-                   "db_rows_per_s": D / t}
+                   "db_rows_per_s": D / t, "fallbacks": index.last_fallbacks()}
             if Q * D <= 4096 * 1_000_000:
                 def lib():
                     s = q @ db.T

@@ -86,6 +86,10 @@ _SIGNATURES = {
     "gfx_topk_workspace_bytes": (_sz, [_i64, _i64, C.c_int]),
     "gfx_topk": (C.c_int, [_p, _i64, _p, _i64, C.c_int, C.c_int, C.c_int, _i64,
                            _p, _p, _p, _sz, _p]),
+    "gfx_topk_f32_prepare": (C.c_int, [_p, _i64, _p, _p]),
+    "gfx_topk_f32_workspace_bytes": (_sz, [_i64, _i64, C.c_int]),
+    "gfx_topk_f32": (C.c_int, [_p, _i64, _p, _p, _i64, C.c_int, C.c_int, C.c_int, _i64,
+                               _p, _p, _p, _sz, _p]),
     "gfx_topk_merge": (C.c_int, [_p, _p, C.c_int, _i64, C.c_int, _p, _p, _p]),
     "gfx_profile_enable": (C.c_int, [C.c_uint32]),
     "gfx_profile_read": (C.c_int, [C.c_int, C.POINTER(C.c_double), C.POINTER(_i64), C.c_int]),

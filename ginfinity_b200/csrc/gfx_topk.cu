@@ -85,13 +85,15 @@ struct Plan {
   int kc;
   int64_t sample_tiles;       // 0 = no seeding pre-pass
   size_t off_flagged, off_scores, off_index, off_d2, off_seed_scores, off_seed_index, total;
+  size_t off_qimage;          // fp32 search: [Q, 256] hi | lo image of the queries
 };
 
-static Plan make_plan(int64_t Q, int64_t D, int k) {
+// `q_tile`: queries per work item of the scan (kQTile; kQTile32 for fp32 inputs)
+static Plan make_plan(int64_t Q, int64_t D, int k, int q_tile = kQTile) {
   Plan p{};
-  p.tiles_q = (Q + kQTile - 1) / kQTile;
+  p.tiles_q = (Q + q_tile - 1) / q_tile;
   p.tiles_db = (D + kDbTile - 1) / kDbTile;
-  p.qp = p.tiles_q * kQTile;
+  p.qp = p.tiles_q * q_tile;
   int64_t segs = 1;
   if (p.tiles_q > 0 && p.tiles_q < int64_t(kWaves) * kNumSMs)
     segs = (int64_t(kWaves) * kNumSMs + p.tiles_q - 1) / p.tiles_q;
@@ -731,6 +733,529 @@ static int search(const Maps &maps, const Args &a, const Args &pre, const Plan &
   return GFX_OK;
 }
 
+// =====================================================================================
+// fp32 inputs (gfx_topk_f32): the same contract over float32 rows and queries.  The
+// scores are the sequential fp32 FMA chain over the fp32 values.  The scan multiplies
+// split-fp16 images, x = hi + lo, hi = fp16(x), lo = fp16(x - hi) (the split of
+// gfx_split9.cu): per K step three kind::f16 MMAs, hi.hi + hi.lo + lo.hi, into one fp32
+// TMEM accumulator.  The database image [rows, 256] (hi | lo) is built once per index
+// (gfx_topk_f32_prepare); the queries' image is built per call in the workspace.  Hi and
+// lo operands need twice the shared memory, so a work item holds 128 queries (M = 128):
+//   queries hi + lo 64 KB | 2 database stages x 64 KB (128 rows, hi + lo) | |d|^2 slots
+//   4 KB | candidate lists <= 28 KB  = 224 KB.
+// Warps: 0-3 epilogue (one query per thread), 4 MMA issuer, 5 TMA loader; TMEM 2 x 128
+// columns.  Segments, the seeding pre-pass, kc and the finish / certificate / fallback
+// structure are those above; finish and fallback read the fp32 rows (512 B per row).
+// =====================================================================================
+constexpr int kQTile32 = 128, kStages32 = 2;
+constexpr int kQBytes32 = 4 * kBoxBytes;          // [hi, lo] x 2 K blocks x 128 rows
+constexpr int kDbBytes32 = 4 * kBoxBytes;
+constexpr int kMmaWarp32 = 4, kLoadWarp32 = 5, kWarps32 = 6, kEpiWarps32 = 4;
+
+enum Bar32 {
+  kB32QFull = 0, kB32QEmpty = 1, kB32BFull = 2, kB32BEmpty = 4, kB32DFull = 6, kB32DEmpty = 8,
+  kNumBars32 = 10
+};
+
+struct Smem32 {
+  static constexpr int off_q = 0;
+  static constexpr int off_db = off_q + kQBytes32;
+  static constexpr int off_d2 = off_db + kStages32 * kDbBytes32;
+  static constexpr int off_bar = off_d2 + kD2Slots * kDbTile * 4;
+  static constexpr int off_tmem = off_bar + kNumBars32 * 8;
+  static constexpr int off_list = (off_tmem + 8 + 15) & ~15;
+  static constexpr int total(int kc) { return off_list + kc * kQTile32 * 8; }
+};
+static_assert(Smem32::total(kMaxCand) <= 232448, "exceeds the 227 KB shared-memory limit of sm_100");
+
+static Plan make_plan_f32(int64_t Q, int64_t D, int k) {
+  Plan p = make_plan(Q, D, k, kQTile32);
+  p.off_qimage = p.total;
+  p.total += (size_t(Q) * 2 * kHidden * 2 + 255) & ~size_t(255);
+  return p;
+}
+
+// list_insert with the 128-query stride of the fp32 scan's lists
+__device__ __noinline__ float list_insert32(float *ls, int32_t *li, int kc, float v, int32_t idx) {
+  int j = kc - 1;
+  while (j > 0 && ls[(j - 1) * kQTile32] < v) {
+    ls[j * kQTile32] = ls[(j - 1) * kQTile32];
+    li[j * kQTile32] = li[(j - 1) * kQTile32];
+    --j;
+  }
+  ls[j * kQTile32] = v;
+  li[j * kQTile32] = idx;
+  return ls[(kc - 1) * kQTile32];
+}
+
+template <int METRIC>
+__global__ void __launch_bounds__(kWarps32 * 32, 1)
+split_search_kernel(const __grid_constant__ Maps maps, const Args p) {
+  using L = Smem32;
+  extern __shared__ __align__(1024) uint8_t smem[];
+  uint8_t *qs = smem + L::off_q, *dbs = smem + L::off_db;
+  float *d2s = reinterpret_cast<float *>(smem + L::off_d2);
+  uint64_t *bar = reinterpret_cast<uint64_t *>(smem + L::off_bar);
+  uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(smem + L::off_tmem);
+  float *list_s = reinterpret_cast<float *>(smem + L::off_list);
+
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  if (warp == kMmaWarp32) {
+    tmem_alloc(tmem_slot, 256);
+  } else if (tid == 0) {
+    mbar_init(bar + kB32QFull, 1);
+    mbar_init(bar + kB32QEmpty, 1);
+    for (int s = 0; s < kStages32; ++s) {
+      mbar_init(bar + kB32BFull + s, 1);
+      mbar_init(bar + kB32BEmpty + s, 1);
+    }
+    for (int a = 0; a < 2; ++a) {
+      mbar_init(bar + kB32DFull + a, 1);
+      mbar_init(bar + kB32DEmpty + a, kEpiWarps32);
+    }
+    fence_mbar_init();
+  }
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem = *tmem_slot;
+  const int64_t items = p.tiles_q * p.segs;
+
+  if (warp == kLoadWarp32) {
+    // ================================ TMA loader =================================
+    // Box b of a 128-row block is columns [64 b, 64 b + 64) of the image: hi K block 0, 1,
+    // then lo K block 0, 1 -- in shared memory at b * kBoxBytes.
+    uint32_t elected;
+    asm volatile("{\n.reg .pred q;\nelect.sync _|q, 0xffffffff;\nselp.u32 %0, 1, 0, q;\n}" : "=r"(elected));
+    const bool issuer = elected != 0u;
+    if (issuer) {
+      prefetch_tmap(&maps.q);
+      prefetch_tmap(&maps.db);
+    }
+    uint32_t it = 0, item_n = 0;
+    for (int64_t item = blockIdx.x; item < items; item += gridDim.x, ++item_n) {
+      const int64_t qt = item % p.tiles_q, seg = item / p.tiles_q;
+      mbar_wait(bar + kB32QEmpty, (item_n & 1) ^ 1);
+      if (issuer) {
+        mbar_arrive_expect_tx(bar + kB32QFull, kQBytes32);
+#pragma unroll
+        for (int b = 0; b < 4; ++b)
+          tma_load_2d(qs + b * kBoxBytes, &maps.q, b * 64, int(qt * kQTile32), bar + kB32QFull);
+      }
+      __syncwarp();
+      const int64_t t0 = seg * p.tiles_per_seg;
+      const int64_t t1 = t0 + p.tiles_per_seg < p.tiles_db ? t0 + p.tiles_per_seg : p.tiles_db;
+      for (int64_t t = t0; t < t1; ++t, ++it) {
+        const uint32_t s = it % kStages32, ph = (it / kStages32) & 1;
+        uint8_t *dst = dbs + s * kDbBytes32;
+        mbar_wait(bar + kB32BEmpty + s, ph ^ 1);
+        if (issuer) {
+          mbar_arrive_expect_tx(bar + kB32BFull + s, kDbBytes32 + (METRIC == 1 ? kDbTile * 4 : 0));
+#pragma unroll
+          for (int b = 0; b < 4; ++b)
+            tma_load_2d(dst + b * kBoxBytes, &maps.db, b * 64, int(t * kDbTile), bar + kB32BFull + s);
+          if (METRIC == 1)
+            bulk_g2s(d2s + (it % kD2Slots) * kDbTile, p.d2 + t * kDbTile, kDbTile * 4,
+                     bar + kB32BFull + s);
+        }
+        __syncwarp();
+      }
+    }
+    __syncwarp();
+  } else if (warp == kMmaWarp32) {
+    // ================================ MMA issuer =================================
+    // whole warp in the loop, one elected lane issues with warp-uniform operands (see topk_scan_kernel)
+    constexpr uint32_t idesc = idesc_f16(kQTile32, kDbTile);
+    const uint32_t qa = smem_u32(qs), ba = smem_u32(dbs);
+    const uint32_t tm = __shfl_sync(0xffffffffu, tmem, 0);
+    uint32_t elected;
+    asm volatile("{\n.reg .pred q;\nelect.sync _|q, 0xffffffff;\nselp.u32 %0, 1, 0, q;\n}" : "=r"(elected));
+    const bool issuer = elected != 0u;
+    uint32_t it = 0, item_n = 0;
+    for (int64_t item = blockIdx.x; item < items; item += gridDim.x, ++item_n) {
+      const int64_t seg = item / p.tiles_q;
+      const int64_t t0 = seg * p.tiles_per_seg;
+      const int64_t t1 = t0 + p.tiles_per_seg < p.tiles_db ? t0 + p.tiles_per_seg : p.tiles_db;
+      mbar_wait(bar + kB32QFull, item_n & 1);
+      for (int64_t t = t0; t < t1; ++t, ++it) {
+        const uint32_t s = it % kStages32, ph = (it / kStages32) & 1, a = it & 1, pha = (it >> 1) & 1;
+        mbar_wait(bar + kB32BFull + s, ph);
+        mbar_wait(bar + kB32DEmpty + a, pha ^ 1);
+        tc_fence_after();
+        if (issuer) {
+#pragma unroll
+          for (int kk = 0; kk < 8; ++kk) {
+            const int kb = kk >> 2, k = kk & 3;
+#pragma unroll
+            for (int term = 0; term < 3; ++term) {       // hi.hi, hi.lo, lo.hi
+              const int qlo = term == 2, dlo = term == 1;
+              const uint64_t da = smem_desc_sw128(qa + (qlo * 2 + kb) * kBoxBytes + k * 32);
+              const uint64_t db = smem_desc_sw128(ba + s * kDbBytes32 + (dlo * 2 + kb) * kBoxBytes + k * 32);
+              mma_f16_ss(tm + a * kDbTile, da, db, idesc, (kk | term) != 0);
+            }
+          }
+          mma_commit(bar + kB32BEmpty + s);
+          mma_commit(bar + kB32DFull + a);
+        }
+        __syncwarp();
+      }
+      if (issuer) mma_commit(bar + kB32QEmpty);
+      __syncwarp();
+    }
+    __syncwarp();
+  } else {
+    // ============ epilogue: running top-k, one query per thread (as topk_scan_kernel) ========
+    const int row = warp * 32 + lane;                       // query inside the item = TMEM lane
+    const uint32_t tbase = tmem + (uint32_t(warp * 32) << 16);
+    const int kc = p.kc;
+    const int32_t rows = int32_t(p.num_rows);
+    float *ls = list_s + tid;
+    int32_t *li = reinterpret_cast<int32_t *>(list_s + kc * kQTile32) + tid;
+    const float ninf = -INFINITY;
+    uint32_t it = 0;
+    for (int64_t item = blockIdx.x; item < items; item += gridDim.x) {
+      const int64_t qt = item % p.tiles_q, seg = item / p.tiles_q;
+      const int64_t t0 = seg * p.tiles_per_seg;
+      const int64_t t1 = t0 + p.tiles_per_seg < p.tiles_db ? t0 + p.tiles_per_seg : p.tiles_db;
+      for (int j = 0; j < kc; ++j) {
+        ls[j * kQTile32] = ninf;
+        li[j * kQTile32] = INT_MAX;
+      }
+      float seed = ninf;
+      if (p.seed) seed = seed_threshold(p.seed[(size_t(qt) * kQTile32 + row) * kc + kc - 1]);
+      float thr = seed;
+      for (int64_t t = t0; t < t1; ++t, ++it) {
+        const uint32_t a = it & 1, pha = (it >> 1) & 1;
+        mbar_wait(bar + kB32DFull + a, pha);
+        tc_fence_after();
+        float v[kDbTile];
+#pragma unroll
+        for (int cb = 0; cb < 4; ++cb) tmem_ld32(tbase + a * kDbTile + cb * 32, v + cb * 32);
+        tmem_ld_wait();
+        tc_fence_before();
+        __syncwarp();
+        if (lane == 0) mbar_arrive(bar + kB32DEmpty + a);
+        const int32_t base = int32_t(t * kDbTile);
+        if (METRIC == 1) {
+          const float4 *d2 = reinterpret_cast<const float4 *>(d2s + (it % kD2Slots) * kDbTile);
+#pragma unroll
+          for (int c4 = 0; c4 < kDbTile / 4; ++c4) {
+            const float4 n = d2[c4];
+            v[4 * c4] = fmaf(2.f, v[4 * c4], -n.x);
+            v[4 * c4 + 1] = fmaf(2.f, v[4 * c4 + 1], -n.y);
+            v[4 * c4 + 2] = fmaf(2.f, v[4 * c4 + 2], -n.z);
+            v[4 * c4 + 3] = fmaf(2.f, v[4 * c4 + 3], -n.w);
+          }
+        }
+        float t4[4];
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+          t4[q] = fmaxf(v[32 * q], v[32 * q + 1]);
+#pragma unroll
+          for (int c = 2; c < 32; c += 2) t4[q] = max3(t4[q], v[32 * q + c], v[32 * q + c + 1]);
+        }
+        const float top = fmaxf(fmaxf(t4[0], t4[1]), fmaxf(t4[2], t4[3]));
+        if (top > thr) {
+#pragma unroll
+          for (int g = 0; g < kDbTile / 8; ++g) {
+            const float gm = fmaxf(max3(v[8 * g], v[8 * g + 1], v[8 * g + 2]),
+                                   max3(v[8 * g + 3], v[8 * g + 4],
+                                        max3(v[8 * g + 5], v[8 * g + 6], v[8 * g + 7])));
+            if (gm > thr) {
+#pragma unroll
+              for (int j = 0; j < 8; ++j)
+                if (v[8 * g + j] > thr && base + 8 * g + j < rows)
+                  thr = fmaxf(seed, list_insert32(ls, li, kc, v[8 * g + j], base + 8 * g + j));
+            }
+          }
+        }
+      }
+      const size_t out = (size_t(seg) * p.qp + size_t(qt) * kQTile32 + row) * kc;
+      for (int j = 0; j < kc; ++j) {
+        p.part_scores[out + j] = ls[j * kQTile32];
+        p.part_index[out + j] = li[j * kQTile32];
+      }
+    }
+  }
+  tc_fence_before();
+  __syncthreads();
+  if (warp == kMmaWarp32) tmem_dealloc(tmem, 256);
+}
+
+// [rows, 128] fp32 -> [rows, 256] fp16 image hi | lo, hi = fp16(x), lo = fp16(x - hi)
+// (round to nearest; fp16 subnormals kept).  One thread per 4 components.
+__global__ void __launch_bounds__(256)
+split_rows_kernel(const float *__restrict__ x, int64_t rows, __half *__restrict__ image) {
+  const int64_t n = rows * (kHidden / 4);
+  for (int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x; i < n; i += int64_t(gridDim.x) * blockDim.x) {
+    const int64_t r = i / (kHidden / 4), c = (i % (kHidden / 4)) * 4;
+    const float4 v = __ldg(reinterpret_cast<const float4 *>(x) + i);
+    const __half2 h0 = __floats2half2_rn(v.x, v.y), h1 = __floats2half2_rn(v.z, v.w);
+    const float2 b0 = __half22float2(h0), b1 = __half22float2(h1);
+    const __half2 l0 = __floats2half2_rn(v.x - b0.x, v.y - b0.y), l1 = __floats2half2_rn(v.z - b1.x, v.w - b1.y);
+    __half2 *hi = reinterpret_cast<__half2 *>(image + r * 2 * kHidden + c);
+    __half2 *lo = reinterpret_cast<__half2 *>(image + r * 2 * kHidden + kHidden + c);
+    hi[0] = h0;
+    hi[1] = h1;
+    lo[0] = l0;
+    lo[1] = l1;
+  }
+}
+
+// row_sqnorm_kernel over fp32 rows
+__global__ void __launch_bounds__(256)
+row_sqnorm32_kernel(const float *__restrict__ db, int64_t rows, int64_t padded, float *__restrict__ out,
+                    unsigned int *__restrict__ max_sqnorm) {
+  const int sub = threadIdx.x & 15;
+  const int64_t per_pass = int64_t(gridDim.x) * (blockDim.x >> 4);
+  float top = 0.f;
+  for (int64_t i = int64_t(blockIdx.x) * (blockDim.x >> 4) + (threadIdx.x >> 4); i < padded;
+       i += per_pass) {
+    float s = 0.f;
+    if (i < rows) {
+      const float4 *r = reinterpret_cast<const float4 *>(db + i * kHidden) + sub * 2;
+#pragma unroll
+      for (int j = 0; j < 2; ++j) {
+        const float4 f = __ldg(r + j);
+        s = fmaf(f.x, f.x, s);
+        s = fmaf(f.y, f.y, s);
+        s = fmaf(f.z, f.z, s);
+        s = fmaf(f.w, f.w, s);
+      }
+    }
+#pragma unroll
+    for (int d = 8; d > 0; d >>= 1) s += __shfl_xor_sync(0xffffffffu, s, d, 16);
+    if (sub == 0) out[i] = i < rows ? s : INFINITY;
+    if (i < rows) top = fmaxf(top, s);
+  }
+#pragma unroll
+  for (int d = 16; d > 0; d >>= 1) top = fmaxf(top, __shfl_xor_sync(0xffffffffu, top, d));
+  if ((threadIdx.x & 31) == 0) atomicMax(max_sqnorm, __float_as_uint(top));
+}
+
+// exact_score over an fp32 row: the same chain
+template <int METRIC>
+__device__ __forceinline__ float exact_score32(const float *q, const float *row) {
+  float acc = 0.f;
+#pragma unroll 4
+  for (int c = 0; c < kHidden / 4; ++c) {
+    const float4 x = __ldg(reinterpret_cast<const float4 *>(row) + c);
+    acc = exact_step<METRIC>(acc, q[c * 4], x.x);
+    acc = exact_step<METRIC>(acc, q[c * 4 + 1], x.y);
+    acc = exact_step<METRIC>(acc, q[c * 4 + 2], x.z);
+    acc = exact_step<METRIC>(acc, q[c * 4 + 3], x.w);
+  }
+  return METRIC == 0 ? acc : -acc;
+}
+
+// Certificate margin of the split scan:
+//   cosine  eps = kCertRelSplit |q| N_max + kCertAbsSplit (|q| + N_max)
+//   L2      eps = kCertRelSplit (2 |q| N_max + N_max^2 + |q|^2) + 2 kCertAbsSplit (|q| + N_max)
+// (the scan's frame, as kCertRel).  Against the real dot product R = sum q_i x_i:
+//  * the split.  With fp16 hi and lo normal, q_i = qh_i + ql_i + e_i, |e_i| <= 2^-22 |q_i|
+//    (hi is within 2^-11 |q_i|, lo within 2^-11 of the rest), and the same for x.  The scan
+//    sums qh.xh + qh.xl + ql.xh = (q - e_q).(x - e_x) - ql.xl; with |ql_i| <= 2^-11 (1 + 2^-11)
+//    |q_i| that is within (3 + 2^-9) 2^-22 < 2^-20 of sum |q_i x_i| from R, the dropped lo.lo
+//    term included;
+//  * subnormals.  Where x_i - hi_i (or x_i itself) is below 2^-14, lo (or hi) is rounded onto
+//    the fp16 subnormal grid of spacing 2^-24: an absolute error of at most 2^-25 per
+//    component, which sums to 2^-25 (|q|_1 + |x|_1) <= 2^-25 sqrt(128) (|q| + N_max)
+//    < 2^-21 (|q| + N_max) = kCertAbsSplit (|q| + N_max).  This assumes that kind::f16 takes
+//    subnormal fp16 operands at their value; an MMA that flushed them would lose up to 2^-14
+//    per component;
+//  * the tensor-core accumulator.  3 x 128 products go into one fp32 accumulator; on the
+//    truncation argument of kCertRel (about 2^-23 per addition) that is within
+//    384 x 2^-23 (1 + 2^-10) < 2^-14.4 of sum |q_i x_i|;
+//  * the exact chain: within 2^-17 sum |q_i x_i| (kCertRel).  For L2 the fp32 difference
+//    q_i - x_i adds 2^-23 relative per term of sum (q_i - x_i)^2 <= (|q| + N_max)^2.
+// The sum is below 2^-14.1 sum |q_i x_i| <= 2^-14.1 |q| N_max; 2^-13 leaves more than 2x
+// (for L2, 2 q.d doubles the first and the |d|^2, |q|^2 and chain errors, each <= 2^-16.9 of
+// their square, stay inside the other terms).  As for kCertRel, the B200's accumulator has not
+// been measured: this margin rests on the argument, not on a measurement.  Without the split
+// (a scan of fp16(x) only) the rounding of the inputs alone is 2^-11 sum |q_i x_i| per side.
+constexpr float kCertRelSplit = 1.f / 8192.f, kCertAbsSplit = 1.f / 2097152.f;
+
+// topk_finish_kernel for fp32 inputs.  A query with a component above the fp16 range (its hi
+// part is inf; the scan's scores for it are meaningless) is flagged whatever its certificate.
+template <int METRIC>
+__global__ void __launch_bounds__(kFinishWarps * 32)
+topk32_finish_kernel(const float *__restrict__ queries, const float *__restrict__ db,
+                     float *__restrict__ part_scores, const int32_t *__restrict__ part_index,
+                     const float *__restrict__ seed, const unsigned int *__restrict__ max_sqnorm,
+                     int64_t segs, int64_t qp, int kc, int64_t Q, int k, int64_t index_base,
+                     float *__restrict__ out_scores, int64_t *__restrict__ out_index,
+                     unsigned long long *__restrict__ fallbacks, int32_t *__restrict__ flagged) {
+  __shared__ float qsm[kFinishWarps][kHidden];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int64_t qi = int64_t(blockIdx.x) * kFinishWarps + warp;
+  if (qi >= Q) return;
+  float *q = qsm[warp];
+  float qq = 0.f, qmax = 0.f;
+  const float4 v = __ldg(reinterpret_cast<const float4 *>(queries + qi * kHidden) + lane);
+  q[lane * 4] = v.x;
+  q[lane * 4 + 1] = v.y;
+  q[lane * 4 + 2] = v.z;
+  q[lane * 4 + 3] = v.w;
+  qq = fmaf(v.x, v.x, fmaf(v.y, v.y, fmaf(v.z, v.z, fmaf(v.w, v.w, qq))));
+  qmax = fmaxf(fmaxf(fabsf(v.x), fabsf(v.y)), fmaxf(fabsf(v.z), fabsf(v.w)));
+  float bound = seed ? seed_threshold(seed[qi * kc + kc - 1]) : -INFINITY;
+  for (int64_t s = lane; s < segs; s += 32) {
+    const size_t off = (size_t(s) * qp + qi) * kc + kc - 1;
+    if (part_index[off] != INT_MAX) bound = fmaxf(bound, part_scores[off]);
+  }
+#pragma unroll
+  for (int d = 16; d > 0; d >>= 1) {
+    qq += __shfl_xor_sync(0xffffffffu, qq, d);
+    qmax = fmaxf(qmax, __shfl_xor_sync(0xffffffffu, qmax, d));
+    bound = fmaxf(bound, __shfl_xor_sync(0xffffffffu, bound, d));
+  }
+  __syncwarp();
+  const int64_t C = segs * kc;
+  for (int64_t c = lane; c < C; c += 32) {
+    const size_t off = (size_t(c / kc) * qp + qi) * kc + (c % kc);
+    const int32_t idx = part_index[off];
+    part_scores[off] = idx == INT_MAX ? -INFINITY : exact_score32<METRIC>(q, db + int64_t(idx) * kHidden);
+  }
+  __syncwarp();
+  const float sk = select_topk(part_scores, part_index, segs, qp, kc, qi, k, index_base, out_scores,
+                               out_index);
+  const float n2 = __uint_as_float(*max_sqnorm), qn = sqrtf(qq), nmax = sqrtf(n2);
+  const float abs_eps = kCertAbsSplit * (qn + nmax);
+  const float eps = METRIC == 0 ? kCertRelSplit * qn * nmax + abs_eps
+                                : kCertRelSplit * (2.f * qn * nmax + n2 + qq) + 2.f * abs_eps;
+  const float sk_scan = METRIC == 0 ? sk : sk + qq;
+  const bool out_of_range = !(qmax <= 65504.f);
+  if (lane == 0 && (out_of_range || (bound > -INFINITY && !(bound + eps < sk_scan))))
+    flagged[atomicAdd(fallbacks, 1ull)] = int32_t(qi);
+}
+
+// topk_fallback_scan_kernel for fp32 inputs: rows staged from the fp32 database directly
+template <int METRIC>
+__global__ void __launch_bounds__(kFbWarps * 32)
+topk32_fallback_scan_kernel(const float *__restrict__ queries, const float *__restrict__ db,
+                            int64_t num_rows, int64_t rows_per_seg, int64_t segs, int64_t qp, int kc, int k,
+                            const unsigned long long *__restrict__ fallbacks,
+                            const int32_t *__restrict__ flagged, float *__restrict__ part_scores,
+                            int32_t *__restrict__ part_index) {
+  __shared__ float xs[kFbRows * kFbStride];
+  __shared__ float qsm[kFbWarps][kHidden];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int64_t n = int64_t(*fallbacks);
+  const int64_t groups = (n + kFbWarps - 1) / kFbWarps;
+  for (int64_t w = blockIdx.x; w < groups * segs; w += gridDim.x) {
+    const int64_t g = w % groups, seg = w / groups;
+    const bool active = g * kFbWarps + warp < n;
+    const int64_t qi = active ? flagged[g * kFbWarps + warp] : 0;
+    __syncthreads();
+    if (active) {
+#pragma unroll
+      for (int j = 0; j < 4; ++j) qsm[warp][lane * 4 + j] = queries[qi * kHidden + lane * 4 + j];
+    }
+    const float *q = qsm[warp];
+    float ls = -INFINITY, ts = -INFINITY;
+    int32_t li = INT_MAX, ti = INT_MAX;
+    const int64_t r0 = seg * rows_per_seg;
+    const int64_t r1 = r0 + rows_per_seg < num_rows ? r0 + rows_per_seg : num_rows;
+    for (int64_t t = r0; t < r1; t += kFbRows) {
+      __syncthreads();
+#pragma unroll 1   // unrolled, ptxas spills at 48 registers
+      for (int e = threadIdx.x; e < kFbRows * (kHidden / 4); e += kFbWarps * 32) {
+        const int r = e / (kHidden / 4), c = e % (kHidden / 4);
+        float4 x = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (t + r < r1) x = __ldg(reinterpret_cast<const float4 *>(db + (t + r) * kHidden) + c);
+        float *dst = xs + r * kFbStride + c * 4;
+        dst[0] = x.x;
+        dst[1] = x.y;
+        dst[2] = x.z;
+        dst[3] = x.w;
+      }
+      __syncthreads();
+      if (!active) continue;
+      const float *x0 = xs + lane * kFbStride, *x1 = xs + (lane + 32) * kFbStride;
+      float a0 = 0.f, a1 = 0.f;
+#pragma unroll 16
+      for (int d = 0; d < kHidden; ++d) {
+        a0 = exact_step<METRIC>(a0, q[d], x0[d]);
+        a1 = exact_step<METRIC>(a1, q[d], x1[d]);
+      }
+#pragma unroll
+      for (int h = 0; h < 2; ++h) {
+        const float s = METRIC == 0 ? (h ? a1 : a0) : -(h ? a1 : a0);
+        const int32_t i = int32_t(t + h * 32 + lane);
+        unsigned int m = __ballot_sync(0xffffffffu, t + h * 32 + lane < r1 && better<int32_t>(s, i, ts, ti));
+        while (m) {
+          const int src = __ffs(m) - 1;
+          m &= m - 1;
+          const float cs = __shfl_sync(0xffffffffu, s, src);
+          const int32_t ci = __shfl_sync(0xffffffffu, i, src);
+          if (!better<int32_t>(cs, ci, ts, ti)) continue;
+          const int pos = __popc(__ballot_sync(0xffffffffu, lane < k && better<int32_t>(ls, li, cs, ci)));
+          const float us = __shfl_up_sync(0xffffffffu, ls, 1);
+          const int32_t ui = __shfl_up_sync(0xffffffffu, li, 1);
+          if (lane > pos) {
+            ls = us;
+            li = ui;
+          } else if (lane == pos) {
+            ls = cs;
+            li = ci;
+          }
+          ts = __shfl_sync(0xffffffffu, ls, k - 1);
+          ti = __shfl_sync(0xffffffffu, li, k - 1);
+        }
+      }
+    }
+    if (active && lane < kc) {
+      const size_t off = (size_t(seg) * qp + qi) * kc + lane;
+      part_scores[off] = lane < k ? ls : -INFINITY;
+      part_index[off] = lane < k ? li : INT_MAX;
+    }
+  }
+}
+
+template <int METRIC>
+static int launch_split_scan(const Maps &maps, const Args &a, int64_t items, cudaStream_t st) {
+  const int smem = Smem32::total(a.kc);
+  GFX_CUDA(cudaFuncSetAttribute(split_search_kernel<METRIC>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                232448));
+  const int grid = int(items < kNumSMs ? items : kNumSMs);
+  split_search_kernel<METRIC><<<grid, kWarps32 * 32, smem, st>>>(maps, a);
+  GFX_LAUNCH_CHECK();
+  return GFX_OK;
+}
+
+// search() for fp32 inputs
+template <int METRIC>
+static int search32(const Maps &maps, const Args &a, const Args &pre, const Plan &plan, const float *q,
+                    const float *db, int64_t Q, int64_t num_rows, int k, int64_t index_base,
+                    float *out_scores, int64_t *out_index, unsigned long long *fallbacks,
+                    const unsigned int *max_sqnorm, int32_t *flagged, cudaStream_t st) {
+  int rc = plan.sample_tiles ? launch_split_scan<METRIC>(maps, pre, plan.tiles_q, st) : GFX_OK;
+  if (!rc) rc = launch_split_scan<METRIC>(maps, a, plan.tiles_q * plan.segs, st);
+  if (rc) return rc;
+  const int finish_blocks = int((Q + kFinishWarps - 1) / kFinishWarps);
+  topk32_finish_kernel<METRIC><<<finish_blocks, kFinishWarps * 32, 0, st>>>(
+      q, db, a.part_scores, a.part_index, a.seed, max_sqnorm,
+      plan.segs, plan.qp, plan.kc, Q, k, index_base, out_scores, out_index, fallbacks, flagged);
+  GFX_LAUNCH_CHECK();
+  topk32_fallback_scan_kernel<METRIC><<<kNumSMs * kFbBlocksPerSM, kFbWarps * 32, 0, st>>>(
+      q, db, num_rows, plan.tiles_per_seg * kDbTile, plan.segs, plan.qp, plan.kc, k, fallbacks, flagged,
+      a.part_scores, a.part_index);
+  GFX_LAUNCH_CHECK();
+  topk_fallback_select_kernel<<<kNumSMs, kFinishWarps * 32, 0, st>>>(
+      a.part_scores, a.part_index, plan.segs, plan.qp, plan.kc, k, index_base, fallbacks, flagged,
+      out_scores, out_index);
+  GFX_LAUNCH_CHECK();
+  return GFX_OK;
+}
+
+static int split_rows(const float *x, int64_t rows, __half *image, cudaStream_t st) {
+  int64_t blocks = (rows * (kHidden / 4) + 255) / 256;
+  if (blocks > int64_t(kNumSMs) * 16) blocks = int64_t(kNumSMs) * 16;
+  split_rows_kernel<<<int(blocks), 256, 0, st>>>(x, rows, image);
+  GFX_LAUNCH_CHECK();
+  return GFX_OK;
+}
+
 }  // namespace topk
 }  // namespace gfx
 
@@ -831,4 +1356,93 @@ extern "C" int gfx_topk_merge(const float *in_scores, const int64_t *in_index, i
                                                                      num_queries, k, out_scores, out_index);
   GFX_LAUNCH_CHECK();
   return GFX_OK;
+}
+
+extern "C" int gfx_topk_f32_prepare(const float *database, int64_t num_rows, void *image, void *stream) {
+  if (num_rows < 0 || num_rows > int64_t(INT_MAX) - 256)
+    return fail(GFX_ERR_ARGUMENT, "gfx_topk_f32_prepare: bad sizes (rows per call must fit int32)");
+  if (num_rows == 0) return GFX_OK;
+  if (!database || !image) return fail(GFX_ERR_ARGUMENT, "gfx_topk_f32_prepare: null pointer");
+  if ((reinterpret_cast<uintptr_t>(database) | reinterpret_cast<uintptr_t>(image)) & 15)
+    return fail(GFX_ERR_ARGUMENT, "gfx_topk_f32_prepare: database and image must be 16-byte aligned");
+  cudaStream_t st = as_stream(stream);
+  StageScope scope(GFX_STAGE_TOPK, st, 1);
+  return topk::split_rows(database, num_rows, static_cast<__half *>(image), st);
+}
+
+extern "C" size_t gfx_topk_f32_workspace_bytes(int64_t num_queries, int64_t num_rows, int k) {
+  if (num_queries <= 0 || num_rows < 0 || k <= 0) return 256;
+  return topk::make_plan_f32(num_queries, num_rows, k).total;
+}
+
+extern "C" int gfx_topk_f32(const float *queries, int64_t num_queries, const float *database,
+                            const void *image, int64_t num_rows, int dim, int k, int metric,
+                            int64_t index_base, float *out_scores, int64_t *out_index, void *workspace,
+                            size_t workspace_bytes, void *stream) {
+  if (dim != kHidden) return fail(GFX_ERR_UNSUPPORTED, "gfx_topk_f32: kernels are specialised for dim = 128");
+  if (k < 1 || k > topk::kMaxK) return fail(GFX_ERR_ARGUMENT, "gfx_topk_f32: k must be in [1, 24]");
+  if (metric != 0 && metric != 1)
+    return fail(GFX_ERR_ARGUMENT, "gfx_topk_f32: metric must be 0 (cosine) or 1 (L2)");
+  if (num_queries < 0 || num_rows < 0 || num_rows > int64_t(INT_MAX) - 256)
+    return fail(GFX_ERR_ARGUMENT, "gfx_topk_f32: bad sizes (rows per call must fit int32)");
+  if (num_queries == 0) return GFX_OK;
+  if (!queries || !out_scores || !out_index || (num_rows > 0 && (!database || !image)))
+    return fail(GFX_ERR_ARGUMENT, "gfx_topk_f32: null pointer");
+  if ((reinterpret_cast<uintptr_t>(queries) | reinterpret_cast<uintptr_t>(database) |
+       reinterpret_cast<uintptr_t>(image)) & 15)
+    return fail(GFX_ERR_ARGUMENT, "gfx_topk_f32: queries, database and image must be 16-byte aligned");
+  topk::Plan plan = topk::make_plan_f32(num_queries, num_rows, k);
+  if (workspace_bytes < plan.total || !workspace)
+    return fail(GFX_ERR_WORKSPACE, "gfx_topk_f32: workspace too small");
+  cudaStream_t st = as_stream(stream);
+  char *ws = static_cast<char *>(workspace);
+  topk::Args a{};
+  a.part_scores = reinterpret_cast<float *>(ws + plan.off_scores);
+  a.part_index = reinterpret_cast<int32_t *>(ws + plan.off_index);
+  a.d2 = reinterpret_cast<float *>(ws + plan.off_d2);
+  a.tiles_q = plan.tiles_q; a.tiles_db = plan.tiles_db; a.segs = plan.segs;
+  a.tiles_per_seg = plan.tiles_per_seg; a.qp = plan.qp; a.num_rows = num_rows; a.kc = plan.kc;
+  const int finish_blocks = int((num_queries + topk::kFinishWarps - 1) / topk::kFinishWarps);
+  GFX_CUDA(cudaMemsetAsync(ws, 0, topk::kHeaderBytes, st));
+  if (num_rows == 0) {
+    StageScope scope(GFX_STAGE_TOPK, st, 1);
+    topk::topk_merge_kernel<<<finish_blocks, topk::kFinishWarps * 32, 0, st>>>(
+        nullptr, nullptr, 0, num_queries, k, out_scores, out_index);
+    GFX_LAUNCH_CHECK();
+    return GFX_OK;
+  }
+  __half *qimage = reinterpret_cast<__half *>(ws + plan.off_qimage);
+  topk::Maps maps;
+  int rc = tma::make_rows_map(&maps.q, qimage, num_queries, 2 * kHidden, topk::kQTile32);
+  if (!rc) rc = tma::make_rows_map(&maps.db, image, num_rows, 2 * kHidden, topk::kDbTile);
+  if (rc) return rc;
+  // query split, sqnorm, [pre-pass,] scan, finish, fallback scan, fallback select
+  StageScope scope(GFX_STAGE_TOPK, st, 6 + (plan.sample_tiles ? 1 : 0));
+  rc = topk::split_rows(queries, num_queries, qimage, st);
+  if (rc) return rc;
+  topk::Args pre = a;
+  if (plan.sample_tiles) {
+    pre.part_scores = reinterpret_cast<float *>(ws + plan.off_seed_scores);
+    pre.part_index = reinterpret_cast<int32_t *>(ws + plan.off_seed_index);
+    pre.tiles_db = pre.tiles_per_seg = plan.sample_tiles;
+    pre.segs = 1;
+    pre.num_rows = plan.sample_tiles * topk::kDbTile;
+    a.seed = pre.part_scores;
+  }
+  auto *fallbacks = reinterpret_cast<unsigned long long *>(ws + topk::kOffFallbacks);
+  auto *max_sqnorm = reinterpret_cast<unsigned int *>(ws + topk::kOffMaxSqNorm);
+  auto *flagged = reinterpret_cast<int32_t *>(ws + plan.off_flagged);
+  {
+    const int64_t padded = plan.tiles_db * topk::kDbTile;
+    int64_t blocks = (padded + 15) / 16;
+    if (blocks > int64_t(kNumSMs) * 8) blocks = int64_t(kNumSMs) * 8;
+    topk::row_sqnorm32_kernel<<<int(blocks), 256, 0, st>>>(database, num_rows, padded,
+                                                          const_cast<float *>(a.d2), max_sqnorm);
+    GFX_LAUNCH_CHECK();
+  }
+  return metric == 1
+      ? topk::search32<1>(maps, a, pre, plan, queries, database, num_queries, num_rows, k, index_base,
+                          out_scores, out_index, fallbacks, max_sqnorm, flagged, st)
+      : topk::search32<0>(maps, a, pre, plan, queries, database, num_queries, num_rows, k, index_base,
+                          out_scores, out_index, fallbacks, max_sqnorm, flagged, st);
 }

@@ -371,12 +371,33 @@ int gfx_encode_described_f32(const gfx_model *model, const float *x,
  * with many near-duplicates of a query's best rows, pays for that fallback.
  * The first 8 bytes of the workspace hold, after the call, the number of
  * queries that took it (int64).
+ *
+ * float32 inputs (the encoder's full_precision output): gfx_topk_f32 has the
+ * same contract over float32 queries and rows -- scores are the sequential
+ * fp32 FMA chain over the fp32 values (L2: the difference in fp32, squared by
+ * FMA), same order, padding, certificate-and-fallback and workspace header.
+ * Its scan multiplies the split-fp16 images x = hi + lo, hi = fp16(x),
+ * lo = fp16(x - hi): three fp16 MMAs per K step (hi.hi + hi.lo + lo.hi), so
+ * its margin is 2^-13 |q| N_max + 2^-21 (|q| + N_max) (L2:
+ * 2^-13 (2 |q| N_max + N_max^2 + |q|^2) + 2^-20 (|q| + N_max)).
+ * gfx_topk_f32_prepare writes the database's [rows, 256] fp16 image hi | lo
+ * once (`image`: rows * 512 bytes, 16-byte aligned); every row component
+ * must be at most 65504 in magnitude (the fp16 range of hi).  A query
+ * component above that is allowed: the query takes the exact fallback.
+ * The queries' image is built per call in the workspace.
  * ------------------------------------------------------------------------ */
 size_t gfx_topk_workspace_bytes(int64_t num_queries, int64_t num_rows, int k);
 int gfx_topk(const void *queries, int64_t num_queries, const void *database,
              int64_t num_rows, int dim, int k, int metric, int64_t index_base,
              float *out_scores, int64_t *out_index, void *workspace,
              size_t workspace_bytes, void *stream);
+int gfx_topk_f32_prepare(const float *database, int64_t num_rows, void *image,
+                         void *stream);
+size_t gfx_topk_f32_workspace_bytes(int64_t num_queries, int64_t num_rows, int k);
+int gfx_topk_f32(const float *queries, int64_t num_queries, const float *database,
+                 const void *image, int64_t num_rows, int dim, int k, int metric,
+                 int64_t index_base, float *out_scores, int64_t *out_index,
+                 void *workspace, size_t workspace_bytes, void *stream);
 
 /* k-way merge of `parts` per-query sorted lists (all-gathered from the
  * ranks) into the global top-k: in_* are [parts, Q, k]. */

@@ -406,6 +406,46 @@ int gfx_topk_merge(const float *in_scores, const int64_t *in_index, int parts,
                    int64_t *out_index, void *stream);
 
 /* ------------------------------------------------------------------------
+ * K8  local alignment of embedding segments (Smith-Waterman, affine gaps;
+ * no reference counterpart: the reference ships parameters for an external
+ * aligner, api.py:47-50, and this contract is the library's own).
+ * queries [q_rows,128], targets [t_rows,128]: GFX_F16 row-major tables (may
+ * be the same).  pairs int64 [P,4]: (q_start, q_len, t_start, t_len), rows
+ * q_start .. q_start+q_len-1 of queries against t_start .. of targets, each
+ * length 0..4096 and inside its table.  For query row i and target row j of a
+ * pair, every operation fp32 round-to-nearest, in this order:
+ *   S(i,j) = q_i . t_j     tcgen05.mma: fp16 inputs, fp32 accumulation
+ *   s      = S(i,j) - offset
+ *   E(i,j) = max(H(i,j-1) - gap_open, E(i,j-1) - gap_extend)   gap in the query
+ *   F(i,j) = max(H(i-1,j) - gap_open, F(i-1,j) - gap_extend)   gap in the target
+ *   H(i,j) = max(0, H(i-1,j-1) + s, E(i,j), F(i,j))
+ *   H(-1,.) = H(.,-1) = 0,  E(.,-1) = F(-1,.) = -inf
+ * Ties: a positive H takes its start from the first of diagonal, E, F that
+ * attains it; a diagonal step from H = 0 starts at (i,j), otherwise the start
+ * is inherited; E and F prefer opening to extending; the end cell is the
+ * largest H, then the smallest i, then the smallest j.
+ * Output: out_score float32 [P] (the largest H); out_coords int32 [P,4] =
+ * (query_begin, query_end, target_begin, target_end), half-open, relative to
+ * the segments.  No positive cell (zero-length segments included): score 0,
+ * coordinates -1.  A pair outside these limits gets score NaN and -1 (the
+ * kernel reads nothing for it); callers validate.
+ * Accuracy: |S - exact| <= 2^-14 |q_i| |t_j| (kAlignRel in gfx_align.cu), so the
+ * score is within min(q_len, t_len) 2^-14 max|q| max|t| of the float64
+ * optimum, plus (q_len + t_len) fp32 additions at 2^-24 relative.  A pair's
+ * result does not depend on the rest of the batch or on table offsets.
+ * gap_open, gap_extend > 0 and offset finite, else GFX_ERR_ARGUMENT; table
+ * components must be finite (not checked here).
+ * Workspace: gfx_align_workspace_bytes(P, m) serves every pair whose t_len is
+ * at most m among those with q_len > 128 (the others need none).
+ * ------------------------------------------------------------------------ */
+size_t gfx_align_workspace_bytes(int64_t num_pairs, int64_t max_t_len);
+int gfx_align(const void *queries, int64_t q_rows, const void *targets,
+              int64_t t_rows, const int64_t *pairs, int64_t num_pairs,
+              float offset, float gap_open, float gap_extend, float *out_score,
+              int32_t *out_coords, void *workspace, size_t workspace_bytes,
+              void *stream);
+
+/* ------------------------------------------------------------------------
  * Instrumentation (used by bench.py; no effect on results).
  * Every kernel launch made by this library is counted per stage.  When a
  * stage's bit is set in the profile mask, each call of that stage is
@@ -423,7 +463,8 @@ enum {
   GFX_STAGE_FUSED_LAYER = 7,
   GFX_STAGE_TOPK = 8,
   GFX_STAGE_BUILD = 9,
-  GFX_NUM_STAGES = 10
+  GFX_STAGE_ALIGN = 10,
+  GFX_NUM_STAGES = 11
 };
 int gfx_profile_enable(uint32_t stage_mask);
 int gfx_profile_read(int stage, double *total_ms, int64_t *timed_calls, int reset);

@@ -1,20 +1,33 @@
-// K5  similarity search: per-query top-k of a [Q,128] fp16 query set against a
-// [D,128] fp16 embedding database (cosine = dot product of unit vectors, or
-// negative squared L2 distance).  No reference counterpart (north-star item 4).
+// K5  similarity search: per-query top-k of a [Q,128] query set against a
+// [D,128] embedding database of fp16 rows (gfx_topk) or fp32 rows (gfx_topk_f32)
+// (cosine = dot product of unit vectors, or negative squared L2 distance).  No
+// reference counterpart (north-star item 4).
 //
-//   scan    tcgen05 GEMM  S = Q_tile(256) x DB_tile(128)^T  with the running
-//           top-k fused into the TMEM epilogue: the score matrix never exists
-//           in memory.  One persistent CTA per SM; a work item is (query tile,
-//           database segment).  Warps: 0-7 epilogue (one query per thread),
-//           8 MMA issuer, 9 TMA loader.  Database tiles stream through a
-//           3-stage TMA ring (the same tile is read by every resident CTA at
-//           about the same time, so all but the first read hit L2); the 256
-//           queries of the item stay in shared memory; accumulators are
-//           double-buffered in TMEM (2 x 2 x 128 columns).
-//   finish  exact re-scoring of the surviving candidates (sequential fp32 FMA
-//           in dimension order: reproducible and restatable on the CPU),
-//           selection of the k best by (score desc, index asc), and a
-//           certificate per query (below).
+//   scan    tcgen05 GEMM  S = Q_tile x DB_tile(128)^T  with the running top-k
+//           fused into the TMEM epilogue: the score matrix never exists in
+//           memory.  One persistent CTA per SM; a work item is (query tile,
+//           database segment).  Warps: epilogue (one query per thread), then the
+//           MMA issuer and the TMA loader.  Database tiles stream through a TMA
+//           ring (the same tile is read by every resident CTA at about the same
+//           time, so all but the first read hit L2); the queries of the item
+//           stay in shared memory; accumulators are double-buffered in TMEM.
+//           Two configurations of the same code:
+//             F16Scan    fp16 rows (topk_scan_kernel): 256-query tiles, 8 epilogue warps, 3 stages,
+//                        TMEM 2 x 2 x 128 columns, one MMA per K step.
+//             SplitScan  fp32 rows (split_search_kernel): the operands are split-fp16 images,
+//                        x = hi + lo, hi = fp16(x), lo = fp16(x - hi) (the split
+//                        of gfx_split9.cu), [rows, 256] = hi | lo; per K step
+//                        three kind::f16 MMAs, hi.hi + hi.lo + lo.hi, into one
+//                        fp32 accumulator.  The database image is built once per
+//                        index (gfx_topk_f32_prepare), the queries' per call in
+//                        the workspace.  Hi and lo need twice the shared memory,
+//                        so a work item holds 128 queries: queries 64 KB |
+//                        2 stages x 64 KB | |d|^2 slots 4 KB | lists <= 28 KB =
+//                        224 KB; 4 epilogue warps; TMEM 2 x 128 columns.
+//   finish  exact re-scoring of the surviving candidates from the rows as given
+//           (sequential fp32 FMA in dimension order: reproducible and restatable
+//           on the CPU), selection of the k best by (score desc, index asc), and
+//           a certificate per query (below).
 //   fallback  for the queries whose certificate fails: an exact scan of the
 //           whole database (the same FMA chain for every row) and the same
 //           selection.  Launched unconditionally; its grid reads the number
@@ -33,7 +46,8 @@
 #include <limits.h>
 #include <math.h>
 
-#include <cstdlib>
+#include <string>
+#include <type_traits>
 
 #include "gfx_common.cuh"
 #include "gfx_tma.cuh"
@@ -44,31 +58,92 @@ namespace topk {
 
 using namespace ptx;
 
-constexpr int kQTile = 256, kDbTile = 128, kStages = 3;
-constexpr int kBoxBytes = 128 * 128;              // [128 rows x 64 cols] fp16
-constexpr int kQBytes = 4 * kBoxBytes;            // 2 row blocks x 2 K blocks
-constexpr int kDbBytes = 2 * kBoxBytes;
-constexpr int kEpiWarps = 8, kMmaWarp = 8, kLoadWarp = 9, kWarps = 10;
+constexpr int kDbTile = 128;
+constexpr int kBoxBytes = 128 * 128;              // [128 rows x 64 cols] fp16: one TMA box
 constexpr int kD2Slots = 8;                       // loader runs <= 5 tiles ahead of the epilogue
 constexpr int kMaxCand = 28, kMaxK = 24;
 constexpr int kWaves = 8;                         // work items per CTA aimed for
 constexpr int kSampleTiles = 128;                 // database tiles of the threshold-seeding pre-pass
 
-enum Bar {
-  kBarQFull = 0, kBarQEmpty = 1, kBarBFull = 2, kBarBEmpty = 5, kBarDFull = 8, kBarDEmpty = 10,
-  kNumBars = 12
-};
-
-struct Smem {
+// Compile-time shape of a scan over rows of type ROW.  The MMA operands are fp16
+// images of kParts x 64-column K blocks per row: the rows themselves (fp16), or
+// hi | lo (fp32, kParts = 2).  Box (row block rb, part p, K block kb) holds
+// image columns [(p * 2 + kb) * 64, +64) of rows [qt * kQTile + rb * 128, +128)
+// and sits in shared memory at box index (rb * kParts + p) * 2 + kb; a database
+// tile is one row block.
+template <typename ROW, int QTILE, int STAGES>
+struct ScanShape {
+  using Row = ROW;
+  static constexpr bool kSplit = std::is_same<ROW, float>::value;
+  static constexpr int kQTile = QTILE, kStages = STAGES;
+  static constexpr int kParts = kSplit ? 2 : 1, kCols = kParts * kHidden;
+  static constexpr int kRowBlocks = QTILE / 128;
+  static constexpr int kTerms = kSplit ? 3 : 1;     // MMAs per K step: hi.hi [, hi.lo, lo.hi]
+  static constexpr int kQBoxes = kRowBlocks * kParts * 2, kDbBoxes = kParts * 2;
+  static constexpr int kQBytes = kQBoxes * kBoxBytes, kDbBytes = kDbBoxes * kBoxBytes;
+  static constexpr int kAccCols = kRowBlocks * 128; // TMEM columns of one of the two accumulators
+  static constexpr int kEpiWarps = QTILE / 32, kMmaWarp = kEpiWarps, kLoadWarp = kEpiWarps + 1,
+                       kWarps = kEpiWarps + 2;
+  // barriers
+  static constexpr int kBarQFull = 0, kBarQEmpty = 1, kBarBFull = 2, kBarBEmpty = kBarBFull + STAGES,
+                       kBarDFull = kBarBEmpty + STAGES, kBarDEmpty = kBarDFull + 2, kNumBars = kBarDEmpty + 2;
+  // dynamic shared memory
   static constexpr int off_q = 0;
   static constexpr int off_db = off_q + kQBytes;
-  static constexpr int off_d2 = off_db + kStages * kDbBytes;
+  static constexpr int off_d2 = off_db + STAGES * kDbBytes;
   static constexpr int off_bar = off_d2 + kD2Slots * kDbTile * 4;
   static constexpr int off_tmem = off_bar + kNumBars * 8;
   static constexpr int off_list = (off_tmem + 8 + 15) & ~15;
-  static constexpr int total(int kc) { return off_list + kc * kQTile * 8; }   // per-thread sorted lists
+  static constexpr int smem_bytes(int kc) { return off_list + kc * QTILE * 8; }   // per-thread sorted lists
 };
-static_assert(Smem::total(kMaxCand) <= 232448, "exceeds the 227 KB shared-memory limit of sm_100");
+
+// Certificate margin of the fp16 scan, relative: eps = 2^-14 |q| N_max (cosine) or
+// 2^-14 (2 |q| N_max + N_max^2 + |q|^2) (L2, the scan's frame), N_max the
+// largest row norm.  It has to cover the exact chain's error plus the tensor
+// cores' error on the same dot product.  The sequential chain of 128 FMAs is
+// within 128 * 2^-24 * sum|q_i x_i| = 2^-17 sum|q_i x_i| of the real value.
+// Published measurements of fp16-input, fp32-accumulate tensor cores on earlier
+// NVIDIA generations show an accumulator that truncates, about 2^-23 per
+// addition, which over 128 products is 2^-16 sum|q_i x_i|; and
+// sum|q_i x_i| <= |q| N_max (for L2 the terms of 2 q.d - |d|^2 and |q|^2 add
+// the other two parts).  2^-14 leaves a margin of at least 4x over the sum.
+// The B200's accumulator has not been measured: this constant rests on that
+// argument, not on a measurement.
+struct F16Scan : ScanShape<__half, 256, 3> {
+  static constexpr float kCertRel = 1.f / 16384.f;
+};
+
+// Certificate margin of the split scan:
+//   cosine  eps = kCertRel |q| N_max + kCertAbs (|q| + N_max)
+//   L2      eps = kCertRel (2 |q| N_max + N_max^2 + |q|^2) + 2 kCertAbs (|q| + N_max)
+// (the scan's frame, as F16Scan).  Against the real dot product R = sum q_i x_i:
+//  * the split.  With fp16 hi and lo normal, q_i = qh_i + ql_i + e_i, |e_i| <= 2^-22 |q_i|
+//    (hi is within 2^-11 |q_i|, lo within 2^-11 of the rest), and the same for x.  The scan
+//    sums qh.xh + qh.xl + ql.xh = (q - e_q).(x - e_x) - ql.xl; with |ql_i| <= 2^-11 (1 + 2^-11)
+//    |q_i| that is within (3 + 2^-9) 2^-22 < 2^-20 of sum |q_i x_i| from R, the dropped lo.lo
+//    term included;
+//  * subnormals.  Where x_i - hi_i (or x_i itself) is below 2^-14, lo (or hi) is rounded onto
+//    the fp16 subnormal grid of spacing 2^-24: an absolute error of at most 2^-25 per
+//    component, which sums to 2^-25 (|q|_1 + |x|_1) <= 2^-25 sqrt(128) (|q| + N_max)
+//    < 2^-21 (|q| + N_max) = kCertAbs (|q| + N_max).  This assumes that kind::f16 takes
+//    subnormal fp16 operands at their value; an MMA that flushed them would lose up to 2^-14
+//    per component;
+//  * the tensor-core accumulator.  3 x 128 products go into one fp32 accumulator; on the
+//    truncation argument of F16Scan (about 2^-23 per addition) that is within
+//    384 x 2^-23 (1 + 2^-10) < 2^-14.4 of sum |q_i x_i|;
+//  * the exact chain: within 2^-17 sum |q_i x_i| (F16Scan).  For L2 the fp32 difference
+//    q_i - x_i adds 2^-23 relative per term of sum (q_i - x_i)^2 <= (|q| + N_max)^2.
+// The sum is below 2^-14.1 sum |q_i x_i| <= 2^-14.1 |q| N_max; 2^-13 leaves more than 2x
+// (for L2, 2 q.d doubles the first and the |d|^2, |q|^2 and chain errors, each <= 2^-16.9 of
+// their square, stay inside the other terms).  As for F16Scan, the B200's accumulator has not
+// been measured: this margin rests on the argument, not on a measurement.  Without the split
+// (a scan of fp16(x) only) the rounding of the inputs alone is 2^-11 sum |q_i x_i| per side.
+struct SplitScan : ScanShape<float, 128, 2> {
+  static constexpr float kCertRel = 1.f / 8192.f, kCertAbs = 1.f / 2097152.f;
+};
+
+static_assert(F16Scan::smem_bytes(kMaxCand) <= 232448, "exceeds the 227 KB shared-memory limit of sm_100");
+static_assert(SplitScan::smem_bytes(kMaxCand) <= 232448, "exceeds the 227 KB shared-memory limit of sm_100");
 
 struct alignas(64) Maps {
   CUtensorMap q, db;
@@ -85,15 +160,15 @@ struct Plan {
   int kc;
   int64_t sample_tiles;       // 0 = no seeding pre-pass
   size_t off_flagged, off_scores, off_index, off_d2, off_seed_scores, off_seed_index, total;
-  size_t off_qimage;          // fp32 search: [Q, 256] hi | lo image of the queries
+  size_t off_qimage;          // split scan: [Q, 256] hi | lo image of the queries
 };
 
-// `q_tile`: queries per work item of the scan (kQTile; kQTile32 for fp32 inputs)
-static Plan make_plan(int64_t Q, int64_t D, int k, int q_tile = kQTile) {
+template <class Cfg>
+static Plan make_plan(int64_t Q, int64_t D, int k) {
   Plan p{};
-  p.tiles_q = (Q + q_tile - 1) / q_tile;
+  p.tiles_q = (Q + Cfg::kQTile - 1) / Cfg::kQTile;
   p.tiles_db = (D + kDbTile - 1) / kDbTile;
-  p.qp = p.tiles_q * q_tile;
+  p.qp = p.tiles_q * Cfg::kQTile;
   int64_t segs = 1;
   if (p.tiles_q > 0 && p.tiles_q < int64_t(kWaves) * kNumSMs)
     segs = (int64_t(kWaves) * kNumSMs + p.tiles_q - 1) / p.tiles_q;
@@ -115,6 +190,10 @@ static Plan make_plan(int64_t Q, int64_t D, int k, int q_tile = kQTile) {
   p.off_seed_scores = p.total;
   p.off_seed_index = p.off_seed_scores + up(size_t(p.qp) * p.kc * 4);
   if (p.sample_tiles) p.total = p.off_seed_index + up(size_t(p.qp) * p.kc * 4);
+  if (Cfg::kSplit) {
+    p.off_qimage = p.total;
+    p.total += up(size_t(Q) * Cfg::kCols * 2);
+  }
   return p;
 }
 
@@ -132,20 +211,21 @@ struct Args {
 };
 
 // Insert (v, idx) into the thread's descending list (column `ls`/`li`, stride
-// kQTile).  Strict comparisons: among equal scores the earlier (lower) index
-// stays ahead.  Returns the new threshold (the list's last score).  (An
-// unsorted set with a tracked eviction slot was tried: its full rescan per
-// insert costs more than the average shift here.)
+// STRIDE = the scan's query tile).  Strict comparisons: among equal scores the
+// earlier (lower) index stays ahead.  Returns the new threshold (the list's last
+// score).  (An unsorted set with a tracked eviction slot was tried: its full
+// rescan per insert costs more than the average shift here.)
+template <int STRIDE>
 __device__ __noinline__ float list_insert(float *ls, int32_t *li, int kc, float v, int32_t idx) {
   int j = kc - 1;
-  while (j > 0 && ls[(j - 1) * kQTile] < v) {
-    ls[j * kQTile] = ls[(j - 1) * kQTile];
-    li[j * kQTile] = li[(j - 1) * kQTile];
+  while (j > 0 && ls[(j - 1) * STRIDE] < v) {
+    ls[j * STRIDE] = ls[(j - 1) * STRIDE];
+    li[j * STRIDE] = li[(j - 1) * STRIDE];
     --j;
   }
-  ls[j * kQTile] = v;
-  li[j * kQTile] = idx;
-  return ls[(kc - 1) * kQTile];
+  ls[j * STRIDE] = v;
+  li[j * STRIDE] = idx;
+  return ls[(kc - 1) * STRIDE];
 }
 
 // Threshold a scan starts from, given the kc-th score of the seeding sample:
@@ -158,10 +238,10 @@ __device__ __forceinline__ float max3(float a, float b, float c) {
   return r;
 }
 
-template <int METRIC>
-__global__ void __launch_bounds__(kWarps * 32, 1)
-topk_scan_kernel(const __grid_constant__ Maps maps, const Args p) {
-  using L = Smem;
+// The scan, for the entry points below.
+template <class Cfg, int METRIC>
+__device__ __forceinline__ void scan(const Maps &maps, const Args &p) {
+  using L = Cfg;
   extern __shared__ __align__(1024) uint8_t smem[];
   uint8_t *qs = smem + L::off_q, *dbs = smem + L::off_db;
   float *d2s = reinterpret_cast<float *>(smem + L::off_d2);
@@ -169,19 +249,22 @@ topk_scan_kernel(const __grid_constant__ Maps maps, const Args p) {
   uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(smem + L::off_tmem);
   float *list_s = reinterpret_cast<float *>(smem + L::off_list);
 
+  // The entry point's __launch_bounds__ bounds threadIdx.x only inside the kernel's
+  // own body; stated here too, the warp-role arithmetic compiles as it would there.
+  __builtin_assume(threadIdx.x < L::kWarps * 32);
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  if (warp == kMmaWarp) {
-    tmem_alloc(tmem_slot, 512);
+  if (warp == L::kMmaWarp) {
+    tmem_alloc(tmem_slot, 2 * L::kAccCols);
   } else if (tid == 0) {
-    mbar_init(bar + kBarQFull, 1);
-    mbar_init(bar + kBarQEmpty, 1);
-    for (int s = 0; s < kStages; ++s) {
-      mbar_init(bar + kBarBFull + s, 1);
-      mbar_init(bar + kBarBEmpty + s, 1);
+    mbar_init(bar + L::kBarQFull, 1);
+    mbar_init(bar + L::kBarQEmpty, 1);
+    for (int s = 0; s < L::kStages; ++s) {
+      mbar_init(bar + L::kBarBFull + s, 1);
+      mbar_init(bar + L::kBarBEmpty + s, 1);
     }
     for (int a = 0; a < 2; ++a) {
-      mbar_init(bar + kBarDFull + a, 1);
-      mbar_init(bar + kBarDEmpty + a, kEpiWarps);
+      mbar_init(bar + L::kBarDFull + a, 1);
+      mbar_init(bar + L::kBarDEmpty + a, L::kEpiWarps);
     }
     fence_mbar_init();
   }
@@ -191,49 +274,50 @@ topk_scan_kernel(const __grid_constant__ Maps maps, const Args p) {
   const uint32_t tmem = *tmem_slot;
   const int64_t items = p.tiles_q * p.segs;
 
-  if (warp == kLoadWarp) {
+  if (warp == L::kLoadWarp) {
     // ================================ TMA loader =================================
     // (whole warp in the loop, one elected lane issues: see the MMA issuer below)
-    {
-      uint32_t elected;
-      asm volatile("{\n.reg .pred q;\nelect.sync _|q, 0xffffffff;\nselp.u32 %0, 1, 0, q;\n}" : "=r"(elected));
-      const bool issuer = elected != 0u;
+    uint32_t elected;
+    asm volatile("{\n.reg .pred q;\nelect.sync _|q, 0xffffffff;\nselp.u32 %0, 1, 0, q;\n}" : "=r"(elected));
+    const bool issuer = elected != 0u;
+    if (issuer) {
+      prefetch_tmap(&maps.q);
+      prefetch_tmap(&maps.db);
+    }
+    uint32_t it = 0, item_n = 0;
+    for (int64_t item = blockIdx.x; item < items; item += gridDim.x, ++item_n) {
+      const int64_t qt = item % p.tiles_q, seg = item / p.tiles_q;
+      mbar_wait(bar + L::kBarQEmpty, (item_n & 1) ^ 1);
       if (issuer) {
-        prefetch_tmap(&maps.q);
-        prefetch_tmap(&maps.db);
-      }
-      uint32_t it = 0, item_n = 0;
-      for (int64_t item = blockIdx.x; item < items; item += gridDim.x, ++item_n) {
-        const int64_t qt = item % p.tiles_q, seg = item / p.tiles_q;
-        mbar_wait(bar + kBarQEmpty, (item_n & 1) ^ 1);
-        if (issuer) {
-          mbar_arrive_expect_tx(bar + kBarQFull, kQBytes);
+        mbar_arrive_expect_tx(bar + L::kBarQFull, L::kQBytes);
 #pragma unroll
-          for (int b = 0; b < 4; ++b)
-            tma_load_2d(qs + b * kBoxBytes, &maps.q, (b & 1) * 64, int(qt * kQTile + (b >> 1) * 128),
-                        bar + kBarQFull);
+        for (int b = 0; b < L::kQBoxes; ++b) {        // b = (rb * kParts + p) * 2 + kb
+          const int rb = b / (2 * L::kParts), pk = b % (2 * L::kParts);
+          tma_load_2d(qs + b * kBoxBytes, &maps.q, pk * 64, int(qt * L::kQTile + rb * 128),
+                      bar + L::kBarQFull);
+        }
+      }
+      __syncwarp();
+      const int64_t t0 = seg * p.tiles_per_seg;
+      const int64_t t1 = t0 + p.tiles_per_seg < p.tiles_db ? t0 + p.tiles_per_seg : p.tiles_db;
+      for (int64_t t = t0; t < t1; ++t, ++it) {
+        const uint32_t s = it % L::kStages, ph = (it / L::kStages) & 1;
+        uint8_t *dst = dbs + s * L::kDbBytes;
+        mbar_wait(bar + L::kBarBEmpty + s, ph ^ 1);
+        if (issuer) {
+          mbar_arrive_expect_tx(bar + L::kBarBFull + s, L::kDbBytes + (METRIC == 1 ? kDbTile * 4 : 0));
+#pragma unroll
+          for (int b = 0; b < L::kDbBoxes; ++b)
+            tma_load_2d(dst + b * kBoxBytes, &maps.db, b * 64, int(t * kDbTile), bar + L::kBarBFull + s);
+          if (METRIC == 1)
+            bulk_g2s(d2s + (it % kD2Slots) * kDbTile, p.d2 + t * kDbTile, kDbTile * 4,
+                     bar + L::kBarBFull + s);
         }
         __syncwarp();
-        const int64_t t0 = seg * p.tiles_per_seg;
-        const int64_t t1 = t0 + p.tiles_per_seg < p.tiles_db ? t0 + p.tiles_per_seg : p.tiles_db;
-        for (int64_t t = t0; t < t1; ++t, ++it) {
-          const uint32_t s = it % kStages, ph = (it / kStages) & 1;
-          uint8_t *dst = dbs + s * kDbBytes;
-          mbar_wait(bar + kBarBEmpty + s, ph ^ 1);
-          if (issuer) {
-            mbar_arrive_expect_tx(bar + kBarBFull + s, kDbBytes + (METRIC == 1 ? kDbTile * 4 : 0));
-            tma_load_2d(dst, &maps.db, 0, int(t * kDbTile), bar + kBarBFull + s);
-            tma_load_2d(dst + kBoxBytes, &maps.db, 64, int(t * kDbTile), bar + kBarBFull + s);
-            if (METRIC == 1)
-              bulk_g2s(d2s + (it % kD2Slots) * kDbTile, p.d2 + t * kDbTile, kDbTile * 4,
-                       bar + kBarBFull + s);
-          }
-          __syncwarp();
-        }
       }
     }
     __syncwarp();
-  } else if (warp == kMmaWarp) {
+  } else if (warp == L::kMmaWarp) {
     // ================================ MMA issuer =================================
     // The whole warp runs the loop and waits on the barriers; one elected lane issues.  Issued
     // from inside `if (lane == 0)` the operands of every MMA were ordinary registers to the
@@ -241,54 +325,58 @@ topk_scan_kernel(const __grid_constant__ Maps maps, const Args p) {
     // (11-13 instructions per MMA on a warp that shares its scheduler with epilogue warps: more
     // than the 64 cycles an MMA of this shape takes); with warp-uniform operands they live in
     // uniform registers (measured on the fused layer kernel, DESIGN.md section 9.1).
-    {
-      constexpr uint32_t idesc = idesc_f16(128, kDbTile);
-      const uint32_t qa = smem_u32(qs), ba = smem_u32(dbs);
-      const uint32_t tm = __shfl_sync(0xffffffffu, tmem, 0);
-      uint32_t elected;
-      asm volatile("{\n.reg .pred q;\nelect.sync _|q, 0xffffffff;\nselp.u32 %0, 1, 0, q;\n}" : "=r"(elected));
-      const bool issuer = elected != 0u;
-      uint32_t it = 0, item_n = 0;
-      for (int64_t item = blockIdx.x; item < items; item += gridDim.x, ++item_n) {
-        const int64_t seg = item / p.tiles_q;
-        const int64_t t0 = seg * p.tiles_per_seg;
-        const int64_t t1 = t0 + p.tiles_per_seg < p.tiles_db ? t0 + p.tiles_per_seg : p.tiles_db;
-        mbar_wait(bar + kBarQFull, item_n & 1);
-        for (int64_t t = t0; t < t1; ++t, ++it) {
-          const uint32_t s = it % kStages, ph = (it / kStages) & 1, a = it & 1, pha = (it >> 1) & 1;
-          mbar_wait(bar + kBarBFull + s, ph);
-          mbar_wait(bar + kBarDEmpty + a, pha ^ 1);
-          tc_fence_after();
-          if (issuer) {
+    constexpr uint32_t idesc = idesc_f16(128, kDbTile);
+    const uint32_t qa = smem_u32(qs), ba = smem_u32(dbs);
+    const uint32_t tm = __shfl_sync(0xffffffffu, tmem, 0);
+    uint32_t elected;
+    asm volatile("{\n.reg .pred q;\nelect.sync _|q, 0xffffffff;\nselp.u32 %0, 1, 0, q;\n}" : "=r"(elected));
+    const bool issuer = elected != 0u;
+    uint32_t it = 0, item_n = 0;
+    for (int64_t item = blockIdx.x; item < items; item += gridDim.x, ++item_n) {
+      const int64_t seg = item / p.tiles_q;
+      const int64_t t0 = seg * p.tiles_per_seg;
+      const int64_t t1 = t0 + p.tiles_per_seg < p.tiles_db ? t0 + p.tiles_per_seg : p.tiles_db;
+      mbar_wait(bar + L::kBarQFull, item_n & 1);
+      for (int64_t t = t0; t < t1; ++t, ++it) {
+        const uint32_t s = it % L::kStages, ph = (it / L::kStages) & 1, a = it & 1, pha = (it >> 1) & 1;
+        mbar_wait(bar + L::kBarBFull + s, ph);
+        mbar_wait(bar + L::kBarDEmpty + a, pha ^ 1);
+        tc_fence_after();
+        if (issuer) {
 #pragma unroll
-            for (int half = 0; half < 2; ++half) {
+          for (int rb = 0; rb < L::kRowBlocks; ++rb) {
 #pragma unroll
-              for (int kk = 0; kk < 8; ++kk) {
-                const int kb = kk >> 2, k = kk & 3;
-                const uint64_t da = smem_desc_sw128(qa + (half * 2 + kb) * kBoxBytes + k * 32);
-                const uint64_t db = smem_desc_sw128(ba + s * kDbBytes + kb * kBoxBytes + k * 32);
-                mma_f16_ss(tm + a * 256 + half * 128, da, db, idesc, kk != 0);
+            for (int kk = 0; kk < 8; ++kk) {
+              const int kb = kk >> 2, k = kk & 3;
+#pragma unroll
+              for (int term = 0; term < L::kTerms; ++term) {   // hi.hi, hi.lo, lo.hi
+                const int qpart = term == 2, dpart = term == 1;
+                const uint64_t da = smem_desc_sw128(qa + ((rb * L::kParts + qpart) * 2 + kb) * kBoxBytes + k * 32);
+                const uint64_t db = smem_desc_sw128(ba + s * L::kDbBytes + (dpart * 2 + kb) * kBoxBytes + k * 32);
+                mma_f16_ss(tm + a * L::kAccCols + rb * 128, da, db, idesc, (kk | term) != 0);
               }
             }
-            mma_commit(bar + kBarBEmpty + s);
-            mma_commit(bar + kBarDFull + a);
           }
-          __syncwarp();
+          mma_commit(bar + L::kBarBEmpty + s);
+          mma_commit(bar + L::kBarDFull + a);
         }
-        if (issuer) mma_commit(bar + kBarQEmpty);   // every MMA reading this item's queries is done
         __syncwarp();
       }
+      if (issuer) mma_commit(bar + L::kBarQEmpty);   // every MMA reading this item's queries is done
+      __syncwarp();
     }
     __syncwarp();
   } else {
     // ============ epilogue: running top-k, one query per thread ====================
+    // A warp reads TMEM lanes 32 (warp % 4) .. +31 (the tcgen05 lane-access rule);
+    // with two row blocks, warps 4-7 take the second one's columns.
     const int quad = warp & 3, half = warp >> 2;
     const int row = half * 128 + quad * 32 + lane;          // query inside the item
     const uint32_t tbase = tmem + (uint32_t(quad * 32) << 16) + half * 128;
     const int kc = p.kc;
     const int32_t rows = int32_t(p.num_rows);
     float *ls = list_s + tid;
-    int32_t *li = reinterpret_cast<int32_t *>(list_s + kc * kQTile) + tid;
+    int32_t *li = reinterpret_cast<int32_t *>(list_s + kc * L::kQTile) + tid;
     const float ninf = -INFINITY;
     uint32_t it = 0;
     for (int64_t item = blockIdx.x; item < items; item += gridDim.x) {
@@ -296,24 +384,24 @@ topk_scan_kernel(const __grid_constant__ Maps maps, const Args p) {
       const int64_t t0 = seg * p.tiles_per_seg;
       const int64_t t1 = t0 + p.tiles_per_seg < p.tiles_db ? t0 + p.tiles_per_seg : p.tiles_db;
       for (int j = 0; j < kc; ++j) {
-        ls[j * kQTile] = ninf;
-        li[j * kQTile] = INT_MAX;
+        ls[j * L::kQTile] = ninf;
+        li[j * L::kQTile] = INT_MAX;
       }
       float seed = ninf;
       if (p.seed)                                   // kc-th best of the sample (lists are sorted)
-        seed = seed_threshold(p.seed[(size_t(qt) * kQTile + row) * kc + kc - 1]);
+        seed = seed_threshold(p.seed[(size_t(qt) * L::kQTile + row) * kc + kc - 1]);
       float thr = seed;
       for (int64_t t = t0; t < t1; ++t, ++it) {
         const uint32_t a = it & 1, pha = (it >> 1) & 1;
-        mbar_wait(bar + kBarDFull + a, pha);
+        mbar_wait(bar + L::kBarDFull + a, pha);
         tc_fence_after();
         float v[kDbTile];
 #pragma unroll
-        for (int cb = 0; cb < 4; ++cb) tmem_ld32(tbase + a * 256 + cb * 32, v + cb * 32);
+        for (int cb = 0; cb < 4; ++cb) tmem_ld32(tbase + a * L::kAccCols + cb * 32, v + cb * 32);
         tmem_ld_wait();
         tc_fence_before();
         __syncwarp();
-        if (lane == 0) mbar_arrive(bar + kBarDEmpty + a);   // accumulator is in registers now
+        if (lane == 0) mbar_arrive(bar + L::kBarDEmpty + a);   // accumulator is in registers now
         const int32_t base = int32_t(t * kDbTile);
         if (METRIC == 1) {
           // -|q-d|^2 = 2 q.d - |d|^2 - |q|^2 ; the last term is constant per query
@@ -338,8 +426,7 @@ topk_scan_kernel(const __grid_constant__ Maps maps, const Args p) {
           for (int c = 2; c < 32; c += 2) t4[q] = max3(t4[q], v[32 * q + c], v[32 * q + c + 1]);
         }
         const float top = fmaxf(fmaxf(t4[0], t4[1]), fmaxf(t4[2], t4[3]));
-        const bool hit = top > thr;
-        if (hit) {
+        if (top > thr) {
           // rare once the list has warmed up: find the values above the threshold
 #pragma unroll
           for (int g = 0; g < kDbTile / 8; ++g) {
@@ -350,29 +437,76 @@ topk_scan_kernel(const __grid_constant__ Maps maps, const Args p) {
 #pragma unroll
               for (int j = 0; j < 8; ++j)
                 if (v[8 * g + j] > thr && base + 8 * g + j < rows)
-                  thr = fmaxf(seed, list_insert(ls, li, kc, v[8 * g + j], base + 8 * g + j));
+                  thr = fmaxf(seed, list_insert<L::kQTile>(ls, li, kc, v[8 * g + j], base + 8 * g + j));
             }
           }
         }
       }
       // hand the segment's candidates to the finish kernel
-      const size_t out = (size_t(seg) * p.qp + size_t(qt) * kQTile + row) * kc;
+      const size_t out = (size_t(seg) * p.qp + size_t(qt) * L::kQTile + row) * kc;
       for (int j = 0; j < kc; ++j) {
-        p.part_scores[out + j] = ls[j * kQTile];
-        p.part_index[out + j] = li[j * kQTile];
+        p.part_scores[out + j] = ls[j * L::kQTile];
+        p.part_index[out + j] = li[j * L::kQTile];
       }
     }
   }
   tc_fence_before();
   __syncthreads();
-  if (warp == kMmaWarp) tmem_dealloc(tmem, 512);
+  if (warp == L::kMmaWarp) tmem_dealloc(tmem, 2 * L::kAccCols);
 }
+
+// One kernel per row type; each __launch_bounds__ gives ptxas the register limit
+// of that configuration's warp count.
+template <int METRIC>
+__global__ void __launch_bounds__(F16Scan::kWarps * 32, 1)
+topk_scan_kernel(const __grid_constant__ Maps maps, const Args p) {
+  scan<F16Scan, METRIC>(maps, p);
+}
+
+template <int METRIC>
+__global__ void __launch_bounds__(SplitScan::kWarps * 32, 1)
+split_search_kernel(const __grid_constant__ Maps maps, const Args p) {
+  scan<SplitScan, METRIC>(maps, p);
+}
+
+// ---- loads of row components as fp32 ------------------------------------------------
+// 16 bytes: 8 fp16 or 4 fp32 components.  (Both forms become the same read-only
+// LDG.128; they differ in how far ptxas unrolls the row-norm pass around them,
+// and each keeps the unrolling measured with it.)
+__device__ __forceinline__ void load_f32(const __half *p, float (&x)[8]) {
+  const uint4 raw = *reinterpret_cast<const uint4 *>(p);
+  const __half2 *h = reinterpret_cast<const __half2 *>(&raw);
+#pragma unroll
+  for (int j = 0; j < 4; ++j) {
+    const float2 f = __half22float2(h[j]);
+    x[2 * j] = f.x;
+    x[2 * j + 1] = f.y;
+  }
+}
+__device__ __forceinline__ void load_f32(const float *p, float (&x)[4]) {
+  const float4 v = __ldg(reinterpret_cast<const float4 *>(p));
+  x[0] = v.x;
+  x[1] = v.y;
+  x[2] = v.z;
+  x[3] = v.w;
+}
+// 4 fp16 components (a lane's quarter of a query), 2 bytes at a time
+__device__ __forceinline__ void load_f32(const __half *p, float (&x)[4]) {
+#pragma unroll
+  for (int j = 0; j < 4; ++j) x[j] = __half2float(p[j]);
+}
+
+// components of a row per 16-byte load
+template <typename Row>
+constexpr int kChunk = 16 / int(sizeof(Row));
 
 // ---- |d|^2 per database row (L2 metric); +inf for the padding rows; and the ----------
 // largest |d|^2 of the real rows into *max_sqnorm (float bits, zeroed by the caller)
+template <typename Row>
 __global__ void __launch_bounds__(256)
-row_sqnorm_kernel(const __half *__restrict__ db, int64_t rows, int64_t padded, float *__restrict__ out,
+row_sqnorm_kernel(const Row *__restrict__ db, int64_t rows, int64_t padded, float *__restrict__ out,
                   unsigned int *__restrict__ max_sqnorm) {
+  constexpr int n = kChunk<Row>;
   const int sub = threadIdx.x & 15;
   const int64_t per_pass = int64_t(gridDim.x) * (blockDim.x >> 4);
   float top = 0.f;
@@ -380,13 +514,12 @@ row_sqnorm_kernel(const __half *__restrict__ db, int64_t rows, int64_t padded, f
        i += per_pass) {
     float s = 0.f;
     if (i < rows) {
-      const uint4 raw = *reinterpret_cast<const uint4 *>(db + i * kHidden + sub * 8);
-      const __half2 *h = reinterpret_cast<const __half2 *>(&raw);
 #pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        const float2 f = __half22float2(h[j]);
-        s = fmaf(f.x, f.x, s);
-        s = fmaf(f.y, f.y, s);
+      for (int c = 0; c < 8; c += n) {
+        float x[n];
+        load_f32(db + i * kHidden + sub * 8 + c, x);
+#pragma unroll
+        for (int j = 0; j < n; ++j) s = fmaf(x[j], x[j], s);
       }
     }
 #pragma unroll
@@ -430,34 +563,21 @@ __device__ __forceinline__ float exact_step(float acc, float q, float x) {
 
 // Exact score of (query in shared memory as fp32, database row): a sequential
 // fp32 FMA chain in dimension order.
-template <int METRIC>
-__device__ __forceinline__ float exact_score(const float *q, const __half *row) {
+template <int METRIC, typename Row>
+__device__ __forceinline__ float exact_score(const float *q, const Row *row) {
+  constexpr int n = kChunk<Row>;
   float acc = 0.f;
 #pragma unroll 4
-  for (int c = 0; c < kHidden / 8; ++c) {
-    const uint4 raw = __ldg(reinterpret_cast<const uint4 *>(row) + c);
-    const __half *h = reinterpret_cast<const __half *>(&raw);
+  for (int c = 0; c < kHidden / n; ++c) {
+    float x[n];
+    load_f32(row + c * n, x);
 #pragma unroll
-    for (int j = 0; j < 8; ++j) acc = exact_step<METRIC>(acc, q[c * 8 + j], __half2float(h[j]));
+    for (int j = 0; j < n; ++j) acc = exact_step<METRIC>(acc, q[c * n + j], x[j]);
   }
   return METRIC == 0 ? acc : -acc;
 }
 
 constexpr int kFinishWarps = 4;
-
-// Certificate margin, relative: eps = 2^-14 |q| N_max (cosine) or
-// 2^-14 (2 |q| N_max + N_max^2 + |q|^2) (L2, the scan's frame), N_max the
-// largest row norm.  It has to cover the exact chain's error plus the tensor
-// cores' error on the same dot product.  The sequential chain of 128 FMAs is
-// within 128 * 2^-24 * sum|q_i x_i| = 2^-17 sum|q_i x_i| of the real value.
-// Published measurements of fp16-input, fp32-accumulate tensor cores on earlier
-// NVIDIA generations show an accumulator that truncates, about 2^-23 per
-// addition, which over 128 products is 2^-16 sum|q_i x_i|; and
-// sum|q_i x_i| <= |q| N_max (for L2 the terms of 2 q.d - |d|^2 and |q|^2 add
-// the other two parts).  2^-14 leaves a margin of at least 4x over the sum.
-// The B200's accumulator has not been measured: this constant rests on that
-// argument, not on a measurement.
-constexpr float kCertRel = 1.f / 16384.f;
 
 // k selection rounds over the (score desc, index asc) order of query qi's
 // segs x kc candidate slots (index INT_MAX = empty slot).  Writes the output
@@ -501,10 +621,12 @@ __device__ __forceinline__ float select_topk(const float *__restrict__ part_scor
 
 // One warp per query: exact rescoring of the candidates, selection, and the
 // certificate.  `seed` is the seeding pre-pass's [qp][kc] lists or NULL;
-// uncertified queries are appended to `flagged` (count in *fallbacks).
-template <int METRIC>
+// uncertified queries are appended to `flagged` (count in *fallbacks).  For fp32
+// rows a query with a component above the fp16 range (its hi part is inf; the
+// scan's scores for it are meaningless) is flagged whatever its certificate.
+template <class Cfg, int METRIC>
 __global__ void __launch_bounds__(kFinishWarps * 32)
-topk_finish_kernel(const __half *__restrict__ queries, const __half *__restrict__ db,
+topk_finish_kernel(const typename Cfg::Row *__restrict__ queries, const typename Cfg::Row *__restrict__ db,
                    float *__restrict__ part_scores, const int32_t *__restrict__ part_index,
                    const float *__restrict__ seed, const unsigned int *__restrict__ max_sqnorm,
                    int64_t segs, int64_t qp, int kc, int64_t Q, int k, int64_t index_base,
@@ -515,12 +637,19 @@ topk_finish_kernel(const __half *__restrict__ queries, const __half *__restrict_
   const int64_t qi = int64_t(blockIdx.x) * kFinishWarps + warp;
   if (qi >= Q) return;
   float *q = qsm[warp];
-  float qq = 0.f;
+  float v[4];
+  load_f32(queries + qi * kHidden + lane * 4, v);
 #pragma unroll
-  for (int j = 0; j < 4; ++j) {
-    const float v = __half2float(queries[qi * kHidden + lane * 4 + j]);
-    q[lane * 4 + j] = v;
-    qq = fmaf(v, v, qq);
+  for (int j = 0; j < 4; ++j) q[lane * 4 + j] = v[j];
+  // |q|^2 sets eps to its last bit, and so which borderline queries are
+  // certified: each row type keeps its own order of the sum.
+  float qq = 0.f, qmax = 0.f;
+  if constexpr (Cfg::kSplit) {
+    qq = fmaf(v[0], v[0], fmaf(v[1], v[1], fmaf(v[2], v[2], fmaf(v[3], v[3], qq))));
+    qmax = fmaxf(fmaxf(fabsf(v[0]), fabsf(v[1])), fmaxf(fabsf(v[2]), fabsf(v[3])));
+  } else {
+#pragma unroll
+    for (int j = 0; j < 4; ++j) qq = fmaf(v[j], v[j], qq);
   }
   // pass 0, before the tensor-core scores are overwritten: every row the scan
   // dropped has a tensor-core score <= max(seed', last entry of a full list)
@@ -532,6 +661,7 @@ topk_finish_kernel(const __half *__restrict__ queries, const __half *__restrict_
 #pragma unroll
   for (int d = 16; d > 0; d >>= 1) {
     qq += __shfl_xor_sync(0xffffffffu, qq, d);
+    if constexpr (Cfg::kSplit) qmax = fmaxf(qmax, __shfl_xor_sync(0xffffffffu, qmax, d));
     bound = fmaxf(bound, __shfl_xor_sync(0xffffffffu, bound, d));
   }
   __syncwarp();
@@ -546,13 +676,20 @@ topk_finish_kernel(const __half *__restrict__ queries, const __half *__restrict_
   // pass 2: selection
   const float sk = select_topk(part_scores, part_index, segs, qp, kc, qi, k, index_base, out_scores,
                                out_index);
-  // certificate: no dropped row can reach the k-th exact score (kCertRel above).
+  // certificate: no dropped row can reach the k-th exact score (the Cfg's margin).
   // A query whose scan dropped nothing (B = -inf: small databases) is exact as it is.
   const float n2 = __uint_as_float(*max_sqnorm), qn = sqrtf(qq), nmax = sqrtf(n2);
-  const float eps = METRIC == 0 ? kCertRel * qn * nmax : kCertRel * (2.f * qn * nmax + n2 + qq);
+  float eps = METRIC == 0 ? Cfg::kCertRel * qn * nmax : Cfg::kCertRel * (2.f * qn * nmax + n2 + qq);
+  if constexpr (Cfg::kSplit) {
+    const float abs_eps = Cfg::kCertAbs * (qn + nmax);
+    eps += METRIC == 0 ? abs_eps : 2.f * abs_eps;
+  }
   const float sk_scan = METRIC == 0 ? sk : sk + qq;
-  if (lane == 0 && bound > -INFINITY && !(bound + eps < sk_scan))
-    flagged[atomicAdd(fallbacks, 1ull)] = int32_t(qi);
+  // (For fp16 rows the compiler fuses `bound + eps` with eps's last product: rewriting
+  // these lines can move that rounding, and with it last_fallbacks().)
+  bool flag = bound > -INFINITY && !(bound + eps < sk_scan);
+  if constexpr (Cfg::kSplit) flag = !(qmax <= 65504.f) || flag;
+  if (lane == 0 && flag) flagged[atomicAdd(fallbacks, 1ull)] = int32_t(qi);
 }
 
 // ---- exact fallback -----------------------------------------------------------------
@@ -566,9 +703,30 @@ topk_finish_kernel(const __half *__restrict__ queries, const __half *__restrict_
 constexpr int kFbWarps = 8, kFbRows = 64, kFbStride = kHidden + 1;   // +1: conflict-free columns
 constexpr int kFbBlocksPerSM = 4;
 
-template <int METRIC>
+// Rows [t, min(t + kFbRows, r1)) of the database into xs as fp32, zeros past r1.
+__device__ __forceinline__ void stage_rows(float *xs, const __half *db, int64_t t, int64_t r1) {
+  for (int e = threadIdx.x; e < kFbRows * (kHidden / 8); e += kFbWarps * 32) {
+    const int r = e / (kHidden / 8), c = e % (kHidden / 8);
+    float x[8] = {};
+    if (t + r < r1) load_f32(db + (t + r) * kHidden + c * 8, x);
+#pragma unroll
+    for (int j = 0; j < 8; ++j) xs[r * kFbStride + c * 8 + j] = x[j];
+  }
+}
+__device__ __forceinline__ void stage_rows(float *xs, const float *db, int64_t t, int64_t r1) {
+#pragma unroll 1   // unrolled, ptxas spills at 48 registers
+  for (int e = threadIdx.x; e < kFbRows * (kHidden / 4); e += kFbWarps * 32) {
+    const int r = e / (kHidden / 4), c = e % (kHidden / 4);
+    float x[4] = {};
+    if (t + r < r1) load_f32(db + (t + r) * kHidden + c * 4, x);
+#pragma unroll
+    for (int j = 0; j < 4; ++j) xs[r * kFbStride + c * 4 + j] = x[j];
+  }
+}
+
+template <class Cfg, int METRIC>
 __global__ void __launch_bounds__(kFbWarps * 32)
-topk_fallback_scan_kernel(const __half *__restrict__ queries, const __half *__restrict__ db,
+topk_fallback_scan_kernel(const typename Cfg::Row *__restrict__ queries, const typename Cfg::Row *__restrict__ db,
                           int64_t num_rows, int64_t rows_per_seg, int64_t segs, int64_t qp, int kc, int k,
                           const unsigned long long *__restrict__ fallbacks,
                           const int32_t *__restrict__ flagged, float *__restrict__ part_scores,
@@ -584,8 +742,10 @@ topk_fallback_scan_kernel(const __half *__restrict__ queries, const __half *__re
     const int64_t qi = active ? flagged[g * kFbWarps + warp] : 0;
     __syncthreads();                                    // the previous item is done with qsm / xs
     if (active) {
+      float v[4];
+      load_f32(queries + qi * kHidden + lane * 4, v);
 #pragma unroll
-      for (int j = 0; j < 4; ++j) qsm[warp][lane * 4 + j] = __half2float(queries[qi * kHidden + lane * 4 + j]);
+      for (int j = 0; j < 4; ++j) qsm[warp][lane * 4 + j] = v[j];
     }
     const float *q = qsm[warp];
     float ls = -INFINITY, ts = -INFINITY;               // this lane's entry; the k-th entry
@@ -594,14 +754,7 @@ topk_fallback_scan_kernel(const __half *__restrict__ queries, const __half *__re
     const int64_t r1 = r0 + rows_per_seg < num_rows ? r0 + rows_per_seg : num_rows;
     for (int64_t t = r0; t < r1; t += kFbRows) {
       __syncthreads();
-      for (int e = threadIdx.x; e < kFbRows * (kHidden / 8); e += kFbWarps * 32) {
-        const int r = e / (kHidden / 8), c = e % (kHidden / 8);
-        uint4 raw = make_uint4(0u, 0u, 0u, 0u);
-        if (t + r < r1) raw = __ldg(reinterpret_cast<const uint4 *>(db + (t + r) * kHidden) + c);
-        const __half *h = reinterpret_cast<const __half *>(&raw);
-#pragma unroll
-        for (int j = 0; j < 8; ++j) xs[r * kFbStride + c * 8 + j] = __half2float(h[j]);
-      }
+      stage_rows(xs, db, t, r1);
       __syncthreads();
       if (!active) continue;
       const float *x0 = xs + lane * kFbStride, *x1 = xs + (lane + 32) * kFbStride;
@@ -696,292 +849,6 @@ topk_merge_kernel(const float *__restrict__ in_scores, const int64_t *__restrict
   }
 }
 
-template <int METRIC>
-static int launch_scan(const Maps &maps, const Args &a, int64_t items, cudaStream_t st) {
-  const int smem = Smem::total(a.kc);
-  GFX_CUDA(cudaFuncSetAttribute(topk_scan_kernel<METRIC>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                232448));
-  const int grid = int(items < kNumSMs ? items : kNumSMs);
-  topk_scan_kernel<METRIC><<<grid, kWarps * 32, smem, st>>>(maps, a);
-  GFX_LAUNCH_CHECK();
-  return GFX_OK;
-}
-
-// scan (after the optional seeding pre-pass), finish with the certificate, and
-// the exact fallback for the flagged queries -- all stream-ordered, no host sync
-template <int METRIC>
-static int search(const Maps &maps, const Args &a, const Args &pre, const Plan &plan, const __half *q,
-                  const __half *db, int64_t Q, int64_t num_rows, int k, int64_t index_base,
-                  float *out_scores, int64_t *out_index, unsigned long long *fallbacks,
-                  const unsigned int *max_sqnorm, int32_t *flagged, cudaStream_t st) {
-  int rc = plan.sample_tiles ? launch_scan<METRIC>(maps, pre, plan.tiles_q, st) : GFX_OK;
-  if (!rc) rc = launch_scan<METRIC>(maps, a, plan.tiles_q * plan.segs, st);
-  if (rc) return rc;
-  const int finish_blocks = int((Q + kFinishWarps - 1) / kFinishWarps);
-  topk_finish_kernel<METRIC><<<finish_blocks, kFinishWarps * 32, 0, st>>>(
-      q, db, a.part_scores, a.part_index, a.seed, max_sqnorm,
-      plan.segs, plan.qp, plan.kc, Q, k, index_base, out_scores, out_index, fallbacks, flagged);
-  GFX_LAUNCH_CHECK();
-  topk_fallback_scan_kernel<METRIC><<<kNumSMs * kFbBlocksPerSM, kFbWarps * 32, 0, st>>>(
-      q, db, num_rows, plan.tiles_per_seg * kDbTile, plan.segs, plan.qp, plan.kc, k, fallbacks, flagged,
-      a.part_scores, a.part_index);
-  GFX_LAUNCH_CHECK();
-  topk_fallback_select_kernel<<<kNumSMs, kFinishWarps * 32, 0, st>>>(
-      a.part_scores, a.part_index, plan.segs, plan.qp, plan.kc, k, index_base, fallbacks, flagged,
-      out_scores, out_index);
-  GFX_LAUNCH_CHECK();
-  return GFX_OK;
-}
-
-// =====================================================================================
-// fp32 inputs (gfx_topk_f32): the same contract over float32 rows and queries.  The
-// scores are the sequential fp32 FMA chain over the fp32 values.  The scan multiplies
-// split-fp16 images, x = hi + lo, hi = fp16(x), lo = fp16(x - hi) (the split of
-// gfx_split9.cu): per K step three kind::f16 MMAs, hi.hi + hi.lo + lo.hi, into one fp32
-// TMEM accumulator.  The database image [rows, 256] (hi | lo) is built once per index
-// (gfx_topk_f32_prepare); the queries' image is built per call in the workspace.  Hi and
-// lo operands need twice the shared memory, so a work item holds 128 queries (M = 128):
-//   queries hi + lo 64 KB | 2 database stages x 64 KB (128 rows, hi + lo) | |d|^2 slots
-//   4 KB | candidate lists <= 28 KB  = 224 KB.
-// Warps: 0-3 epilogue (one query per thread), 4 MMA issuer, 5 TMA loader; TMEM 2 x 128
-// columns.  Segments, the seeding pre-pass, kc and the finish / certificate / fallback
-// structure are those above; finish and fallback read the fp32 rows (512 B per row).
-// =====================================================================================
-constexpr int kQTile32 = 128, kStages32 = 2;
-constexpr int kQBytes32 = 4 * kBoxBytes;          // [hi, lo] x 2 K blocks x 128 rows
-constexpr int kDbBytes32 = 4 * kBoxBytes;
-constexpr int kMmaWarp32 = 4, kLoadWarp32 = 5, kWarps32 = 6, kEpiWarps32 = 4;
-
-enum Bar32 {
-  kB32QFull = 0, kB32QEmpty = 1, kB32BFull = 2, kB32BEmpty = 4, kB32DFull = 6, kB32DEmpty = 8,
-  kNumBars32 = 10
-};
-
-struct Smem32 {
-  static constexpr int off_q = 0;
-  static constexpr int off_db = off_q + kQBytes32;
-  static constexpr int off_d2 = off_db + kStages32 * kDbBytes32;
-  static constexpr int off_bar = off_d2 + kD2Slots * kDbTile * 4;
-  static constexpr int off_tmem = off_bar + kNumBars32 * 8;
-  static constexpr int off_list = (off_tmem + 8 + 15) & ~15;
-  static constexpr int total(int kc) { return off_list + kc * kQTile32 * 8; }
-};
-static_assert(Smem32::total(kMaxCand) <= 232448, "exceeds the 227 KB shared-memory limit of sm_100");
-
-static Plan make_plan_f32(int64_t Q, int64_t D, int k) {
-  Plan p = make_plan(Q, D, k, kQTile32);
-  p.off_qimage = p.total;
-  p.total += (size_t(Q) * 2 * kHidden * 2 + 255) & ~size_t(255);
-  return p;
-}
-
-// list_insert with the 128-query stride of the fp32 scan's lists
-__device__ __noinline__ float list_insert32(float *ls, int32_t *li, int kc, float v, int32_t idx) {
-  int j = kc - 1;
-  while (j > 0 && ls[(j - 1) * kQTile32] < v) {
-    ls[j * kQTile32] = ls[(j - 1) * kQTile32];
-    li[j * kQTile32] = li[(j - 1) * kQTile32];
-    --j;
-  }
-  ls[j * kQTile32] = v;
-  li[j * kQTile32] = idx;
-  return ls[(kc - 1) * kQTile32];
-}
-
-template <int METRIC>
-__global__ void __launch_bounds__(kWarps32 * 32, 1)
-split_search_kernel(const __grid_constant__ Maps maps, const Args p) {
-  using L = Smem32;
-  extern __shared__ __align__(1024) uint8_t smem[];
-  uint8_t *qs = smem + L::off_q, *dbs = smem + L::off_db;
-  float *d2s = reinterpret_cast<float *>(smem + L::off_d2);
-  uint64_t *bar = reinterpret_cast<uint64_t *>(smem + L::off_bar);
-  uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(smem + L::off_tmem);
-  float *list_s = reinterpret_cast<float *>(smem + L::off_list);
-
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  if (warp == kMmaWarp32) {
-    tmem_alloc(tmem_slot, 256);
-  } else if (tid == 0) {
-    mbar_init(bar + kB32QFull, 1);
-    mbar_init(bar + kB32QEmpty, 1);
-    for (int s = 0; s < kStages32; ++s) {
-      mbar_init(bar + kB32BFull + s, 1);
-      mbar_init(bar + kB32BEmpty + s, 1);
-    }
-    for (int a = 0; a < 2; ++a) {
-      mbar_init(bar + kB32DFull + a, 1);
-      mbar_init(bar + kB32DEmpty + a, kEpiWarps32);
-    }
-    fence_mbar_init();
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem = *tmem_slot;
-  const int64_t items = p.tiles_q * p.segs;
-
-  if (warp == kLoadWarp32) {
-    // ================================ TMA loader =================================
-    // Box b of a 128-row block is columns [64 b, 64 b + 64) of the image: hi K block 0, 1,
-    // then lo K block 0, 1 -- in shared memory at b * kBoxBytes.
-    uint32_t elected;
-    asm volatile("{\n.reg .pred q;\nelect.sync _|q, 0xffffffff;\nselp.u32 %0, 1, 0, q;\n}" : "=r"(elected));
-    const bool issuer = elected != 0u;
-    if (issuer) {
-      prefetch_tmap(&maps.q);
-      prefetch_tmap(&maps.db);
-    }
-    uint32_t it = 0, item_n = 0;
-    for (int64_t item = blockIdx.x; item < items; item += gridDim.x, ++item_n) {
-      const int64_t qt = item % p.tiles_q, seg = item / p.tiles_q;
-      mbar_wait(bar + kB32QEmpty, (item_n & 1) ^ 1);
-      if (issuer) {
-        mbar_arrive_expect_tx(bar + kB32QFull, kQBytes32);
-#pragma unroll
-        for (int b = 0; b < 4; ++b)
-          tma_load_2d(qs + b * kBoxBytes, &maps.q, b * 64, int(qt * kQTile32), bar + kB32QFull);
-      }
-      __syncwarp();
-      const int64_t t0 = seg * p.tiles_per_seg;
-      const int64_t t1 = t0 + p.tiles_per_seg < p.tiles_db ? t0 + p.tiles_per_seg : p.tiles_db;
-      for (int64_t t = t0; t < t1; ++t, ++it) {
-        const uint32_t s = it % kStages32, ph = (it / kStages32) & 1;
-        uint8_t *dst = dbs + s * kDbBytes32;
-        mbar_wait(bar + kB32BEmpty + s, ph ^ 1);
-        if (issuer) {
-          mbar_arrive_expect_tx(bar + kB32BFull + s, kDbBytes32 + (METRIC == 1 ? kDbTile * 4 : 0));
-#pragma unroll
-          for (int b = 0; b < 4; ++b)
-            tma_load_2d(dst + b * kBoxBytes, &maps.db, b * 64, int(t * kDbTile), bar + kB32BFull + s);
-          if (METRIC == 1)
-            bulk_g2s(d2s + (it % kD2Slots) * kDbTile, p.d2 + t * kDbTile, kDbTile * 4,
-                     bar + kB32BFull + s);
-        }
-        __syncwarp();
-      }
-    }
-    __syncwarp();
-  } else if (warp == kMmaWarp32) {
-    // ================================ MMA issuer =================================
-    // whole warp in the loop, one elected lane issues with warp-uniform operands (see topk_scan_kernel)
-    constexpr uint32_t idesc = idesc_f16(kQTile32, kDbTile);
-    const uint32_t qa = smem_u32(qs), ba = smem_u32(dbs);
-    const uint32_t tm = __shfl_sync(0xffffffffu, tmem, 0);
-    uint32_t elected;
-    asm volatile("{\n.reg .pred q;\nelect.sync _|q, 0xffffffff;\nselp.u32 %0, 1, 0, q;\n}" : "=r"(elected));
-    const bool issuer = elected != 0u;
-    uint32_t it = 0, item_n = 0;
-    for (int64_t item = blockIdx.x; item < items; item += gridDim.x, ++item_n) {
-      const int64_t seg = item / p.tiles_q;
-      const int64_t t0 = seg * p.tiles_per_seg;
-      const int64_t t1 = t0 + p.tiles_per_seg < p.tiles_db ? t0 + p.tiles_per_seg : p.tiles_db;
-      mbar_wait(bar + kB32QFull, item_n & 1);
-      for (int64_t t = t0; t < t1; ++t, ++it) {
-        const uint32_t s = it % kStages32, ph = (it / kStages32) & 1, a = it & 1, pha = (it >> 1) & 1;
-        mbar_wait(bar + kB32BFull + s, ph);
-        mbar_wait(bar + kB32DEmpty + a, pha ^ 1);
-        tc_fence_after();
-        if (issuer) {
-#pragma unroll
-          for (int kk = 0; kk < 8; ++kk) {
-            const int kb = kk >> 2, k = kk & 3;
-#pragma unroll
-            for (int term = 0; term < 3; ++term) {       // hi.hi, hi.lo, lo.hi
-              const int qlo = term == 2, dlo = term == 1;
-              const uint64_t da = smem_desc_sw128(qa + (qlo * 2 + kb) * kBoxBytes + k * 32);
-              const uint64_t db = smem_desc_sw128(ba + s * kDbBytes32 + (dlo * 2 + kb) * kBoxBytes + k * 32);
-              mma_f16_ss(tm + a * kDbTile, da, db, idesc, (kk | term) != 0);
-            }
-          }
-          mma_commit(bar + kB32BEmpty + s);
-          mma_commit(bar + kB32DFull + a);
-        }
-        __syncwarp();
-      }
-      if (issuer) mma_commit(bar + kB32QEmpty);
-      __syncwarp();
-    }
-    __syncwarp();
-  } else {
-    // ============ epilogue: running top-k, one query per thread (as topk_scan_kernel) ========
-    const int row = warp * 32 + lane;                       // query inside the item = TMEM lane
-    const uint32_t tbase = tmem + (uint32_t(warp * 32) << 16);
-    const int kc = p.kc;
-    const int32_t rows = int32_t(p.num_rows);
-    float *ls = list_s + tid;
-    int32_t *li = reinterpret_cast<int32_t *>(list_s + kc * kQTile32) + tid;
-    const float ninf = -INFINITY;
-    uint32_t it = 0;
-    for (int64_t item = blockIdx.x; item < items; item += gridDim.x) {
-      const int64_t qt = item % p.tiles_q, seg = item / p.tiles_q;
-      const int64_t t0 = seg * p.tiles_per_seg;
-      const int64_t t1 = t0 + p.tiles_per_seg < p.tiles_db ? t0 + p.tiles_per_seg : p.tiles_db;
-      for (int j = 0; j < kc; ++j) {
-        ls[j * kQTile32] = ninf;
-        li[j * kQTile32] = INT_MAX;
-      }
-      float seed = ninf;
-      if (p.seed) seed = seed_threshold(p.seed[(size_t(qt) * kQTile32 + row) * kc + kc - 1]);
-      float thr = seed;
-      for (int64_t t = t0; t < t1; ++t, ++it) {
-        const uint32_t a = it & 1, pha = (it >> 1) & 1;
-        mbar_wait(bar + kB32DFull + a, pha);
-        tc_fence_after();
-        float v[kDbTile];
-#pragma unroll
-        for (int cb = 0; cb < 4; ++cb) tmem_ld32(tbase + a * kDbTile + cb * 32, v + cb * 32);
-        tmem_ld_wait();
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(bar + kB32DEmpty + a);
-        const int32_t base = int32_t(t * kDbTile);
-        if (METRIC == 1) {
-          const float4 *d2 = reinterpret_cast<const float4 *>(d2s + (it % kD2Slots) * kDbTile);
-#pragma unroll
-          for (int c4 = 0; c4 < kDbTile / 4; ++c4) {
-            const float4 n = d2[c4];
-            v[4 * c4] = fmaf(2.f, v[4 * c4], -n.x);
-            v[4 * c4 + 1] = fmaf(2.f, v[4 * c4 + 1], -n.y);
-            v[4 * c4 + 2] = fmaf(2.f, v[4 * c4 + 2], -n.z);
-            v[4 * c4 + 3] = fmaf(2.f, v[4 * c4 + 3], -n.w);
-          }
-        }
-        float t4[4];
-#pragma unroll
-        for (int q = 0; q < 4; ++q) {
-          t4[q] = fmaxf(v[32 * q], v[32 * q + 1]);
-#pragma unroll
-          for (int c = 2; c < 32; c += 2) t4[q] = max3(t4[q], v[32 * q + c], v[32 * q + c + 1]);
-        }
-        const float top = fmaxf(fmaxf(t4[0], t4[1]), fmaxf(t4[2], t4[3]));
-        if (top > thr) {
-#pragma unroll
-          for (int g = 0; g < kDbTile / 8; ++g) {
-            const float gm = fmaxf(max3(v[8 * g], v[8 * g + 1], v[8 * g + 2]),
-                                   max3(v[8 * g + 3], v[8 * g + 4],
-                                        max3(v[8 * g + 5], v[8 * g + 6], v[8 * g + 7])));
-            if (gm > thr) {
-#pragma unroll
-              for (int j = 0; j < 8; ++j)
-                if (v[8 * g + j] > thr && base + 8 * g + j < rows)
-                  thr = fmaxf(seed, list_insert32(ls, li, kc, v[8 * g + j], base + 8 * g + j));
-            }
-          }
-        }
-      }
-      const size_t out = (size_t(seg) * p.qp + size_t(qt) * kQTile32 + row) * kc;
-      for (int j = 0; j < kc; ++j) {
-        p.part_scores[out + j] = ls[j * kQTile32];
-        p.part_index[out + j] = li[j * kQTile32];
-      }
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == kMmaWarp32) tmem_dealloc(tmem, 256);
-}
-
 // [rows, 128] fp32 -> [rows, 256] fp16 image hi | lo, hi = fp16(x), lo = fp16(x - hi)
 // (round to nearest; fp16 subnormals kept).  One thread per 4 components.
 __global__ void __launch_bounds__(256)
@@ -1002,242 +869,41 @@ split_rows_kernel(const float *__restrict__ x, int64_t rows, __half *__restrict_
   }
 }
 
-// row_sqnorm_kernel over fp32 rows
-__global__ void __launch_bounds__(256)
-row_sqnorm32_kernel(const float *__restrict__ db, int64_t rows, int64_t padded, float *__restrict__ out,
-                    unsigned int *__restrict__ max_sqnorm) {
-  const int sub = threadIdx.x & 15;
-  const int64_t per_pass = int64_t(gridDim.x) * (blockDim.x >> 4);
-  float top = 0.f;
-  for (int64_t i = int64_t(blockIdx.x) * (blockDim.x >> 4) + (threadIdx.x >> 4); i < padded;
-       i += per_pass) {
-    float s = 0.f;
-    if (i < rows) {
-      const float4 *r = reinterpret_cast<const float4 *>(db + i * kHidden) + sub * 2;
-#pragma unroll
-      for (int j = 0; j < 2; ++j) {
-        const float4 f = __ldg(r + j);
-        s = fmaf(f.x, f.x, s);
-        s = fmaf(f.y, f.y, s);
-        s = fmaf(f.z, f.z, s);
-        s = fmaf(f.w, f.w, s);
-      }
-    }
-#pragma unroll
-    for (int d = 8; d > 0; d >>= 1) s += __shfl_xor_sync(0xffffffffu, s, d, 16);
-    if (sub == 0) out[i] = i < rows ? s : INFINITY;
-    if (i < rows) top = fmaxf(top, s);
-  }
-#pragma unroll
-  for (int d = 16; d > 0; d >>= 1) top = fmaxf(top, __shfl_xor_sync(0xffffffffu, top, d));
-  if ((threadIdx.x & 31) == 0) atomicMax(max_sqnorm, __float_as_uint(top));
-}
-
-// exact_score over an fp32 row: the same chain
-template <int METRIC>
-__device__ __forceinline__ float exact_score32(const float *q, const float *row) {
-  float acc = 0.f;
-#pragma unroll 4
-  for (int c = 0; c < kHidden / 4; ++c) {
-    const float4 x = __ldg(reinterpret_cast<const float4 *>(row) + c);
-    acc = exact_step<METRIC>(acc, q[c * 4], x.x);
-    acc = exact_step<METRIC>(acc, q[c * 4 + 1], x.y);
-    acc = exact_step<METRIC>(acc, q[c * 4 + 2], x.z);
-    acc = exact_step<METRIC>(acc, q[c * 4 + 3], x.w);
-  }
-  return METRIC == 0 ? acc : -acc;
-}
-
-// Certificate margin of the split scan:
-//   cosine  eps = kCertRelSplit |q| N_max + kCertAbsSplit (|q| + N_max)
-//   L2      eps = kCertRelSplit (2 |q| N_max + N_max^2 + |q|^2) + 2 kCertAbsSplit (|q| + N_max)
-// (the scan's frame, as kCertRel).  Against the real dot product R = sum q_i x_i:
-//  * the split.  With fp16 hi and lo normal, q_i = qh_i + ql_i + e_i, |e_i| <= 2^-22 |q_i|
-//    (hi is within 2^-11 |q_i|, lo within 2^-11 of the rest), and the same for x.  The scan
-//    sums qh.xh + qh.xl + ql.xh = (q - e_q).(x - e_x) - ql.xl; with |ql_i| <= 2^-11 (1 + 2^-11)
-//    |q_i| that is within (3 + 2^-9) 2^-22 < 2^-20 of sum |q_i x_i| from R, the dropped lo.lo
-//    term included;
-//  * subnormals.  Where x_i - hi_i (or x_i itself) is below 2^-14, lo (or hi) is rounded onto
-//    the fp16 subnormal grid of spacing 2^-24: an absolute error of at most 2^-25 per
-//    component, which sums to 2^-25 (|q|_1 + |x|_1) <= 2^-25 sqrt(128) (|q| + N_max)
-//    < 2^-21 (|q| + N_max) = kCertAbsSplit (|q| + N_max).  This assumes that kind::f16 takes
-//    subnormal fp16 operands at their value; an MMA that flushed them would lose up to 2^-14
-//    per component;
-//  * the tensor-core accumulator.  3 x 128 products go into one fp32 accumulator; on the
-//    truncation argument of kCertRel (about 2^-23 per addition) that is within
-//    384 x 2^-23 (1 + 2^-10) < 2^-14.4 of sum |q_i x_i|;
-//  * the exact chain: within 2^-17 sum |q_i x_i| (kCertRel).  For L2 the fp32 difference
-//    q_i - x_i adds 2^-23 relative per term of sum (q_i - x_i)^2 <= (|q| + N_max)^2.
-// The sum is below 2^-14.1 sum |q_i x_i| <= 2^-14.1 |q| N_max; 2^-13 leaves more than 2x
-// (for L2, 2 q.d doubles the first and the |d|^2, |q|^2 and chain errors, each <= 2^-16.9 of
-// their square, stay inside the other terms).  As for kCertRel, the B200's accumulator has not
-// been measured: this margin rests on the argument, not on a measurement.  Without the split
-// (a scan of fp16(x) only) the rounding of the inputs alone is 2^-11 sum |q_i x_i| per side.
-constexpr float kCertRelSplit = 1.f / 8192.f, kCertAbsSplit = 1.f / 2097152.f;
-
-// topk_finish_kernel for fp32 inputs.  A query with a component above the fp16 range (its hi
-// part is inf; the scan's scores for it are meaningless) is flagged whatever its certificate.
-template <int METRIC>
-__global__ void __launch_bounds__(kFinishWarps * 32)
-topk32_finish_kernel(const float *__restrict__ queries, const float *__restrict__ db,
-                     float *__restrict__ part_scores, const int32_t *__restrict__ part_index,
-                     const float *__restrict__ seed, const unsigned int *__restrict__ max_sqnorm,
-                     int64_t segs, int64_t qp, int kc, int64_t Q, int k, int64_t index_base,
-                     float *__restrict__ out_scores, int64_t *__restrict__ out_index,
-                     unsigned long long *__restrict__ fallbacks, int32_t *__restrict__ flagged) {
-  __shared__ float qsm[kFinishWarps][kHidden];
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int64_t qi = int64_t(blockIdx.x) * kFinishWarps + warp;
-  if (qi >= Q) return;
-  float *q = qsm[warp];
-  float qq = 0.f, qmax = 0.f;
-  const float4 v = __ldg(reinterpret_cast<const float4 *>(queries + qi * kHidden) + lane);
-  q[lane * 4] = v.x;
-  q[lane * 4 + 1] = v.y;
-  q[lane * 4 + 2] = v.z;
-  q[lane * 4 + 3] = v.w;
-  qq = fmaf(v.x, v.x, fmaf(v.y, v.y, fmaf(v.z, v.z, fmaf(v.w, v.w, qq))));
-  qmax = fmaxf(fmaxf(fabsf(v.x), fabsf(v.y)), fmaxf(fabsf(v.z), fabsf(v.w)));
-  float bound = seed ? seed_threshold(seed[qi * kc + kc - 1]) : -INFINITY;
-  for (int64_t s = lane; s < segs; s += 32) {
-    const size_t off = (size_t(s) * qp + qi) * kc + kc - 1;
-    if (part_index[off] != INT_MAX) bound = fmaxf(bound, part_scores[off]);
-  }
-#pragma unroll
-  for (int d = 16; d > 0; d >>= 1) {
-    qq += __shfl_xor_sync(0xffffffffu, qq, d);
-    qmax = fmaxf(qmax, __shfl_xor_sync(0xffffffffu, qmax, d));
-    bound = fmaxf(bound, __shfl_xor_sync(0xffffffffu, bound, d));
-  }
-  __syncwarp();
-  const int64_t C = segs * kc;
-  for (int64_t c = lane; c < C; c += 32) {
-    const size_t off = (size_t(c / kc) * qp + qi) * kc + (c % kc);
-    const int32_t idx = part_index[off];
-    part_scores[off] = idx == INT_MAX ? -INFINITY : exact_score32<METRIC>(q, db + int64_t(idx) * kHidden);
-  }
-  __syncwarp();
-  const float sk = select_topk(part_scores, part_index, segs, qp, kc, qi, k, index_base, out_scores,
-                               out_index);
-  const float n2 = __uint_as_float(*max_sqnorm), qn = sqrtf(qq), nmax = sqrtf(n2);
-  const float abs_eps = kCertAbsSplit * (qn + nmax);
-  const float eps = METRIC == 0 ? kCertRelSplit * qn * nmax + abs_eps
-                                : kCertRelSplit * (2.f * qn * nmax + n2 + qq) + 2.f * abs_eps;
-  const float sk_scan = METRIC == 0 ? sk : sk + qq;
-  const bool out_of_range = !(qmax <= 65504.f);
-  if (lane == 0 && (out_of_range || (bound > -INFINITY && !(bound + eps < sk_scan))))
-    flagged[atomicAdd(fallbacks, 1ull)] = int32_t(qi);
-}
-
-// topk_fallback_scan_kernel for fp32 inputs: rows staged from the fp32 database directly
-template <int METRIC>
-__global__ void __launch_bounds__(kFbWarps * 32)
-topk32_fallback_scan_kernel(const float *__restrict__ queries, const float *__restrict__ db,
-                            int64_t num_rows, int64_t rows_per_seg, int64_t segs, int64_t qp, int kc, int k,
-                            const unsigned long long *__restrict__ fallbacks,
-                            const int32_t *__restrict__ flagged, float *__restrict__ part_scores,
-                            int32_t *__restrict__ part_index) {
-  __shared__ float xs[kFbRows * kFbStride];
-  __shared__ float qsm[kFbWarps][kHidden];
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int64_t n = int64_t(*fallbacks);
-  const int64_t groups = (n + kFbWarps - 1) / kFbWarps;
-  for (int64_t w = blockIdx.x; w < groups * segs; w += gridDim.x) {
-    const int64_t g = w % groups, seg = w / groups;
-    const bool active = g * kFbWarps + warp < n;
-    const int64_t qi = active ? flagged[g * kFbWarps + warp] : 0;
-    __syncthreads();
-    if (active) {
-#pragma unroll
-      for (int j = 0; j < 4; ++j) qsm[warp][lane * 4 + j] = queries[qi * kHidden + lane * 4 + j];
-    }
-    const float *q = qsm[warp];
-    float ls = -INFINITY, ts = -INFINITY;
-    int32_t li = INT_MAX, ti = INT_MAX;
-    const int64_t r0 = seg * rows_per_seg;
-    const int64_t r1 = r0 + rows_per_seg < num_rows ? r0 + rows_per_seg : num_rows;
-    for (int64_t t = r0; t < r1; t += kFbRows) {
-      __syncthreads();
-#pragma unroll 1   // unrolled, ptxas spills at 48 registers
-      for (int e = threadIdx.x; e < kFbRows * (kHidden / 4); e += kFbWarps * 32) {
-        const int r = e / (kHidden / 4), c = e % (kHidden / 4);
-        float4 x = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (t + r < r1) x = __ldg(reinterpret_cast<const float4 *>(db + (t + r) * kHidden) + c);
-        float *dst = xs + r * kFbStride + c * 4;
-        dst[0] = x.x;
-        dst[1] = x.y;
-        dst[2] = x.z;
-        dst[3] = x.w;
-      }
-      __syncthreads();
-      if (!active) continue;
-      const float *x0 = xs + lane * kFbStride, *x1 = xs + (lane + 32) * kFbStride;
-      float a0 = 0.f, a1 = 0.f;
-#pragma unroll 16
-      for (int d = 0; d < kHidden; ++d) {
-        a0 = exact_step<METRIC>(a0, q[d], x0[d]);
-        a1 = exact_step<METRIC>(a1, q[d], x1[d]);
-      }
-#pragma unroll
-      for (int h = 0; h < 2; ++h) {
-        const float s = METRIC == 0 ? (h ? a1 : a0) : -(h ? a1 : a0);
-        const int32_t i = int32_t(t + h * 32 + lane);
-        unsigned int m = __ballot_sync(0xffffffffu, t + h * 32 + lane < r1 && better<int32_t>(s, i, ts, ti));
-        while (m) {
-          const int src = __ffs(m) - 1;
-          m &= m - 1;
-          const float cs = __shfl_sync(0xffffffffu, s, src);
-          const int32_t ci = __shfl_sync(0xffffffffu, i, src);
-          if (!better<int32_t>(cs, ci, ts, ti)) continue;
-          const int pos = __popc(__ballot_sync(0xffffffffu, lane < k && better<int32_t>(ls, li, cs, ci)));
-          const float us = __shfl_up_sync(0xffffffffu, ls, 1);
-          const int32_t ui = __shfl_up_sync(0xffffffffu, li, 1);
-          if (lane > pos) {
-            ls = us;
-            li = ui;
-          } else if (lane == pos) {
-            ls = cs;
-            li = ci;
-          }
-          ts = __shfl_sync(0xffffffffu, ls, k - 1);
-          ti = __shfl_sync(0xffffffffu, li, k - 1);
-        }
-      }
-    }
-    if (active && lane < kc) {
-      const size_t off = (size_t(seg) * qp + qi) * kc + lane;
-      part_scores[off] = lane < k ? ls : -INFINITY;
-      part_index[off] = lane < k ? li : INT_MAX;
-    }
-  }
-}
-
-template <int METRIC>
-static int launch_split_scan(const Maps &maps, const Args &a, int64_t items, cudaStream_t st) {
-  const int smem = Smem32::total(a.kc);
-  GFX_CUDA(cudaFuncSetAttribute(split_search_kernel<METRIC>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                232448));
-  const int grid = int(items < kNumSMs ? items : kNumSMs);
-  split_search_kernel<METRIC><<<grid, kWarps32 * 32, smem, st>>>(maps, a);
+static int split_rows(const float *x, int64_t rows, __half *image, cudaStream_t st) {
+  int64_t blocks = (rows * (kHidden / 4) + 255) / 256;
+  if (blocks > int64_t(kNumSMs) * 16) blocks = int64_t(kNumSMs) * 16;
+  split_rows_kernel<<<int(blocks), 256, 0, st>>>(x, rows, image);
   GFX_LAUNCH_CHECK();
   return GFX_OK;
 }
 
-// search() for fp32 inputs
-template <int METRIC>
-static int search32(const Maps &maps, const Args &a, const Args &pre, const Plan &plan, const float *q,
-                    const float *db, int64_t Q, int64_t num_rows, int k, int64_t index_base,
-                    float *out_scores, int64_t *out_index, unsigned long long *fallbacks,
-                    const unsigned int *max_sqnorm, int32_t *flagged, cudaStream_t st) {
-  int rc = plan.sample_tiles ? launch_split_scan<METRIC>(maps, pre, plan.tiles_q, st) : GFX_OK;
-  if (!rc) rc = launch_split_scan<METRIC>(maps, a, plan.tiles_q * plan.segs, st);
+template <class Cfg, int METRIC>
+static int launch_scan(const Maps &maps, const Args &a, int64_t items, cudaStream_t st) {
+  const auto kernel = Cfg::kSplit ? split_search_kernel<METRIC> : topk_scan_kernel<METRIC>;
+  const int smem = Cfg::smem_bytes(a.kc);
+  GFX_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448));
+  const int grid = int(items < kNumSMs ? items : kNumSMs);
+  kernel<<<grid, Cfg::kWarps * 32, smem, st>>>(maps, a);
+  GFX_LAUNCH_CHECK();
+  return GFX_OK;
+}
+
+// scan (after the optional seeding pre-pass), finish with the certificate, and
+// the exact fallback for the flagged queries -- all stream-ordered, no host sync
+template <class Cfg, int METRIC>
+static int search(const Maps &maps, const Args &a, const Args &pre, const Plan &plan,
+                  const typename Cfg::Row *q, const typename Cfg::Row *db, int64_t Q, int64_t num_rows, int k,
+                  int64_t index_base, float *out_scores, int64_t *out_index, unsigned long long *fallbacks,
+                  const unsigned int *max_sqnorm, int32_t *flagged, cudaStream_t st) {
+  int rc = plan.sample_tiles ? launch_scan<Cfg, METRIC>(maps, pre, plan.tiles_q, st) : GFX_OK;
+  if (!rc) rc = launch_scan<Cfg, METRIC>(maps, a, plan.tiles_q * plan.segs, st);
   if (rc) return rc;
   const int finish_blocks = int((Q + kFinishWarps - 1) / kFinishWarps);
-  topk32_finish_kernel<METRIC><<<finish_blocks, kFinishWarps * 32, 0, st>>>(
+  topk_finish_kernel<Cfg, METRIC><<<finish_blocks, kFinishWarps * 32, 0, st>>>(
       q, db, a.part_scores, a.part_index, a.seed, max_sqnorm,
       plan.segs, plan.qp, plan.kc, Q, k, index_base, out_scores, out_index, fallbacks, flagged);
   GFX_LAUNCH_CHECK();
-  topk32_fallback_scan_kernel<METRIC><<<kNumSMs * kFbBlocksPerSM, kFbWarps * 32, 0, st>>>(
+  topk_fallback_scan_kernel<Cfg, METRIC><<<kNumSMs * kFbBlocksPerSM, kFbWarps * 32, 0, st>>>(
       q, db, num_rows, plan.tiles_per_seg * kDbTile, plan.segs, plan.qp, plan.kc, k, fallbacks, flagged,
       a.part_scores, a.part_index);
   GFX_LAUNCH_CHECK();
@@ -1248,12 +914,85 @@ static int search32(const Maps &maps, const Args &a, const Args &pre, const Plan
   return GFX_OK;
 }
 
-static int split_rows(const float *x, int64_t rows, __half *image, cudaStream_t st) {
-  int64_t blocks = (rows * (kHidden / 4) + 255) / 256;
-  if (blocks > int64_t(kNumSMs) * 16) blocks = int64_t(kNumSMs) * 16;
-  split_rows_kernel<<<int(blocks), 256, 0, st>>>(x, rows, image);
-  GFX_LAUNCH_CHECK();
-  return GFX_OK;
+// gfx_topk / gfx_topk_f32.  `image` is the database's MMA operand: the rows
+// themselves for fp16, their [rows, 256] hi | lo image for fp32.
+template <class Cfg>
+static int run_search(const char *name, const typename Cfg::Row *queries, int64_t num_queries,
+                      const typename Cfg::Row *database, const void *image, int64_t num_rows, int dim, int k,
+                      int metric, int64_t index_base, float *out_scores, int64_t *out_index,
+                      void *workspace, size_t workspace_bytes, void *stream) {
+  const std::string fn(name);
+  if (dim != kHidden) return fail(GFX_ERR_UNSUPPORTED, fn + ": kernels are specialised for dim = 128");
+  if (k < 1 || k > kMaxK) return fail(GFX_ERR_ARGUMENT, fn + ": k must be in [1, 24]");
+  if (metric != 0 && metric != 1) return fail(GFX_ERR_ARGUMENT, fn + ": metric must be 0 (cosine) or 1 (L2)");
+  if (num_queries < 0 || num_rows < 0 || num_rows > int64_t(INT_MAX) - 256)
+    return fail(GFX_ERR_ARGUMENT, fn + ": bad sizes (rows per call must fit int32)");
+  if (num_queries == 0) return GFX_OK;
+  if (!queries || !out_scores || !out_index || (num_rows > 0 && (!database || !image)))
+    return fail(GFX_ERR_ARGUMENT, fn + ": null pointer");
+  if ((reinterpret_cast<uintptr_t>(queries) | reinterpret_cast<uintptr_t>(database) |
+       reinterpret_cast<uintptr_t>(image)) & 15)
+    return fail(GFX_ERR_ARGUMENT, fn + (Cfg::kSplit ? ": queries, database and image must be 16-byte aligned"
+                                                    : ": queries and database must be 16-byte aligned"));
+  const Plan plan = make_plan<Cfg>(num_queries, num_rows, k);
+  if (workspace_bytes < plan.total || !workspace)
+    return fail(GFX_ERR_WORKSPACE, fn + ": workspace too small");
+  cudaStream_t st = as_stream(stream);
+  char *ws = static_cast<char *>(workspace);
+  Args a{};
+  a.part_scores = reinterpret_cast<float *>(ws + plan.off_scores);
+  a.part_index = reinterpret_cast<int32_t *>(ws + plan.off_index);
+  a.d2 = reinterpret_cast<float *>(ws + plan.off_d2);
+  a.tiles_q = plan.tiles_q; a.tiles_db = plan.tiles_db; a.segs = plan.segs;
+  a.tiles_per_seg = plan.tiles_per_seg; a.qp = plan.qp; a.num_rows = num_rows; a.kc = plan.kc;
+  const int finish_blocks = int((num_queries + kFinishWarps - 1) / kFinishWarps);
+  // fallback count and largest squared row norm start at 0
+  GFX_CUDA(cudaMemsetAsync(ws, 0, kHeaderBytes, st));
+  if (num_rows == 0) {
+    // empty database: a merge of zero lists writes (-inf, -1) everywhere
+    StageScope scope(GFX_STAGE_TOPK, st, 1);
+    topk_merge_kernel<<<finish_blocks, kFinishWarps * 32, 0, st>>>(nullptr, nullptr, 0, num_queries, k,
+                                                                   out_scores, out_index);
+    GFX_LAUNCH_CHECK();
+    return GFX_OK;
+  }
+  __half *qimage = reinterpret_cast<__half *>(ws + plan.off_qimage);   // split scan only
+  Maps maps;
+  int rc = tma::make_rows_map(&maps.q, Cfg::kSplit ? static_cast<const void *>(qimage) : queries, num_queries,
+                              Cfg::kCols, 128);
+  if (!rc) rc = tma::make_rows_map(&maps.db, image, num_rows, Cfg::kCols, kDbTile);
+  if (rc) return rc;
+  // [query split,] sqnorm, [pre-pass,] scan, finish, fallback scan, fallback select
+  StageScope scope(GFX_STAGE_TOPK, st, 5 + (Cfg::kSplit ? 1 : 0) + (plan.sample_tiles ? 1 : 0));
+  if constexpr (Cfg::kSplit) {
+    rc = split_rows(queries, num_queries, qimage, st);
+    if (rc) return rc;
+  }
+  Args pre = a;                            // seeding pre-pass over the first rows, one segment
+  if (plan.sample_tiles) {
+    pre.part_scores = reinterpret_cast<float *>(ws + plan.off_seed_scores);
+    pre.part_index = reinterpret_cast<int32_t *>(ws + plan.off_seed_index);
+    pre.tiles_db = pre.tiles_per_seg = plan.sample_tiles;
+    pre.segs = 1;
+    pre.num_rows = plan.sample_tiles * kDbTile;
+    a.seed = pre.part_scores;
+  }
+  auto *fallbacks = reinterpret_cast<unsigned long long *>(ws + kOffFallbacks);
+  auto *max_sqnorm = reinterpret_cast<unsigned int *>(ws + kOffMaxSqNorm);
+  auto *flagged = reinterpret_cast<int32_t *>(ws + plan.off_flagged);
+  {
+    const int64_t padded = plan.tiles_db * kDbTile;
+    int64_t blocks = (padded + 15) / 16;
+    if (blocks > int64_t(kNumSMs) * 8) blocks = int64_t(kNumSMs) * 8;
+    row_sqnorm_kernel<<<int(blocks), 256, 0, st>>>(database, num_rows, padded, const_cast<float *>(a.d2),
+                                                   max_sqnorm);
+    GFX_LAUNCH_CHECK();
+  }
+  return metric == 1
+      ? search<Cfg, 1>(maps, a, pre, plan, queries, database, num_queries, num_rows, k, index_base, out_scores,
+                       out_index, fallbacks, max_sqnorm, flagged, st)
+      : search<Cfg, 0>(maps, a, pre, plan, queries, database, num_queries, num_rows, k, index_base, out_scores,
+                       out_index, fallbacks, max_sqnorm, flagged, st);
 }
 
 }  // namespace topk
@@ -1263,82 +1002,17 @@ using namespace gfx;
 
 extern "C" size_t gfx_topk_workspace_bytes(int64_t num_queries, int64_t num_rows, int k) {
   if (num_queries <= 0 || num_rows < 0 || k <= 0) return 256;
-  return topk::make_plan(num_queries, num_rows, k).total;
+  return topk::make_plan<topk::F16Scan>(num_queries, num_rows, k).total;
 }
 
 extern "C" int gfx_topk(const void *queries, int64_t num_queries, const void *database,
                         int64_t num_rows, int dim, int k, int metric, int64_t index_base,
                         float *out_scores, int64_t *out_index, void *workspace,
                         size_t workspace_bytes, void *stream) {
-  if (dim != kHidden) return fail(GFX_ERR_UNSUPPORTED, "gfx_topk: kernels are specialised for dim = 128");
-  if (k < 1 || k > topk::kMaxK) return fail(GFX_ERR_ARGUMENT, "gfx_topk: k must be in [1, 24]");
-  if (metric != 0 && metric != 1) return fail(GFX_ERR_ARGUMENT, "gfx_topk: metric must be 0 (cosine) or 1 (L2)");
-  if (num_queries < 0 || num_rows < 0 || num_rows > int64_t(INT_MAX) - 256)
-    return fail(GFX_ERR_ARGUMENT, "gfx_topk: bad sizes (rows per call must fit int32)");
-  if (num_queries == 0) return GFX_OK;
-  if (!queries || !out_scores || !out_index || (num_rows > 0 && !database))
-    return fail(GFX_ERR_ARGUMENT, "gfx_topk: null pointer");
-  if ((reinterpret_cast<uintptr_t>(queries) | reinterpret_cast<uintptr_t>(database)) & 15)
-    return fail(GFX_ERR_ARGUMENT, "gfx_topk: queries and database must be 16-byte aligned");
-  topk::Plan plan = topk::make_plan(num_queries, num_rows, k);
-  if (workspace_bytes < plan.total || !workspace)
-    return fail(GFX_ERR_WORKSPACE, "gfx_topk: workspace too small");
-  cudaStream_t st = as_stream(stream);
-  char *ws = static_cast<char *>(workspace);
-  topk::Args a{};
-  a.part_scores = reinterpret_cast<float *>(ws + plan.off_scores);
-  a.part_index = reinterpret_cast<int32_t *>(ws + plan.off_index);
-  a.d2 = reinterpret_cast<float *>(ws + plan.off_d2);
-  a.tiles_q = plan.tiles_q; a.tiles_db = plan.tiles_db; a.segs = plan.segs;
-  a.tiles_per_seg = plan.tiles_per_seg; a.qp = plan.qp; a.num_rows = num_rows; a.kc = plan.kc;
-  const __half *q = static_cast<const __half *>(queries), *db = static_cast<const __half *>(database);
-  const int finish_blocks = int((num_queries + topk::kFinishWarps - 1) / topk::kFinishWarps);
-  // fallback count and largest squared row norm start at 0
-  GFX_CUDA(cudaMemsetAsync(ws, 0, topk::kHeaderBytes, st));
-  if (num_rows == 0) {
-    // empty database: a merge of zero lists writes (-inf, -1) everywhere
-    StageScope scope(GFX_STAGE_TOPK, st, 1);
-    topk::topk_merge_kernel<<<finish_blocks, topk::kFinishWarps * 32, 0, st>>>(
-        nullptr, nullptr, 0, num_queries, k, out_scores, out_index);
-    GFX_LAUNCH_CHECK();
-    return GFX_OK;
-  }
-  topk::Maps maps;
-  int rc = tma::make_rows128_map(&maps.q, q, num_queries, 128);
-  if (!rc) rc = tma::make_rows128_map(&maps.db, db, num_rows, 128);
-  if (rc) return rc;
-  // sqnorm, [pre-pass,] scan, finish, fallback scan, fallback select
-  StageScope scope(GFX_STAGE_TOPK, st, 5 + (plan.sample_tiles ? 1 : 0));
-  topk::Args pre = a;                      // seeding pre-pass over the first rows, one segment
-  static const bool seeding = [] {         // developer switch: GFX_TOPK_SEED=0 scans unseeded
-    const char *v = getenv("GFX_TOPK_SEED");
-    return !(v && v[0] == '0');
-  }();
-  if (!seeding) plan.sample_tiles = 0;
-  if (plan.sample_tiles) {
-    pre.part_scores = reinterpret_cast<float *>(ws + plan.off_seed_scores);
-    pre.part_index = reinterpret_cast<int32_t *>(ws + plan.off_seed_index);
-    pre.tiles_db = pre.tiles_per_seg = plan.sample_tiles;
-    pre.segs = 1;
-    pre.num_rows = plan.sample_tiles * topk::kDbTile;
-    a.seed = pre.part_scores;
-  }
-  auto *fallbacks = reinterpret_cast<unsigned long long *>(ws + topk::kOffFallbacks);
-  auto *max_sqnorm = reinterpret_cast<unsigned int *>(ws + topk::kOffMaxSqNorm);
-  auto *flagged = reinterpret_cast<int32_t *>(ws + plan.off_flagged);
-  {
-    const int64_t padded = plan.tiles_db * topk::kDbTile;
-    int64_t blocks = (padded + 15) / 16;
-    if (blocks > int64_t(kNumSMs) * 8) blocks = int64_t(kNumSMs) * 8;
-    topk::row_sqnorm_kernel<<<int(blocks), 256, 0, st>>>(db, num_rows, padded, const_cast<float *>(a.d2),
-                                                        max_sqnorm);
-    GFX_LAUNCH_CHECK();
-  }
-  return metric == 1
-      ? topk::search<1>(maps, a, pre, plan, q, db, num_queries, num_rows, k, index_base, out_scores,
-                        out_index, fallbacks, max_sqnorm, flagged, st)
-      : topk::search<0>(maps, a, pre, plan, q, db, num_queries, num_rows, k, index_base, out_scores,
-                        out_index, fallbacks, max_sqnorm, flagged, st);
+  const auto *db = static_cast<const __half *>(database);
+  return topk::run_search<topk::F16Scan>("gfx_topk", static_cast<const __half *>(queries), num_queries, db, db,
+                                         num_rows, dim, k, metric, index_base, out_scores, out_index,
+                                         workspace, workspace_bytes, stream);
 }
 
 extern "C" int gfx_topk_merge(const float *in_scores, const int64_t *in_index, int parts,
@@ -1372,77 +1046,14 @@ extern "C" int gfx_topk_f32_prepare(const float *database, int64_t num_rows, voi
 
 extern "C" size_t gfx_topk_f32_workspace_bytes(int64_t num_queries, int64_t num_rows, int k) {
   if (num_queries <= 0 || num_rows < 0 || k <= 0) return 256;
-  return topk::make_plan_f32(num_queries, num_rows, k).total;
+  return topk::make_plan<topk::SplitScan>(num_queries, num_rows, k).total;
 }
 
 extern "C" int gfx_topk_f32(const float *queries, int64_t num_queries, const float *database,
                             const void *image, int64_t num_rows, int dim, int k, int metric,
                             int64_t index_base, float *out_scores, int64_t *out_index, void *workspace,
                             size_t workspace_bytes, void *stream) {
-  if (dim != kHidden) return fail(GFX_ERR_UNSUPPORTED, "gfx_topk_f32: kernels are specialised for dim = 128");
-  if (k < 1 || k > topk::kMaxK) return fail(GFX_ERR_ARGUMENT, "gfx_topk_f32: k must be in [1, 24]");
-  if (metric != 0 && metric != 1)
-    return fail(GFX_ERR_ARGUMENT, "gfx_topk_f32: metric must be 0 (cosine) or 1 (L2)");
-  if (num_queries < 0 || num_rows < 0 || num_rows > int64_t(INT_MAX) - 256)
-    return fail(GFX_ERR_ARGUMENT, "gfx_topk_f32: bad sizes (rows per call must fit int32)");
-  if (num_queries == 0) return GFX_OK;
-  if (!queries || !out_scores || !out_index || (num_rows > 0 && (!database || !image)))
-    return fail(GFX_ERR_ARGUMENT, "gfx_topk_f32: null pointer");
-  if ((reinterpret_cast<uintptr_t>(queries) | reinterpret_cast<uintptr_t>(database) |
-       reinterpret_cast<uintptr_t>(image)) & 15)
-    return fail(GFX_ERR_ARGUMENT, "gfx_topk_f32: queries, database and image must be 16-byte aligned");
-  topk::Plan plan = topk::make_plan_f32(num_queries, num_rows, k);
-  if (workspace_bytes < plan.total || !workspace)
-    return fail(GFX_ERR_WORKSPACE, "gfx_topk_f32: workspace too small");
-  cudaStream_t st = as_stream(stream);
-  char *ws = static_cast<char *>(workspace);
-  topk::Args a{};
-  a.part_scores = reinterpret_cast<float *>(ws + plan.off_scores);
-  a.part_index = reinterpret_cast<int32_t *>(ws + plan.off_index);
-  a.d2 = reinterpret_cast<float *>(ws + plan.off_d2);
-  a.tiles_q = plan.tiles_q; a.tiles_db = plan.tiles_db; a.segs = plan.segs;
-  a.tiles_per_seg = plan.tiles_per_seg; a.qp = plan.qp; a.num_rows = num_rows; a.kc = plan.kc;
-  const int finish_blocks = int((num_queries + topk::kFinishWarps - 1) / topk::kFinishWarps);
-  GFX_CUDA(cudaMemsetAsync(ws, 0, topk::kHeaderBytes, st));
-  if (num_rows == 0) {
-    StageScope scope(GFX_STAGE_TOPK, st, 1);
-    topk::topk_merge_kernel<<<finish_blocks, topk::kFinishWarps * 32, 0, st>>>(
-        nullptr, nullptr, 0, num_queries, k, out_scores, out_index);
-    GFX_LAUNCH_CHECK();
-    return GFX_OK;
-  }
-  __half *qimage = reinterpret_cast<__half *>(ws + plan.off_qimage);
-  topk::Maps maps;
-  int rc = tma::make_rows_map(&maps.q, qimage, num_queries, 2 * kHidden, topk::kQTile32);
-  if (!rc) rc = tma::make_rows_map(&maps.db, image, num_rows, 2 * kHidden, topk::kDbTile);
-  if (rc) return rc;
-  // query split, sqnorm, [pre-pass,] scan, finish, fallback scan, fallback select
-  StageScope scope(GFX_STAGE_TOPK, st, 6 + (plan.sample_tiles ? 1 : 0));
-  rc = topk::split_rows(queries, num_queries, qimage, st);
-  if (rc) return rc;
-  topk::Args pre = a;
-  if (plan.sample_tiles) {
-    pre.part_scores = reinterpret_cast<float *>(ws + plan.off_seed_scores);
-    pre.part_index = reinterpret_cast<int32_t *>(ws + plan.off_seed_index);
-    pre.tiles_db = pre.tiles_per_seg = plan.sample_tiles;
-    pre.segs = 1;
-    pre.num_rows = plan.sample_tiles * topk::kDbTile;
-    a.seed = pre.part_scores;
-  }
-  auto *fallbacks = reinterpret_cast<unsigned long long *>(ws + topk::kOffFallbacks);
-  auto *max_sqnorm = reinterpret_cast<unsigned int *>(ws + topk::kOffMaxSqNorm);
-  auto *flagged = reinterpret_cast<int32_t *>(ws + plan.off_flagged);
-  {
-    const int64_t padded = plan.tiles_db * topk::kDbTile;
-    int64_t blocks = (padded + 15) / 16;
-    if (blocks > int64_t(kNumSMs) * 8) blocks = int64_t(kNumSMs) * 8;
-    topk::row_sqnorm32_kernel<<<int(blocks), 256, 0, st>>>(database, num_rows, padded,
-                                                          const_cast<float *>(a.d2), max_sqnorm);
-    GFX_LAUNCH_CHECK();
-  }
-  return metric == 1
-      ? topk::search32<1>(maps, a, pre, plan, queries, database, num_queries, num_rows, k, index_base,
-                          out_scores, out_index, fallbacks, max_sqnorm, flagged, st)
-      : topk::search32<0>(maps, a, pre, plan, queries, database, num_queries, num_rows, k, index_base,
-                          out_scores, out_index, fallbacks, max_sqnorm, flagged, st);
+  return topk::run_search<topk::SplitScan>("gfx_topk_f32", queries, num_queries, database, image, num_rows, dim,
+                                           k, metric, index_base, out_scores, out_index, workspace,
+                                           workspace_bytes, stream);
 }

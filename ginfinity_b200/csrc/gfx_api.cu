@@ -196,7 +196,6 @@ extern "C" int gfx_model_create(const gfx_folded_weights *w, gfx_model **out) {
   append_umma_image(la, w->wa_host, H, H, true);
   append_umma_image(lb, w->wb_host, H, H, true);
   size_t o_l1 = ab.put(l1), o_l2 = ab.put(l2), o_la = ab.put(la), o_lb = ab.put(lb);
-  size_t o_sched = ab.reserve(gfx::kSchedSlots * sizeof(uint32_t));
   std::vector<__half> t16(size_t(L) * ED * H);
   for (size_t i = 0; i < t16.size(); ++i) t16[i] = __float2half_rn(w->table_host[i]);
   size_t o_t16 = ab.put(t16);
@@ -228,7 +227,6 @@ extern "C" int gfx_model_create(const gfx_folded_weights *w, gfx_model **out) {
   m->b_in = f(o_b_in); m->b1 = f(o_b1); m->b2 = f(o_b2); m->ln_g = f(o_g); m->ln_b = f(o_b);
   m->ba = f(o_ba); m->bb = f(o_bb);
   m->w1_img = h(o_i1); m->w2_img = h(o_i2); m->wa_img = h(o_ia); m->wb_img = h(o_ib); m->table16 = h(o_t16);
-  m->sched_counters = reinterpret_cast<uint32_t *>(static_cast<char *>(m->arena) + o_sched);
   m->w1_lo_img = h(o_l1); m->w2_lo_img = h(o_l2); m->wa_lo_img = h(o_la); m->wb_lo_img = h(o_lb);
   *out = m;
   return GFX_OK;

@@ -4,7 +4,6 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
-#include <atomic>
 #include <cstdio>
 #include <string>
 #include <vector>
@@ -23,7 +22,6 @@ constexpr int kFeat = 7;
 constexpr int kMaxLayers = 8;
 constexpr int kMaxEdgeDim = 16;
 constexpr int kNumSMs = 148;  // B200
-constexpr int kSchedSlots = 64; // tile-scheduler counters per model (one per launch in flight)
 
 // Row descriptor of the banded fused layer (gfx_row_describe / gfx_edge_describe -> gfx_fused8.cu):
 // which of (i-1, type 0) (i+1, type 1) [(partner, type 2|3)] (i-2, type 4) (i+2, type 5) -- the
@@ -112,9 +110,5 @@ struct gfx_model {
   // lo parts of the same images, lo = fp16(w - fp16(w)): the split-fp16 tensor-core kernels of
   // the fp32 path (gfx_split9.cu) multiply by hi + lo
   const __half *w1_lo_img, *w2_lo_img, *wa_lo_img, *wb_lo_img;
-  // dynamic tile scheduler of the fused layer kernel: kSchedSlots device counters, handed out
-  // round-robin per launch (so launches of one model in flight on different streams do not share one)
-  uint32_t *sched_counters;
-  mutable std::atomic<uint32_t> sched_next{0};
   gfx_host_vectors host;
 };

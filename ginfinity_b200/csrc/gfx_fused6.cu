@@ -41,8 +41,6 @@
 // Barriers that collect arrivals from both CTAs (z full, A2 full, D2 empty,
 // weights ready) live in rank 0 and are reached with mapa + a cluster-scope
 // arrive; completions of the MMAs are multicast to both CTAs by tcgen05.commit.
-#include <cstdlib>
-
 #include "gfx_common.cuh"
 #include "gfx_tma.cuh"
 #include "gfx_pair.cuh"
@@ -104,7 +102,6 @@ struct Args {
   int64_t n;
   int edge_dim;
   uint32_t eps1_h2;          // (1 + eps) rounded to fp16, in both halves of the word
-  long long *trace;          // developer timeline (tools/fused_trace.py); null in production
 };
 
 // parked wait (suspend-time hint) on a local barrier
@@ -201,12 +198,6 @@ __device__ __forceinline__ void epi_a(const Consts &c, uint32_t trow, uint64_t *
   if (lane == 0) mbar_arrive_cluster(leader_bar);
 }
 
-// developer timeline: event `ev` of tile iteration `it`, CTA 0 only
-__device__ __forceinline__ void trace_ev(const Args &p, uint32_t it, int ev) {
-  if (p.trace != nullptr && blockIdx.x == 0 && it < 64) p.trace[it * 16 + ev] = clock64();
-}
-
-template <bool WIDE>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kWarps * 32, 1)
 fused_pair_kernel(const __grid_constant__ Maps maps, const __grid_constant__ Consts c, const Args p) {
   using L = Smem;
@@ -219,11 +210,6 @@ fused_pair_kernel(const __grid_constant__ Maps maps, const __grid_constant__ Con
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const uint32_t rank = cluster_ctarank();
-  if (p.trace != nullptr && tid == 0) {          // every CTA: wall-clock start (end below)
-    unsigned long long ns;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(ns));
-    p.trace[1024 + 2 * blockIdx.x] = (long long)ns;
-  }
   if (warp == kMmaWarp) {
     tmem_alloc2(tmem_slot, kTmemCols);
   } else if (tid == 0) {
@@ -270,10 +256,8 @@ fused_pair_kernel(const __grid_constant__ Maps maps, const __grid_constant__ Con
     const uint32_t a2a = leader(kBarA2aFull), a2b = leader(kBarA2bFull);
     uint32_t it = 0;
     for (int pair = cluster_id; pair < pairs; pair += clusters, ++it) {
-      if (tid == 0) trace_ev(p, it, 6);
       epi_a<0>(c, trow, bar, it & 1, lane, a2a);
       epi_a<1>(c, trow, bar, it & 1, lane, a2b);
-      if (tid == 0) trace_ev(p, it, 7);
     }
   } else if (warp < kProdWarp0) {
     // ================= epilogue B (group g takes iterations it % 2 == g) ===========
@@ -287,7 +271,6 @@ fused_pair_kernel(const __grid_constant__ Maps maps, const __grid_constant__ Con
       const uint32_t hb = it % kHBufs;
       mbar_wait_c(bar + kBarD2Full + g, (it >> 1) & 1);
       tc_fence_after();
-      if (lane == 0 && quad == 0) trace_ev(p, it, 8);
       // the arithmetic of gfx_fused8.cu's epilogue B (gfx_layer_math.cuh), both column halves of
       // the row on this thread: same operations in the same order, same bits
       // (the column half is a run-time value here: two unrolled copies with their 384 constant
@@ -312,7 +295,6 @@ fused_pair_kernel(const __grid_constant__ Maps maps, const __grid_constant__ Con
       fence_async_smem();
       __syncwarp();
       if (lane == 0) mbar_arrive(bar + kBarOReady + hb);
-      if (lane == 0 && quad == 0) trace_ev(p, it, 9);
     }
   } else if (warp < kMmaWarp) {
     // ================= producers: aggregation into the z stage ======================
@@ -375,7 +357,6 @@ fused_pair_kernel(const __grid_constant__ Maps maps, const __grid_constant__ Con
       if (k == 0) {
         mbar_wait_c(bar + kBarHFull + hb, (it / kHBufs) & 1);
         mbar_wait_c(bar + kBarA1Empty + s, ((it >> 1) & 1) ^ 1);
-        if (ptid == 0) trace_ev(p, it, 0);
       }
       const int lr = qid + kQuarters * k;
       uint32_t acc[8];                 // 16 channels as 8 half pairs (+0)
@@ -438,7 +419,6 @@ fused_pair_kernel(const __grid_constant__ Maps maps, const __grid_constant__ Con
         fence_async_smem();
         __syncwarp();
         if (lane == 0) mbar_arrive_cluster(a1f[s]);
-        if (ptid == 0) trace_ev(p, it, 1);
       }
     }
   } else if (warp == kMmaWarp) {
@@ -454,9 +434,8 @@ fused_pair_kernel(const __grid_constant__ Maps maps, const __grid_constant__ Con
       for (int kb = 0; kb < 2; ++kb)
         for (int half = 0; half < 2; ++half)
           bulk_g2s(w1s + (kb * 2 + half) * kWPiece,
-                   w1g + kb * (HID * 128) +
-                       (WIDE ? H * int(rank) + 64 * half : H * half + 64 * int(rank)) * 128,
-                   kWPiece, bar + kBarWLocal);
+                   w1g + kb * (HID * 128) + (H * int(rank) + 64 * half) * 128, kWPiece,
+                   bar + kBarWLocal);
       for (int kb = 0; kb < 4; ++kb)              // rows [64 rank, +64) of K block kb
         bulk_g2s(w2s + kb * kWPiece, w2g + kb * (kHidden * 128) + 64 * int(rank) * 128, kWPiece,
                  bar + kBarWLocal);
@@ -483,8 +462,6 @@ fused_pair_kernel(const __grid_constant__ Maps maps, const __grid_constant__ Con
           mbar_wait_c(bar + kBarA1Full + s, ph2);
           tc_fence_after();
           if (issuer) {
-          trace_ev(p, it, 2);
-          if (WIDE) {
             constexpr uint32_t idesc_w = idesc_f16(2 * kTileM, HID);   // GEMM 1: N = 256
 #pragma unroll
             for (int kk = 0; kk < 8; ++kk) {
@@ -495,28 +472,13 @@ fused_pair_kernel(const __grid_constant__ Maps maps, const __grid_constant__ Con
             }
             mma2_commit(bar + kBarD1aFull);
             mma2_commit(bar + kBarD1bFull);
-          } else {                      // two column halves of N = 128 (rows [128 half + 64 rank, +64))
-#pragma unroll
-            for (int half = 0; half < 2; ++half) {
-#pragma unroll
-              for (int kk = 0; kk < 8; ++kk) {
-                const int kb = kk >> 2, k = kk & 3;
-                const uint64_t da = smem_desc_sw128(za + kb * kKbBytes + k * 32);
-                const uint64_t db = smem_desc_sw128(w1a + (kb * 2 + half) * kWPiece + k * 32);
-                mma2_f16_ss(tmem_u + half * H, da, db, idesc, kk != 0);
-              }
-              mma2_commit(bar + (half ? kBarD1bFull : kBarD1aFull));
-            }
-          }
-          mma2_commit(bar + kBarA1Empty + s);          // z consumed in both CTAs
-          trace_ev(p, it, 3);
+            mma2_commit(bar + kBarA1Empty + s);        // z consumed in both CTAs
           }
           __syncwarp();
           mbar_wait_c(bar + kBarA2aFull, ph);
           mbar_wait_c(bar + kBarD2Empty + g, ph2 ^ 1);
           tc_fence_after();
           if (issuer) {
-            trace_ev(p, it, 4);
 #pragma unroll
             for (int kk = 0; kk < H / 16; ++kk) {
               const uint64_t db = smem_desc_sw128(w2a + (kk >> 2) * kWPiece + (kk & 3) * 32);
@@ -533,7 +495,6 @@ fused_pair_kernel(const __grid_constant__ Maps maps, const __grid_constant__ Con
               mma2_f16_ts(tmem_u + kD2Col + g * kHidden, tmem_u + kk * 8, db, idesc, 1u);
             }
             mma2_commit(bar + kBarD2Full + g);
-            trace_ev(p, it, 5);
           }
           __syncwarp();
         }
@@ -551,7 +512,6 @@ fused_pair_kernel(const __grid_constant__ Maps maps, const __grid_constant__ Con
         const int row0 = (2 * pair + int(rank)) * kTileM;
         uint8_t *dst = hs + hb * kTileBytes;
         mbar_wait_parked(bar + kBarHEmpty + hb, ((it / kHBufs) & 1) ^ 1);
-        trace_ev(p, it, 12);
         mbar_arrive_expect_tx(bar + kBarHFull + hb, kTileBytes);
         tma_load_2d(dst, &maps.h, 0, row0, bar + kBarHFull + hb);
         tma_load_2d(dst + kKbBytes, &maps.h, 64, row0, bar + kBarHFull + hb);
@@ -569,7 +529,6 @@ fused_pair_kernel(const __grid_constant__ Maps maps, const __grid_constant__ Con
         const int row0 = (2 * pair + int(rank)) * kTileM;
         const uint8_t *src = hs + hb * kTileBytes;
         mbar_wait_parked(bar + kBarOReady + hb, (it / kHBufs) & 1);
-        trace_ev(p, it, 10);
         if (row0 < n) {
           tma_store_2d(&maps.out, 0, row0, src);
           tma_store_2d(&maps.out, 64, row0, src + kKbBytes);
@@ -577,7 +536,6 @@ fused_pair_kernel(const __grid_constant__ Maps maps, const __grid_constant__ Con
         bulk_commit();
         bulk_wait_read<0>();                      // shared memory has been read: the buffer is free
         mbar_arrive(bar + kBarHEmpty + hb);
-        trace_ev(p, it, 11);
       }
       bulk_wait_all();
     }
@@ -589,16 +547,9 @@ fused_pair_kernel(const __grid_constant__ Maps maps, const __grid_constant__ Con
   __syncthreads();
   cluster_sync_all();                             // the peer may still be arriving on our barriers
   if (warp == kMmaWarp) tmem_dealloc2(tmem, kTmemCols);
-  if (p.trace != nullptr && tid == 0) {
-    unsigned long long ns;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(ns));
-    p.trace[1024 + 2 * blockIdx.x + 1] = (long long)ns;
-  }
 }
 
 }  // namespace v6
-
-long long *g_trace = nullptr;       // shared with gfx_fused8.cu
 
 int fused6_layer(const gfx_model *m, int layer, const __half *h, const int32_t *row_ptr,
                  const int32_t *col_src, const uint8_t *col_type, int64_t n, __half *h_out,
@@ -630,59 +581,20 @@ int fused6_layer(const gfx_model *m, int layer, const __half *h, const int32_t *
   a.n = n; a.edge_dim = m->edge_dim;
   const uint32_t e16 = __half_as_ushort(__float2half_rn(m->eps1[layer]));
   a.eps1_h2 = e16 | (e16 << 16);
-  a.trace = g_trace;
-  static const bool wide = [] {
-    const char *v = getenv("GFX_FUSED_WIDE");      // developer switch: "0" = GEMM 1 as two N = 128 halves
-    return !(v && *v == '0');
-  }();
-  auto kernel = wide ? v6::fused_pair_kernel<true> : v6::fused_pair_kernel<false>;
-  GFX_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, v6::Smem::total));
+  GFX_CUDA(cudaFuncSetAttribute(v6::fused_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                v6::Smem::total));
   const int64_t tiles = (n + v6::kTileM - 1) / v6::kTileM;
   const int64_t pairs = (tiles + 1) / 2;
-  // One CTA pair per TPC -- but only as many as this GPU can hold at once: which SMs are fused off
-  // differs from chip to chip, and a pair that does not fit waits for a whole wave to finish.
-  static int resident[64] = {};                   // per device; 0 = not asked yet
-  int device = 0;
-  GFX_CUDA(cudaGetDevice(&device));
-  if (device >= 0 && device < 64 && resident[device] == 0) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(kNumSMs, 1, 1);
-    cfg.blockDim = dim3(v6::kWarps * 32, 1, 1);
-    cfg.dynamicSmemBytes = v6::Smem::total;
-    cudaLaunchAttribute attr;
-    attr.id = cudaLaunchAttributeClusterDimension;
-    attr.val.clusterDim.x = 2;
-    attr.val.clusterDim.y = 1;
-    attr.val.clusterDim.z = 1;
-    cfg.attrs = &attr;
-    cfg.numAttrs = 1;
-    int max_clusters = 0;
-    if (cudaOccupancyMaxActiveClusters(&max_clusters, kernel, &cfg) != cudaSuccess ||
-        max_clusters < 1) {
-      (void)cudaGetLastError();
-      max_clusters = kNumSMs / 2;
-    }
-    resident[device] = max_clusters < kNumSMs / 2 ? max_clusters : kNumSMs / 2;
-    if (getenv("GFX_VERBOSE"))
-      fprintf(stderr, "libgfx: fused pair kernel: %d resident CTA pairs on device %d\n",
-              resident[device], device);
-  }
-  const int cap = device >= 0 && device < 64 ? resident[device] : kNumSMs / 2;
+  int cap = 0;
+  rc = resident_pairs<v6::fused_pair_kernel>(v6::kWarps * 32, v6::Smem::total, &cap);
+  if (rc) return rc;
   const int clusters = int(pairs < cap ? pairs : cap);
-  kernel<<<2 * clusters, v6::kWarps * 32, v6::Smem::total, st>>>(maps, c, a);
+  v6::fused_pair_kernel<<<2 * clusters, v6::kWarps * 32, v6::Smem::total, st>>>(maps, c, a);
   GFX_LAUNCH_CHECK();
   return GFX_OK;
 }
 
 }  // namespace gfx
-
-// developer hook (not part of include/gfx.h): device buffer of 64 x 16 + 2 x 160 int64; CTA 0 of the
-// next gfx_layer_fused_pair launches fills the first part with clock64() stamps, every CTA writes its
-// wall-clock start and end (globaltimer) into the second; null switches it off
-extern "C" int gfx_debug_fused_trace(long long *device_buffer) {
-  gfx::g_trace = device_buffer;
-  return GFX_OK;
-}
 
 extern "C" int gfx_layer_fused_pair(const gfx_model *m, int layer, const void *h,
                                     const int32_t *row_ptr, const int32_t *col_src,

@@ -41,8 +41,9 @@
 //    instructions per tcgen05.mma), and so does the loader, which also prefetches the next h tile
 //    into L2; every epilogue-B warp stores its own 32 x 64 block by TMA and hands the buffer back
 //    itself (there is no store warp); molecule-end rows are recomputed at the end of their run
-//    from the registers that are still live; the production instance (template DEV = false)
-//    carries none of the developer tests in its loops.
+//    from the registers that are still live.  The loops carry nothing but the layer itself (no
+//    timeline stamps, no experiment switches): the kernel is bound by the number of instructions
+//    its warps issue.
 //    603k-node probe: 0.146 -> 0.099 ms; ncu: 129 -> 87.5 warp instructions per node-layer,
 //    tensor pipe 28.6 -> 45.4 % active (profiles/r02_f_full_encoder_kernels.txt).
 //
@@ -54,9 +55,6 @@
 //   12-19  producers    warp w owns tile rows [16 w, 16 w + 16), two runs of 8 rows
 //   20     MMA issuer (rank 0 issues for the pair; GEMM 1 as 8 MMAs of N = 256), 21 h-tile loader
 //          (TMA), 22-23 spare
-#include <cstdlib>
-#include <type_traits>
-
 #include "gfx_common.cuh"
 #include "gfx_tma.cuh"
 #include "gfx_pair.cuh"
@@ -90,11 +88,10 @@ constexpr int kDescPartnerShift = rowdesc::kPartnerShift, kDescPartnerBits = row
 constexpr uint32_t kDescPartnerMask = rowdesc::kPartnerMask;
 
 enum Bar {
-  kBarWLocal = 0, kBarWReady = 1, kBarHFull = 2, kBarHEmpty = 5, kBarOReady = 8, kBarA1Full = 11,
-  kBarA1Empty = 13, kBarD1aFull = 15, kBarD1bFull = 16, kBarA2aFull = 17, kBarA2bFull = 18,
-  kBarD2Full = 19, kBarD2Empty = 21, kBarSched = 23, kNumBars = 23 + 16
+  kBarWLocal = 0, kBarWReady = 1, kBarHFull = 2, kBarHEmpty = 5, kBarA1Full = 8, kBarA1Empty = 10,
+  kBarD1aFull = 12, kBarD1bFull = 13, kBarA2aFull = 14, kBarA2bFull = 15, kBarD2Full = 16,
+  kBarD2Empty = 18, kNumBars = 20
 };
-constexpr int kRing = 16;                     // tile-pair indices in flight between the roles (kBarSched ..)
 
 struct Smem {
   static constexpr int off_w1 = 0;                                   // [kb 2] x 16 KB (128 rows)
@@ -102,8 +99,7 @@ struct Smem {
   static constexpr int off_z = off_w2 + 4 * kWPiece;                 // 2 stages x 32 KB
   static constexpr int off_h = off_z + kStages * kTileBytes;         // 3 tiles x 32 KB
   static constexpr int off_x = off_h + kHBufs * kTileBytes;          // float2 [2 halves][128 rows]
-  static constexpr int off_ring = off_x + 2 * kTileM * 8;             // int [kRing]: dynamic tile-pair indices
-  static constexpr int off_tab = off_ring + kRing * 4;                // uint32 [8 producer warps][16 rows]: row words
+  static constexpr int off_tab = off_x + 2 * kTileM * 8;              // uint32 [8 producer warps][16 rows]: row words
   static constexpr int off_bar = off_tab + 8 * 16 * 4;
   static constexpr int off_tmem = off_bar + kNumBars * 8;
   static constexpr int total = off_tmem + 8;
@@ -119,34 +115,29 @@ struct Args {
   const int32_t *row_ptr, *col_src;
   const uint8_t *col_type;
   const uint32_t *desc;      // [n] row descriptors
-  uint32_t sleep_ns;         // sleep between barrier polls of the warp-wide waits
   const __half *table16, *w1_img, *w2_img;
   int64_t n;
   int edge_dim;
   uint32_t eps1_h2;          // (1 + eps) rounded to fp16, in both halves of the word
-  long long *trace;          // developer timeline (tools/fused_trace.py); null in production
-  uint32_t dbg;              // developer experiments (GFX_DBG): timing only, results are wrong
-  uint32_t *sched;           // dynamic tile scheduler: device counter, zero at launch (DYN kernels)
 };
 
 __device__ __forceinline__ void mbar_wait_c(uint64_t *bar, uint32_t parity) {
   mbar_wait_parked(bar, parity);
 }
-__device__ __forceinline__ void mbar_wait_s(uint64_t *bar, uint32_t parity, uint32_t sleep_ns) {
-  while (!mbar_try_wait(bar, parity)) {
-    if (sleep_ns) __nanosleep(sleep_ns);
-  }
+// warp-wide wait with a short sleep between polls
+__device__ __forceinline__ void mbar_wait_s(uint64_t *bar, uint32_t parity) {
+  while (!mbar_try_wait(bar, parity)) __nanosleep(64);
 }
 
 // ---- epilogue A: D1[:, HALF*128 .. +128) -> + b1, ReLU -> fp16 -> A2[:, HALF*64 .. +64) ---------
 template <int HALF>
 __device__ __forceinline__ void epi_a(const Consts &c, uint32_t trow, uint64_t *bar, uint32_t ph,
-                                      int lane, uint32_t leader_bar, uint32_t sleep_ns, bool skip) {
+                                      int lane, uint32_t leader_bar) {
   constexpr int col0 = HALF * H;
-  mbar_wait_s(bar + (HALF ? kBarD1bFull : kBarD1aFull), ph, sleep_ns);
+  mbar_wait_s(bar + (HALF ? kBarD1bFull : kBarD1aFull), ph);
   tc_fence_after();
 #pragma unroll
-  for (int q = 0; q < (skip ? 0 : 4); ++q) {
+  for (int q = 0; q < 4; ++q) {
     float v[32];
     tmem_ld32(trow + col0 + 32 * q, v);
     tmem_ld_wait();
@@ -200,30 +191,9 @@ __device__ __forceinline__ bool elect_one() {
   return pred != 0;
 }
 
-// developer timeline: event `ev` of tile iteration `it`, CTA 0 only
-__device__ __forceinline__ void trace_ev(const Args &p, uint32_t it, int ev) {
-  if (p.trace != nullptr && blockIdx.x == 0 && it < 64) p.trace[it * 16 + ev] = clock64();
-}
-
-// DYN (GFX_SCHED=dynamic; off by default, see fused8_layer): tile pairs are handed out by an
-// atomic counter instead of round-robin.  With equal static work the CTA pairs of one launch
-// finish 15 % apart (123 ... 143 us on a 603k-node chunk; the groups follow the GPC placement).
-// Rank 0's loader thread fetches the cluster's next pair index two iterations ahead and publishes
-// it to both CTAs through a 16-entry shared-memory ring (st.shared::cluster + a cluster-scope
-// mbarrier arrive for the peer); every role reads entry it + 1 at the top of iteration it.
-// DEV: the developer build (timeline stamps, GFX_DBG experiments, GFX_SCHED=dynamic).  The
-// production instance has none of those tests in its loops: the kernel is bound by the number of
-// instructions its warps issue.
-template <bool DYN, bool DEV>
+// Tile pairs are assigned round-robin: cluster k takes pairs k, k + clusters, ...
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kWarps * 32, 1)
-fused_banded8_kernel(const __grid_constant__ Maps maps, const __grid_constant__ Consts c, const Args p_in) {
-  static_assert(DEV || !DYN, "the dynamic scheduler is a developer option");
-  Args p = p_in;
-  if (!DEV) {
-    p.dbg = 0u;
-    p.trace = nullptr;
-    p.sleep_ns = 64u;                            // (GFX_FUSED_SLEEP_NS selects the developer instance)
-  }
+fused_banded8_kernel(const __grid_constant__ Maps maps, const __grid_constant__ Consts c, const Args p) {
   using L = Smem;
   extern __shared__ __align__(1024) uint8_t smem[];
   uint8_t *w1s = smem + L::off_w1, *w2s = smem + L::off_w2, *zs = smem + L::off_z;
@@ -233,11 +203,6 @@ fused_banded8_kernel(const __grid_constant__ Maps maps, const __grid_constant__ 
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const uint32_t rank = cluster_ctarank();
-  if (p.trace != nullptr && tid == 0) {          // every CTA: wall-clock start (end below)
-    unsigned long long ns;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(ns));
-    p.trace[1024 + 2 * blockIdx.x] = (long long)ns;
-  }
   if (warp == kMmaWarp) {
     tmem_alloc2(tmem_slot, kTmemCols);
   } else if (tid == 0) {
@@ -246,9 +211,7 @@ fused_banded8_kernel(const __grid_constant__ Maps maps, const __grid_constant__ 
     for (int s = 0; s < kHBufs; ++s) {
       mbar_init(bar + kBarHFull + s, 1);
       mbar_init(bar + kBarHEmpty + s, kEpiBWarps);
-      mbar_init(bar + kBarOReady + s, 1);              // (unused: every epilogue-B warp stores its own block)
     }
-    for (int s = 0; s < kRing; ++s) mbar_init(bar + kBarSched + s, 1);
     for (int s = 0; s < 2; ++s) {
       mbar_init(bar + kBarA1Full + s, 2 * kProdWarps);
       mbar_init(bar + kBarA1Empty + s, 1);
@@ -273,26 +236,6 @@ fused_banded8_kernel(const __grid_constant__ Maps maps, const __grid_constant__ 
   const int cluster_id = blockIdx.x >> 1, clusters = gridDim.x >> 1;
   // barriers of rank 0 that collect arrivals from both CTAs
   auto leader = [&](int b) { return map_to_cta(smem_u32(bar + b), 0); };
-  // the cluster's sequence of tile pairs: entry idx of the ring (DYN) or round-robin
-  int *ring = reinterpret_cast<int *>(smem + L::off_ring);
-  auto sched_read = [&](uint32_t idx) -> int {
-    const uint32_t slot = idx % kRing, addr = smem_u32(bar + kBarSched + slot);
-    uint32_t done;
-    do {
-      asm volatile(
-          "{\n.reg .pred q;\n"
-          "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 q, [%1], %2;\n"
-          "selp.u32 %0, 1, 0, q;\n}"
-          : "=r"(done)
-          : "r"(addr), "r"((idx / kRing) & 1u)
-          : "memory");
-    } while (!done);
-    int v;
-    asm volatile("ld.volatile.shared.s32 %0, [%1];" : "=r"(v) : "r"(smem_u32(ring + slot)) : "memory");
-    return v;
-  };
-  auto first_pair = [&]() -> int { return DYN ? sched_read(0) : cluster_id; };
-  auto next_pair = [&](int pair, uint32_t it) -> int { return DYN ? sched_read(it + 1) : pair + clusters; };
 
   if (warp < kEpiBWarp0) {
     // ================= epilogue A =================================================
@@ -300,11 +243,9 @@ fused_banded8_kernel(const __grid_constant__ Maps maps, const __grid_constant__ 
     const uint32_t trow = tmem + (uint32_t(warp * 32) << 16);
     const uint32_t a2a = leader(kBarA2aFull), a2b = leader(kBarA2bFull);
     uint32_t it = 0;
-    for (int pair = first_pair(); pair < pairs; pair = next_pair(pair, it), ++it) {
-      if (tid == 0) trace_ev(p, it, 6);
-      epi_a<0>(c, trow, bar, it & 1, lane, a2a, p.sleep_ns, (p.dbg & 16u) != 0u);
-      epi_a<1>(c, trow, bar, it & 1, lane, a2b, p.sleep_ns, (p.dbg & 16u) != 0u);
-      if (tid == 0) trace_ev(p, it, 7);
+    for (int pair = cluster_id; pair < pairs; pair += clusters, ++it) {
+      epi_a<0>(c, trow, bar, it & 1, lane, a2a);
+      epi_a<1>(c, trow, bar, it & 1, lane, a2b);
     }
   } else if (warp < kProdWarp0) {
     // ================= epilogue B: every warp, every tile ==========================
@@ -318,18 +259,14 @@ fused_banded8_kernel(const __grid_constant__ Maps maps, const __grid_constant__ 
     const bool issuer = elect_one();              // the same lane every time: bulk groups are per thread
     if (issuer) prefetch_tmap(&maps.out);
     uint32_t it = 0;
-    for (int pair = first_pair(); pair < pairs; pair = next_pair(pair, it), ++it) {
+    for (int pair = cluster_id; pair < pairs; pair += clusters, ++it) {
       const uint32_t g = it & 1, hb = it % kHBufs;
       const uint32_t tcol = tmem + (uint32_t(quad * 32) << 16) + kD2Col + g * kHidden + uint32_t(half) * 64u;
-      mbar_wait_s(bar + kBarD2Full + g, (it >> 1) & 1, p.sleep_ns);
+      mbar_wait_s(bar + kBarD2Full + g, (it >> 1) & 1);
       tc_fence_after();
-      if (lane == 0 && warp == kEpiBWarp0) trace_ev(p, it, 8);
       // one pass over TMEM: the 64 columns stay in registers, D2[g] is released at once
       float t[64];
-      if (p.dbg & 8u) {
-#pragma unroll
-        for (int j = 0; j < 64; ++j) t[j] = 1.f;
-      } else if (half) epi_b_load<1>(c, tcol, t); else epi_b_load<0>(c, tcol, t);
+      if (half) epi_b_load<1>(c, tcol, t); else epi_b_load<0>(c, tcol, t);
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive_cluster(d2e0 + 8u * g);
@@ -344,10 +281,9 @@ fused_banded8_kernel(const __grid_constant__ Maps maps, const __grid_constant__ 
       const float var = fmaxf(sq * (1.f / kHidden) - mean * mean, 0.f);
       const float rstd = rsqrtf(var + 1e-5f);
       const float nm = -mean * rstd;
-      mbar_wait_s(bar + kBarHFull + hb, (it / kHBufs) & 1, 0);   // long complete: visibility only
+      mbar_wait(bar + kBarHFull + hb, (it / kHBufs) & 1);       // long complete: visibility only
       const uint32_t hrow = smem_u32(hs) + hb * kTileBytes;
-      if (p.dbg & 8u) {
-      } else if (half) epi_b_store<1>(c, t, hrow, r, rstd, nm); else epi_b_store<0>(c, t, hrow, r, rstd, nm);
+      if (half) epi_b_store<1>(c, t, hrow, r, rstd, nm); else epi_b_store<0>(c, t, hrow, r, rstd, nm);
       // every warp stores its own 32 x 64 block (4 KB, contiguous in the swizzled tile) as soon
       // as it is written and hands the buffer back when the TMA engine has read it: no store
       // warp in between, no waiting for the slowest of the eight (the buffer's life cycle sets
@@ -364,7 +300,6 @@ fused_banded8_kernel(const __grid_constant__ Maps maps, const __grid_constant__ 
         mbar_arrive(bar + kBarHEmpty + hb);
       }
       __syncwarp();
-      if (lane == 0 && warp == kEpiBWarp0) trace_ev(p, it, 9);
     }
     if (issuer) bulk_wait_all();
     __syncwarp();
@@ -424,23 +359,21 @@ fused_banded8_kernel(const __grid_constant__ Maps maps, const __grid_constant__ 
     };
     // Requested at the hand-over of the previous tile, used after this tile's barrier waits:
     // five registers live across the waits, none across the row code.
-    int pair = first_pair();
+    int pair = cluster_id;
     uint32_t dnext = fetch_desc(pair);
     uint2 hn0, hn1;
     fetch_halo(pair, hn0, hn1);
     uint32_t it = 0;
     for (; pair < pairs; ++it) {
-      const int pair_next = next_pair(pair, it);
+      const int pair_next = pair + clusters;
       const uint32_t s = it & 1, hb = it % kHBufs;
       const int row0 = (2 * pair + int(rank)) * kTileM;
       const uint32_t d = dnext;
       const uint2 halo0 = hn0, halo1 = hn1;
       const uint32_t hbase = smem_u32(hs) + hb * kTileBytes;
       const uint32_t zbase = smem_u32(zs) + s * kTileBytes;
-      mbar_wait_s(bar + kBarHFull + hb, (it / kHBufs) & 1, p.sleep_ns);
-      mbar_wait_s(bar + kBarA1Empty + s, ((it >> 1) & 1) ^ 1, p.sleep_ns);
-      if (warp == kProdWarp0 && lane == 0) trace_ev(p, it, 0);
-      if (warp == kProdWarp0 + 3 && lane == 0) trace_ev(p, it, 13);
+      mbar_wait_s(bar + kBarHFull + hb, (it / kHBufs) & 1);
+      mbar_wait_s(bar + kBarA1Empty + s, ((it >> 1) & 1) ^ 1);
 
       // ---- one word per row: [17:3] shared-memory address of the partner row's first chunk
       // (kb 0, swizzle term of the row in bits 4-6), bit 0 = has a pair message, bit 1 = of type 3
@@ -489,7 +422,6 @@ fused_banded8_kernel(const __grid_constant__ Maps maps, const __grid_constant__ 
       uint2 w[kRun + 4];
 #pragma unroll
       for (int run = 0; run < 2; ++run) {
-        if (p.dbg & 32u) break;                                        // timing experiments only
         const uint32_t ro = uint32_t(run) * 1024u;
         if (run == 0) {
           if (pw == 0) {                                               // warp-uniform
@@ -607,12 +539,9 @@ fused_banded8_kernel(const __grid_constant__ Maps maps, const __grid_constant__ 
       dnext = fetch_desc(pair_next);
       fetch_halo(pair_next, hn0, hn1);
       pair = pair_next;
-      if (warp == kProdWarp0 && lane == 0) trace_ev(p, it, 15);
-      if (warp == kProdWarp0 + 3 && lane == 0) trace_ev(p, it, 14);
-      if (!(p.dbg & 4u)) fence_async_smem();
+      fence_async_smem();
       __syncwarp();
       if (lane == 0) mbar_arrive_cluster(a1f0 + 8u * s);
-      if (warp == kProdWarp0 && lane == 0) trace_ev(p, it, 1);
     }
   } else if (warp == kMmaWarp) {
     // ================= weights (both CTAs) + MMA issue (rank 0) ======================
@@ -650,13 +579,12 @@ fused_banded8_kernel(const __grid_constant__ Maps maps, const __grid_constant__ 
       constexpr uint32_t idesc_w = idesc_f16(2 * kTileM, HID);   // GEMM 1: N = 256
       const uint64_t w1d = smem_desc_sw128(smem_u32(w1s)), w2d = smem_desc_sw128(smem_u32(w2s));
       uint32_t it = 0;
-      for (int pair = first_pair(); pair < pairs; pair = next_pair(pair, it), ++it) {
+      for (int pair = cluster_id; pair < pairs; pair += clusters, ++it) {
         const uint32_t s = it & 1, g = it & 1, ph2 = (it >> 1) & 1, ph = it & 1;
         const uint64_t zd = smem_desc_sw128(smem_u32(zs) + s * kTileBytes);
         mbar_wait_c(bar + kBarA1Full + s, ph2);
         tc_fence_after();
         if (issuer) {
-          trace_ev(p, it, 2);
 #pragma unroll
           for (int kk = 0; kk < 8; ++kk) {
             const int kb = kk >> 2, k = kk & 3;
@@ -666,7 +594,6 @@ fused_banded8_kernel(const __grid_constant__ Maps maps, const __grid_constant__ 
           mma2_commit(bar + kBarD1aFull);
           mma2_commit(bar + kBarD1bFull);
           mma2_commit(bar + kBarA1Empty + s);          // z consumed in both CTAs
-          trace_ev(p, it, 3);
         }
         __syncwarp();
         mbar_wait_c(bar + kBarA2aFull, ph);
@@ -674,7 +601,6 @@ fused_banded8_kernel(const __grid_constant__ Maps maps, const __grid_constant__ 
         tc_fence_after();
         const uint32_t d2 = tm + kD2Col + g * kHidden;
         if (issuer) {
-          trace_ev(p, it, 4);
 #pragma unroll
           for (int kk = 0; kk < H / 16; ++kk)
             mma2_f16_ts(d2, tm + kk * 8, w2d + uint64_t(((kk >> 2) * kWPiece + (kk & 3) * 32) >> 4),
@@ -689,7 +615,6 @@ fused_banded8_kernel(const __grid_constant__ Maps maps, const __grid_constant__ 
             mma2_f16_ts(d2, tm + kk * 8, w2d + uint64_t(((kk >> 2) * kWPiece + (kk & 3) * 32) >> 4),
                         idesc, 1u);
           mma2_commit(bar + kBarD2Full + g);
-          trace_ev(p, it, 5);
         }
         __syncwarp();
       }
@@ -698,77 +623,31 @@ fused_banded8_kernel(const __grid_constant__ Maps maps, const __grid_constant__ 
   } else if (warp == kLoadWarp) {
     // ================= h tiles (TMA) =================================================
     reg_dec<40>();
-    if (DYN && lane == 0) {                       // developer option: one thread, scheduler included
-      prefetch_tmap(&maps.h);
-      auto load_tile = [&](int pair, uint32_t it) {
-        const uint32_t hb = it % kHBufs;
-        const int row0 = (2 * pair + int(rank)) * kTileM;
-        uint8_t *dst = hs + hb * kTileBytes;
-        mbar_wait_s(bar + kBarHEmpty + hb, ((it / kHBufs) & 1) ^ 1, p.sleep_ns);
-        trace_ev(p, it, 12);
+    // The whole warp runs the loop and waits; one elected lane issues (as in the MMA warp:
+    // issued from inside `if (lane == 0)` every TMA instruction came wrapped in an ELECT /
+    // R2UR.BROADCAST loop, ~70 instructions per tile on a warp that gets one issue slot in
+    // six -- between "buffer free" and "load issued", i.e. on the buffer's life cycle).
+    const bool issuer = elect_one();
+    if (issuer) prefetch_tmap(&maps.h);
+    uint32_t it = 0;
+    for (int pair = cluster_id; pair < pairs; pair += clusters, ++it) {
+      const uint32_t hb = it % kHBufs;
+      const int row0 = (2 * pair + int(rank)) * kTileM;
+      uint8_t *dst = hs + hb * kTileBytes;
+      mbar_wait_s(bar + kBarHEmpty + hb, ((it / kHBufs) & 1) ^ 1);
+      if (issuer) {
         mbar_arrive_expect_tx(bar + kBarHFull + hb, kTileBytes);
         tma_load_2d(dst, &maps.h, 0, row0, bar + kBarHFull + hb);
         tma_load_2d(dst + kKbBytes, &maps.h, 64, row0, bar + kBarHFull + hb);
-      };
-      if (rank == 0) {
-        // the cluster's scheduler: entries it + 1 and it + 2 of the ring are always published
-        // before the tile of iteration `it` is requested; once the counter passes the last pair
-        // its value is the end mark every role stops at
-        auto publish = [&](uint32_t idx, int value) {
-          const uint32_t slot = idx % kRing;
-          const uint32_t own = smem_u32(ring + slot), ownbar = smem_u32(bar + kBarSched + slot);
-          asm volatile("st.volatile.shared.s32 [%0], %1;" ::"r"(own), "r"(value) : "memory");
-          mbar_arrive(bar + kBarSched + slot);
-          asm volatile("st.shared::cluster.s32 [%0], %1;" ::"r"(map_to_cta(own, 1)), "r"(value) : "memory");
-          asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(map_to_cta(ownbar, 1))
-                       : "memory");
-        };
-        auto fetch = [&](int prev) -> int { return prev < pairs ? int(atomicAdd(p.sched, 1u)) : prev; };
-        int cur = int(atomicAdd(p.sched, 1u));
-        publish(0, cur);
-        int nxt = fetch(cur);
-        publish(1, nxt);
-        for (uint32_t it = 0; cur < pairs; ++it) {
-          const int after = fetch(nxt);              // in flight while this tile's buffer is awaited
-          load_tile(cur, it);
-          publish(it + 2, after);
-          cur = nxt;
-          nxt = after;
+        // the tile after this one is pulled into L2 now: when its buffer frees, a period
+        // later, the TMA load finds it there (~0.8 k instead of ~1.8 k cycles)
+        const int next_row0 = row0 + 2 * clusters * kTileM;
+        if (pair + clusters < pairs && next_row0 < n) {
+          tma_prefetch_2d(&maps.h, 0, next_row0);
+          tma_prefetch_2d(&maps.h, 64, next_row0);
         }
-      } else {
-        uint32_t it = 0;
-        for (int pair = first_pair(); pair < pairs; pair = next_pair(pair, it), ++it) load_tile(pair, it);
       }
-    }
-    __syncwarp();
-    if (!DYN) {
-      // The whole warp runs the loop and waits; one elected lane issues (as in the MMA warp:
-      // issued from inside `if (lane == 0)` every TMA instruction came wrapped in an ELECT /
-      // R2UR.BROADCAST loop, ~70 instructions per tile on a warp that gets one issue slot in
-      // six -- between "buffer free" and "load issued", i.e. on the buffer's life cycle).
-      const bool issuer = elect_one();
-      if (issuer) prefetch_tmap(&maps.h);
-      uint32_t it = 0;
-      for (int pair = first_pair(); pair < pairs; pair = next_pair(pair, it), ++it) {
-        const uint32_t hb = it % kHBufs;
-        const int row0 = (2 * pair + int(rank)) * kTileM;
-        uint8_t *dst = hs + hb * kTileBytes;
-        mbar_wait_s(bar + kBarHEmpty + hb, ((it / kHBufs) & 1) ^ 1, p.sleep_ns);
-        if (issuer) {
-          trace_ev(p, it, 12);
-          mbar_arrive_expect_tx(bar + kBarHFull + hb, kTileBytes);
-          tma_load_2d(dst, &maps.h, 0, row0, bar + kBarHFull + hb);
-          tma_load_2d(dst + kKbBytes, &maps.h, 64, row0, bar + kBarHFull + hb);
-          // the tile after this one is pulled into L2 now: when its buffer frees, a period
-          // later, the TMA load finds it there (~0.8 k instead of ~1.8 k cycles)
-          const int next_row0 = row0 + 2 * clusters * kTileM;
-          if (pair + clusters < pairs && next_row0 < n && !(p.dbg & 2u)) {
-            tma_prefetch_2d(&maps.h, 0, next_row0);
-            tma_prefetch_2d(&maps.h, 64, next_row0);
-          }
-        }
-        __syncwarp();
-      }
+      __syncwarp();
     }
   } else {
     reg_dec<40>();                                // two spare warps of the utility warpgroup
@@ -777,11 +656,6 @@ fused_banded8_kernel(const __grid_constant__ Maps maps, const __grid_constant__ 
   __syncthreads();
   cluster_sync_all();                             // the peer may still be arriving on our barriers
   if (warp == kMmaWarp) tmem_dealloc2(tmem, kTmemCols);
-  if (p.trace != nullptr && tid == 0) {
-    unsigned long long ns;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(ns));
-    p.trace[1024 + 2 * blockIdx.x + 1] = (long long)ns;
-  }
 }
 
 }  // namespace v8
@@ -810,8 +684,6 @@ row_describe_kernel(const int32_t *__restrict__ row_ptr, const int32_t *__restri
   if (is(i + 2, 5)) { d |= kDescNext2; ++k; }
   desc[i] = k == end ? d : kDescGeneric;
 }
-
-extern long long *g_trace;              // gfx_fused6.cu (gfx_debug_fused_trace)
 
 int fused8_layer(const gfx_model *m, int layer, const __half *h, const int32_t *row_ptr,
                  const int32_t *col_src, const uint8_t *col_type, const uint32_t *desc, int64_t n,
@@ -843,65 +715,15 @@ int fused8_layer(const gfx_model *m, int layer, const __half *h, const int32_t *
   a.n = n; a.edge_dim = m->edge_dim;
   const uint32_t e16 = __half_as_ushort(__float2half_rn(m->eps1[layer]));
   a.eps1_h2 = e16 | (e16 << 16);
-  a.trace = g_trace;
-  static const uint32_t sleep_ns = [] {
-    const char *v = getenv("GFX_FUSED_SLEEP_NS");   // developer switch
-    return uint32_t(v ? atoi(v) : 64);
-  }();
-  a.sleep_ns = sleep_ns;
-  static const uint32_t dbg = [] {
-    const char *v = getenv("GFX_DBG");
-    return uint32_t(v ? atoi(v) : 0);
-  }();
-  a.dbg = dbg;
-  // GFX_SCHED=dynamic: tile pairs from an atomic counter.  Built to recover the 15 % spread of CTA
-  // durations under round-robin assignment (123 ... 143 us on a 603k-node chunk); measured on the
-  // same board it evens them out (139 ... 146 us) and the kernel takes the SAME time (0.145 vs
-  // 0.146 ms): the early finishers were not idle capacity, the aggregate rate of the chip (clock
-  // under load) is what is conserved.  Round-robin stays the default: no counter, no extra
-  // memset per launch.
-  static const bool dynamic = [] {
-    const char *v = getenv("GFX_SCHED");
-    return v && v[0] == 'd';
-  }();
-  if (dynamic) {
-    const uint32_t slot = m->sched_next.fetch_add(1u, std::memory_order_relaxed) % kSchedSlots;
-    a.sched = m->sched_counters + slot;
-    GFX_CUDA(cudaMemsetAsync(a.sched, 0, sizeof(uint32_t), st));
-  }
-  const bool dev = dynamic || a.dbg != 0u || a.trace != nullptr || a.sleep_ns != 64u;
-  auto kernel = dynamic ? v8::fused_banded8_kernel<true, true>
-                        : dev ? v8::fused_banded8_kernel<false, true> : v8::fused_banded8_kernel<false, false>;
-  GFX_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, v8::Smem::total));
+  GFX_CUDA(cudaFuncSetAttribute(v8::fused_banded8_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                v8::Smem::total));
   const int64_t tiles = (n + v8::kTileM - 1) / v8::kTileM;
   const int64_t pairs = (tiles + 1) / 2;
-  // as many CTA pairs as this GPU can hold at once (see gfx_fused6.cu)
-  static int resident[64] = {};                   // per device; 0 = not asked yet
-  int device = 0;
-  GFX_CUDA(cudaGetDevice(&device));
-  if (device >= 0 && device < 64 && resident[device] == 0) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(kNumSMs, 1, 1);
-    cfg.blockDim = dim3(v8::kWarps * 32, 1, 1);
-    cfg.dynamicSmemBytes = v8::Smem::total;
-    cudaLaunchAttribute attr;
-    attr.id = cudaLaunchAttributeClusterDimension;
-    attr.val.clusterDim.x = 2;
-    attr.val.clusterDim.y = 1;
-    attr.val.clusterDim.z = 1;
-    cfg.attrs = &attr;
-    cfg.numAttrs = 1;
-    int max_clusters = 0;
-    if (cudaOccupancyMaxActiveClusters(&max_clusters, kernel, &cfg) != cudaSuccess ||
-        max_clusters < 1) {
-      (void)cudaGetLastError();
-      max_clusters = kNumSMs / 2;
-    }
-    resident[device] = max_clusters < kNumSMs / 2 ? max_clusters : kNumSMs / 2;
-  }
-  const int cap = device >= 0 && device < 64 ? resident[device] : kNumSMs / 2;
+  int cap = 0;
+  rc = resident_pairs<v8::fused_banded8_kernel>(v8::kWarps * 32, v8::Smem::total, &cap);
+  if (rc) return rc;
   const int clusters = int(pairs < cap ? pairs : cap);
-  kernel<<<2 * clusters, v8::kWarps * 32, v8::Smem::total, st>>>(maps, c, a);
+  v8::fused_banded8_kernel<<<2 * clusters, v8::kWarps * 32, v8::Smem::total, st>>>(maps, c, a);
   GFX_LAUNCH_CHECK();
   return GFX_OK;
 }

@@ -1,9 +1,11 @@
 // Inline-PTX wrappers for CTA pairs (thread-block clusters of two, tcgen05 cta_group::2):
 // cluster rank and barrier, remote mbarrier arrives, paired TMEM allocation, M = 256 MMAs over
-// both CTAs' tiles with multicast completion, register reallocation between warpgroups.
+// both CTAs' tiles with multicast completion, register reallocation between warpgroups; and the
+// host-side count of CTA pairs a GPU holds at once.
 #pragma once
 #include <stdint.h>
 
+#include "gfx_common.cuh"
 #include "gfx_umma.cuh"
 
 namespace gfx {
@@ -84,4 +86,39 @@ __device__ __forceinline__ void reg_inc() {
 }
 
 }  // namespace ptx
+
+// *cap = how many CTA pairs of Kernel (2-CTA clusters of `threads` threads with `smem` bytes of
+// dynamic shared memory) the current GPU holds at once, at most one per TPC.  Persistent pair
+// kernels launch no more than that: which SMs are fused off differs from chip to chip, and a pair
+// that does not fit waits for a whole wave to finish.  Asked once per kernel and device (a
+// template instance per kernel, so two instantiations of one kernel template with different
+// shared memory keep separate answers); one pair per TPC when the query fails.
+template <auto Kernel>
+int resident_pairs(int threads, int smem, int *cap) {
+  static int resident[64] = {};                   // per device; 0 = not asked yet
+  int device = 0;
+  GFX_CUDA(cudaGetDevice(&device));
+  if (device >= 0 && device < 64 && resident[device] == 0) {
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(kNumSMs, 1, 1);
+    cfg.blockDim = dim3(threads, 1, 1);
+    cfg.dynamicSmemBytes = smem;
+    cudaLaunchAttribute attr;
+    attr.id = cudaLaunchAttributeClusterDimension;
+    attr.val.clusterDim.x = 2;
+    attr.val.clusterDim.y = 1;
+    attr.val.clusterDim.z = 1;
+    cfg.attrs = &attr;
+    cfg.numAttrs = 1;
+    int max_clusters = 0;
+    if (cudaOccupancyMaxActiveClusters(&max_clusters, Kernel, &cfg) != cudaSuccess || max_clusters < 1) {
+      (void)cudaGetLastError();
+      max_clusters = kNumSMs / 2;
+    }
+    resident[device] = max_clusters < kNumSMs / 2 ? max_clusters : kNumSMs / 2;
+  }
+  *cap = device >= 0 && device < 64 ? resident[device] : kNumSMs / 2;
+  return GFX_OK;
+}
+
 }  // namespace gfx

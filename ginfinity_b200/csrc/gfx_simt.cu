@@ -1,8 +1,6 @@
 // CUDA-core kernels: input projection, K1 neighbour aggregation (the HBM-bound
 // kernel of the path) and an fp32-accumulate MLP / head used for the
 // full-precision model and as the on-device cross-check of the tcgen05 path.
-#include <cstdlib>
-
 #include "gfx_common.cuh"
 #include "gfx_umma.cuh"
 
@@ -885,15 +883,9 @@ extern "C" int gfx_input_linear(const gfx_model *m, const float *x, int64_t n, v
   const int64_t rest = n - lead;
   if (dtype == GFX_F16) {
     __half *hh = static_cast<__half *>(h);
-    // the tensor-core kernel (gfx_input8.cu) when it applies; GFX_INPUT_SIMT=1: the SIMT kernels
-    static const bool simt = [] {
-      const char *v = getenv("GFX_INPUT_SIMT");
-      return v && *v && *v != '0';
-    }();
-    if (!simt) {
-      const int rc = input8_linear(m, x, n, hh, st);
-      if (rc != GFX_ERR_UNSUPPORTED) return rc;
-    }
+    // the tensor-core kernel (gfx_input8.cu) when it applies, else the SIMT kernels
+    const int rc = input8_linear(m, x, n, hh, st);
+    if (rc != GFX_ERR_UNSUPPORTED) return rc;
     if (lead) input_linear_kernel<__half><<<row_grid(lead), 256, 0, st>>>(x, m->w_in[1], m->b_in, lead, hh);
     if (rest)
       input_linear4_kernel<__half><<<row_grid((rest + 3) / 4), 256, 0, st>>>(
@@ -919,11 +911,7 @@ extern "C" int gfx_aggregate(const gfx_model *m, int layer, const void *h, const
   StageScope scope(GFX_STAGE_AGGREGATE, st, 1);
   const size_t toff = size_t(layer) * m->edge_dim * kHidden;
   if (dtype == GFX_F16) {
-    static const bool half_warp = [] {
-      const char *v = getenv("GFX_K1_HALFWARP");     // diagnostic: the previous kernel
-      return v && *v && *v != '0';
-    }();
-    if (!half_warp && n <= (int64_t(1) << kSrcBits)) {
+    if (n <= (int64_t(1) << kSrcBits)) {
       int64_t b = (n + 31) / 32;
       const int grid = int(b > 4 * kNumSMs ? 4 * kNumSMs : b);
       aggregate_f16_q_kernel<<<grid, 256, 0, st>>>(
@@ -935,11 +923,7 @@ extern "C" int gfx_aggregate(const gfx_model *m, int layer, const void *h, const
           m->edge_dim, m->eps1[layer], n, static_cast<__half *>(z));
     }
   } else if (dtype == GFX_F32) {
-    static const bool generic = [] {              // GFX_K1_F32_GENERIC=1: the unpipelined kernel
-      const char *v = getenv("GFX_K1_F32_GENERIC");
-      return v && *v && *v != '0';
-    }();
-    if (!generic && n <= (int64_t(1) << kSrcBits)) {
+    if (n <= (int64_t(1) << kSrcBits)) {
       int64_t b = (n + 15) / 16;
       const int grid = int(b > 2 * kNumSMs ? 2 * kNumSMs : b);
       aggregate_f32_h_kernel<<<grid, 256, 0, st>>>(

@@ -414,29 +414,8 @@ static int launch(const Consts &c, const Args &a, cudaStream_t st) {
   GFX_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
   const int64_t tiles = (a.n + kTileM - 1) / kTileM;
   const int64_t pairs = (tiles + 1) / 2;
-  static int resident[64] = {};                   // per device; 0 = not asked yet
-  int device = 0;
-  GFX_CUDA(cudaGetDevice(&device));
-  if (device >= 0 && device < 64 && resident[device] == 0) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(kNumSMs, 1, 1);
-    cfg.blockDim = dim3(kWarps * 32, 1, 1);
-    cfg.dynamicSmemBytes = smem;
-    cudaLaunchAttribute attr;
-    attr.id = cudaLaunchAttributeClusterDimension;
-    attr.val.clusterDim.x = 2;
-    attr.val.clusterDim.y = 1;
-    attr.val.clusterDim.z = 1;
-    cfg.attrs = &attr;
-    cfg.numAttrs = 1;
-    int max_clusters = 0;
-    if (cudaOccupancyMaxActiveClusters(&max_clusters, kernel, &cfg) != cudaSuccess || max_clusters < 1) {
-      (void)cudaGetLastError();
-      max_clusters = kNumSMs / 2;
-    }
-    resident[device] = max_clusters < kNumSMs / 2 ? max_clusters : kNumSMs / 2;
-  }
-  const int cap = device >= 0 && device < 64 ? resident[device] : kNumSMs / 2;
+  int cap = 0;
+  if (const int rc = resident_pairs<split_kernel<N1, HEAD>>(kWarps * 32, smem, &cap)) return rc;
   const int clusters = int(pairs < cap ? pairs : cap);
   kernel<<<2 * clusters, kWarps * 32, smem, st>>>(c, a);
   GFX_LAUNCH_CHECK();

@@ -62,7 +62,6 @@ RESIDENT_CHUNK_NODES = 1 << 22
 CHUNK_MICROBATCHES = 16
 RESIDENT_CHUNK_MICROBATCHES = 64
 GFX_GRAPH_BAD_EDGE = 16            # include/gfx.h
-_LAYER_KERNEL_CHOICE = {}          # device index -> (gfx_encode `fused` mode, {mode: ms})
 
 
 def _embedding_dtype(value) -> np.dtype:
@@ -216,18 +215,15 @@ class Ginfinity:
         # pairs with CSR-walking producers (bit-identical to 3; gfx_encode falls back where a
         # kernel does not apply), 0 = K1 + K2.  The default is FIXED (3, with 2 for shards that
         # hold context nodes): every process, rank and run computes with the same kernels, so an
-        # input encodes to the same bits fleet-wide.  K1 + K2 agree with the fused forms only to
-        # fp16 rounding (2e-3), so timing-based selection between them is opt-in:
-        # GFX_FUSED=auto times the forms once per device (_choose_layer_kernel); GFX_FUSED=0|2|3
-        # pins one.
-        env = os.environ.get("GFX_FUSED", "3")
-        self.fused = 0 if full_precision else (-1 if env in ("auto", "-1") else int(env))
-        self.layer_kernel_times = None    # {mode: ms} of the tuning chunk (GFX_FUSED=auto only)
+        # input encodes to the same bits fleet-wide (K1 + K2 agree with the fused forms only to
+        # fp16 rounding, 2e-3).  GFX_FUSED=0|2|3 pins one form.
+        self.fused = 0 if full_precision else int(os.environ.get("GFX_FUSED", "3"))
         self.chunk_nodes = DEFAULT_CHUNK_NODES
         self.resident_chunk_nodes = RESIDENT_CHUNK_NODES
         self.device_builder = True       # encode_many builds full-molecule graphs on the GPU
         # banded layer kernel: row descriptors from the edge list, CSR only for GENERIC rows
-        self.describe_from_edges = os.environ.get("GFX_DESCRIBE", "edges") != "csr"
+        # (False: every chunk through the CSR arrays, the path the tests compare against)
+        self.describe_from_edges = True
         self.last_microbatch_bounds: Optional[np.ndarray] = None
 
     def __del__(self):
@@ -351,8 +347,6 @@ class Ginfinity:
         the same bits, so a record encodes to the same values alone, in a batch, and next to
         windowed records; K1 + K2 (`GFX_FUSED=0`, full_precision) use the plain CSR."""
         lib = nat.lib
-        if self.fused < 0:
-            self._choose_layer_kernel()
         mode = int(self.fused)
         if mode == 3 and not banded:
             mode = 2
@@ -390,71 +384,6 @@ class Ginfinity:
         nat.check(lib.gfx_encode(self._handle, x, row_ptr.data_ptr(), col_src.data_ptr(),
                                  col_type.data_ptr(), out_row, n, out, act, out_code, self.impl, mode,
                                  enc_ws.data_ptr(), enc_ws_bytes, stream))
-
-    def _choose_layer_kernel(self) -> None:
-        """Once per device and process: encode a fixed synthetic chunk (2^19 nodes, banded RNA-like
-        graph) with the banded fused kernel, the fused pair kernel and K1 + K2, timed with CUDA
-        events, and keep the fastest.  The choice never depends on user data, so every encoder of a process on a given
-        GPU computes with the same kernels."""
-        key = self._torch_device.index
-        if key is None:
-            key = torch.cuda.current_device()
-        if key not in _LAYER_KERNEL_CHOICE:
-            _LAYER_KERNEL_CHOICE[key] = self._measure_layer_kernels()
-        self.fused, self.layer_kernel_times = _LAYER_KERNEL_CHOICE[key]
-
-    def _measure_layer_kernels(self, nodes: int = 1 << 19):
-        dev, lib = self._torch_device, nat.lib
-        with torch.cuda.device(dev):
-            stream = torch.cuda.current_stream().cuda_stream
-            i = torch.arange(nodes, device=dev, dtype=torch.int32)
-            src, dst, typ = [], [], []
-
-            def band(offset, code):
-                s_ = i + offset
-                ok = (s_ >= 0) & (s_ < nodes)
-                src.append(s_[ok]); dst.append(i[ok])
-                typ.append(torch.full((int(ok.sum()),), code, dtype=torch.uint8, device=dev))
-
-            # the reference builder's edge order (graph.py:494-561): backbone, pairs, skip-2
-            band(-1, 0)
-            band(1, 1)
-            mate = i ^ 32                                                  # a pair 32 nt away
-            src.append(mate); dst.append(i)
-            typ.append(torch.where(mate < i, 2, 3).to(torch.uint8))
-            band(-2, 4)
-            band(2, 5)
-            src, dst, typ = torch.cat(src), torch.cat(dst), torch.cat(typ)
-            e = int(src.shape[0])
-            x = torch.rand((nodes, 7), device=dev, dtype=torch.float32)
-            row_ptr = torch.empty(nodes + 1, dtype=torch.int32, device=dev)
-            col_src = torch.empty(e, dtype=torch.int32, device=dev)
-            col_type = torch.empty(e, dtype=torch.uint8, device=dev)
-            need = lib.gfx_csr_workspace_bytes(nodes, e)
-            ws = torch.empty(need, dtype=torch.uint8, device=dev)
-            nat.check(lib.gfx_csr_build(src.data_ptr(), dst.data_ptr(), typ.data_ptr(), nodes, e, 0,
-                                        row_ptr.data_ptr(), col_src.data_ptr(), col_type.data_ptr(),
-                                        ws.data_ptr(), need, stream))
-            need = lib.gfx_encode_workspace_bytes(nodes, nat.GFX_F16)
-            ews = torch.empty(need, dtype=torch.uint8, device=dev)
-            out = torch.empty((nodes, 128), dtype=torch.float16, device=dev)
-            times = {}
-            for mode in (3, 2, 0):
-                def run():
-                    nat.check(lib.gfx_encode(self._handle, x.data_ptr(), row_ptr.data_ptr(),
-                                             col_src.data_ptr(), col_type.data_ptr(), None, nodes,
-                                             out.data_ptr(), nat.GFX_F16, nat.GFX_F16, self.impl,
-                                             mode, ews.data_ptr(), need, stream))
-                run()                      # first use: module load, attributes, occupancy query
-                start = torch.cuda.Event(enable_timing=True)
-                stop = torch.cuda.Event(enable_timing=True)
-                start.record()
-                run()
-                run()
-                stop.record()
-                stop.synchronize()
-                times[mode] = start.elapsed_time(stop) / 2
-        return min(times, key=times.get), times
 
     # -- shard-level API (api.py:180-230) ------------------------------------
     def _check_request(self, spec, max_nodes_per_record, max_edges_per_record,

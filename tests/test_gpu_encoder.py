@@ -201,30 +201,18 @@ def test_synthetic_shard_matches_oracle_and_is_layout_invariant(gb, syn16, synth
     assert _cos(a, want).min() >= 0.9999
 
 
-def test_layer_kernel_is_fixed_and_all_forms_agree(gb, syn16, synthetic_state, monkeypatch):
+def test_fixed_layer_kernel_and_all_forms_agree(gb, syn16, synthetic_state, monkeypatch):
     """The fp16 model's layer runs as one kernel on CTA pairs (banded producers, or producers that
-    walk the CSR arrays: same bits) or as K1 + K2 (agrees to fp16 rounding only).  By default the
-    choice is FIXED (banded, pair for shards with context nodes) so that an input encodes to the
-    same bits on every board, rank and run; timing-based selection is opt-in (GFX_FUSED=auto), is
-    then made once per device and shared by every encoder of the process.  All forms stay within
-    the fp16-path tolerance of the oracle and of each other."""
-    from ginfinity_b200 import encoder as E
+    walk the CSR arrays: same bits) or as K1 + K2 (agrees to fp16 rounding only).  The choice is
+    FIXED (banded, pair for shards with context nodes) so that an input encodes to the same bits
+    on every board, rank and run.  All forms stay within the fp16-path tolerance of the oracle and
+    of each other."""
     shard = gb.GraphBuilder().build_shard(random_records(35, 120))
     monkeypatch.delenv("GFX_FUSED", raising=False)
     fresh = gb.Ginfinity.from_state(synthetic_state, device="cuda:0")
-    assert fresh.fused == 3 and fresh.layer_kernel_times is None
+    assert fresh.fused == 3
     auto = np.concatenate(fresh.encode_graphs(shard, embedding_dtype=np.float32))
     assert fresh.fused == 3                                # nothing was timed, nothing changed
-    monkeypatch.setenv("GFX_FUSED", "auto")
-    tuned = gb.Ginfinity.from_state(synthetic_state, device="cuda:0")
-    assert tuned.fused == -1
-    tuned.encode_graphs(shard)
-    assert tuned.fused in (0, 2, 3) and set(tuned.layer_kernel_times) == {0, 2, 3}
-    assert E._LAYER_KERNEL_CHOICE[0][0] == tuned.fused
-    other = gb.Ginfinity.from_state(synthetic_state, device="cuda:0")
-    other.encode_graphs(shard)
-    assert other.fused == tuned.fused                      # same choice, not re-measured
-    monkeypatch.delenv("GFX_FUSED")
     outs = {}
     for mode in (0, 2, 3):
         pinned = gb.Ginfinity.from_state(synthetic_state, device="cuda:0")
@@ -254,9 +242,10 @@ def test_layer_kernel_is_fixed_and_all_forms_agree(gb, syn16, synthetic_state, m
 
 def test_full_precision_from_row_descriptors_equals_the_csr_path(gb, synthetic_state):
     """full_precision=True: K1 from row descriptors (gfx_encode_described_f32, the default for
-    full-molecule shards) gives the bits of K1 on the CSR arrays (GFX_DESCRIBE=csr), over several
-    chunks and microbatches, host path and device-resident path; a shard whose edge order is not
-    the reference builder's takes the CSR kernel through the device flag and still agrees."""
+    full-molecule shards) gives the bits of K1 on the CSR arrays (describe_from_edges = False),
+    over several chunks and microbatches, host path and device-resident path; a shard whose edge
+    order is not the reference builder's takes the CSR kernel through the device flag and still
+    agrees."""
     from ginfinity_b200.encoder import DeviceShard
     enc = gb.Ginfinity.from_state(synthetic_state, device="cuda:0", full_precision=True)
     shard = gb.GraphBuilder().build_shard(random_records(37, 120))

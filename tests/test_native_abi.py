@@ -61,32 +61,45 @@ def test_library_is_sm_100a_and_uses_the_blackwell_units(nat):
     assert "STTM" in sass              # tcgen05.st: the hidden activation goes back into TMEM
 
 
+def _kernels_sass(sass: str, needle: str) -> list:
+    """SASS text of every kernel whose (mangled) name contains `needle`."""
+    parts = sass.split("Function : ")
+    return [p for p in parts if needle in p.split("\n", 1)[0]]
+
+
 def _kernel_sass(sass: str, needle: str) -> str:
     """SASS text of the first kernel whose (mangled) name contains `needle`."""
-    parts = sass.split("Function : ")
-    body = [p for p in parts if needle in p.split("\n", 1)[0]]
+    body = _kernels_sass(sass, needle)
     assert body, needle
     return body[0]
 
 
 @pytest.mark.skipif(shutil.which("cuobjdump") is None, reason="cuobjdump is not installed here")
-def test_layer_kernel_issuers_use_uniform_registers(nat):
-    """The banded layer kernel follows its executed-instruction count (DESIGN.md 9.1): the
-    production instance must not carry the developer tests, and its MMA / TMA issuers must be
+def test_each_layer_kernel_is_one_build_with_uniform_issuers(nat):
+    """The layer kernels follow their executed-instruction count (DESIGN.md 9.1): each is built
+    once, with no timeline stamps, and the banded kernel's MMA / TMA issuers must be
     warp-converged with one elected lane -- issued from inside `if (lane == 0)` every
     tcgen05.mma / TMA instruction comes wrapped in an ELECT / R2UR.BROADCAST / BRA.U.ANY loop."""
     sass = subprocess.run(["cuobjdump", "-sass", str(LIB)], capture_output=True, text=True).stdout
-    production = _kernel_sass(sass, "fused_banded8_kernelILb0ELb0")
-    developer = _kernel_sass(sass, "fused_banded8_kernelILb0ELb1")
-    assert production.count("UTCHMMA.2CTA") == 24          # 8 (GEMM 1, N = 256) + 16 (GEMM 2)
-    assert "R2UR.BROADCAST" not in production
-    assert "CS2R" not in production.split("USETMAXREG")[1]  # no clock64 stamps in epilogue A's loop
-    n_prod = sum(1 for line in production.splitlines() if "/*" in line and ";" in line)
-    n_dev = sum(1 for line in developer.splitlines() if "/*" in line and ";" in line)
-    assert n_prod < n_dev
+    banded = _kernels_sass(sass, "fused_banded8_kernel")
+    pair = _kernels_sass(sass, "fused_pair_kernel")
+    assert len(banded) == 1 and len(pair) == 1
+    for body in banded + pair:
+        assert "SR_CLOCKLO" not in body and "SR_GLOBALTIMER" not in body
+    assert banded[0].count("UTCHMMA.2CTA") == 24           # 8 (GEMM 1, N = 256) + 16 (GEMM 2)
+    assert pair[0].count("UTCHMMA.2CTA") == 24             # the same GEMMs
+    assert "R2UR.BROADCAST" not in banded[0]
     # the same for the top-k scan's MMA issuer
     scan = _kernel_sass(sass, "topk_scan")
     assert scan.count("R2UR.BROADCAST") <= 2 * scan.count("UTMALDG")   # none left around the MMAs
+
+
+def test_library_reads_no_environment():
+    """Which kernel runs, and what it computes, depends on the arguments alone: no source file of
+    the library reads an environment variable."""
+    readers = [path.name for path in sorted((ROOT / "ginfinity_b200" / "csrc").glob("*.cu*"))
+               if "getenv" in path.read_text()]
+    assert readers == []
 
 
 def test_argument_errors_surface_through_gfx_last_error(nat):

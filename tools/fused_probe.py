@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Developer probe: run a fused layer entry point (argv[1]: gfx_layer_fused_pair or
-gfx_layer_fused_pair, default the pair kernel) a few times on a synthetic
+gfx_layer_fused_banded, default the pair kernel) a few times on a synthetic
 graph, for ncu captures."""
 import sys
 from pathlib import Path

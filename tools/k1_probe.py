@@ -1,7 +1,5 @@
 #!/usr/bin/env python
-"""Developer probe: K1 (gfx_aggregate, fp16) time on a tiled synthetic shard; argv[1] = nodes.
-Environment switches of the kernel (GFX_K1_WAVES, GFX_K1_HALFWARP) are read once per process."""
-import os
+"""Developer probe: K1 (gfx_aggregate, fp16) time on a tiled synthetic shard; argv[1] = nodes."""
 import sys
 from pathlib import Path
 
@@ -51,5 +49,5 @@ b.record()
 torch.cuda.synchronize()
 t = a.elapsed_time(b) / 20 * 1e-3
 alg = N * 516 + E * 5
-print(f"K1 waves={os.environ.get('GFX_K1_WAVES', '1')} N={N} E={E}: {t * 1e3:.4f} ms  {t / N * 1e9:.4f} ns/node  "
+print(f"K1 N={N} E={E}: {t * 1e3:.4f} ms  {t / N * 1e9:.4f} ns/node  "
       f"{alg / t / 1e9:.0f} GB/s algorithmic")

@@ -4,7 +4,7 @@ Exports the names a user of the reference package imports for this path
 (src/ginfinity/__init__.py:14-36), so `import ginfinity_b200 as ginfinity` is the
 whole migration.  The data plane (records, graph specification, graphs,
 shards and their files) is importable anywhere; `Ginfinity`, `DeviceShard`,
-`EmbeddingIndex` and `align_pairs` need the built libgfx.so and a CUDA device and are resolved on
+`EmbeddingIndex`, `align_pairs` and `align_paths` need the built libgfx.so and a CUDA device and are resolved on
 first use -- they fail loudly without them, there is no CPU fallback.
 """
 import importlib
@@ -26,7 +26,8 @@ _EAGER = {
 }
 # name -> submodule that is imported only when the name is first touched (needs the GPU library)
 _LAZY = {"Ginfinity": "encoder", "DeviceShard": "encoder", "default_alignment_parameters": "encoder",
-         "EmbeddingIndex": "search", "align_pairs": "align", "Alignments": "align"}
+         "EmbeddingIndex": "search", "align_pairs": "align", "Alignments": "align",
+         "align_paths": "align", "AlignmentPaths": "align"}
 
 for _module, _names in _EAGER.items():
     for _name in _names:

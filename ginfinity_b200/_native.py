@@ -94,6 +94,9 @@ _SIGNATURES = {
     "gfx_align_workspace_bytes": (_sz, [_i64, _i64]),
     "gfx_align": (C.c_int, [_p, _i64, _p, _i64, _p, _i64, C.c_float, C.c_float, C.c_float,
                             _p, _p, _p, _sz, _p]),
+    "gfx_align_trace_workspace_bytes": (_sz, [_i64, _i64]),
+    "gfx_align_trace": (C.c_int, [_p, _i64, _p, _i64, _p, _i64, C.c_float, C.c_float, C.c_float,
+                                  _p, _p, _p, _p, _p, _p, _sz, _p]),
     "gfx_profile_enable": (C.c_int, [C.c_uint32]),
     "gfx_profile_read": (C.c_int, [C.c_int, C.POINTER(C.c_double), C.POINTER(_i64), C.c_int]),
     "gfx_launch_counts": (C.c_int, [C.POINTER(_i64), C.c_int]),

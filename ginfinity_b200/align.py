@@ -1,5 +1,6 @@
 """Local alignment of per-nucleotide embeddings (Smith-Waterman, affine gaps)
-on the GPU: K8 of libgfx.so (csrc/gfx_align.cu).
+on the GPU: K8 of libgfx.so (csrc/gfx_align.cu).  `align_pairs` gives each
+pair's score and region, `align_paths` also the aligned path.
 
 The reference ships scoring parameters for a separate aligner
 (`alignment-config`, src/ginfinity/api.py:47-50) but not the aligner, so the
@@ -20,6 +21,9 @@ from .records import MAXIMUM_LENGTH_NT
 
 DIM = 128
 MAX_SEGMENT = MAXIMUM_LENGTH_NT
+# align_paths: bytes of DP pointer record per gfx_align_trace call (4 bits per cell of the boxes
+# in the call).  One 4096 x 4096 box takes 8 MiB, so a single box always fits.
+CODE_BUDGET = 1 << 30
 
 
 class Alignments(NamedTuple):
@@ -86,6 +90,132 @@ def align_pairs(queries, targets, pairs, *, offset: float, gap_open: float,
 
     Float32 embeddings are not supported; cast them to float16.
     """
+    score, coords = _score_pass(_prepare(queries, targets, pairs, offset, gap_open, gap_extend, device))
+    return Alignments(score, *coords.unbind(1))
+
+
+class AlignmentPaths(NamedTuple):
+    """The aligned path of each pair, on the device.  Pair p's path is
+    ops[offsets[p] : offsets[p] + lengths[p]], one op per step from
+    (query_begin, target_begin) to (query_end - 1, target_end - 1):
+    0 = M (query row with target row), 1 = I (query row with a gap),
+    2 = D (target row with a gap)."""
+    ops: torch.Tensor            # uint8
+    offsets: torch.Tensor        # int64 [P]
+    lengths: torch.Tensor        # int32 [P]
+
+    def cigars(self) -> list:
+        """SAM-style run-length strings, one per pair ("12M2I30M1D5M"; "" for a
+        pair without an alignment), from one device-to-host copy."""
+        P = len(self.lengths)
+        buf = torch.cat([self.offsets.to(torch.int64).contiguous().view(torch.uint8),
+                         self.lengths.to(torch.int32).contiguous().view(torch.uint8),
+                         self.ops.reshape(-1).view(torch.uint8)]).cpu().numpy()
+        offsets = buf[:8 * P].view(np.int64)
+        lengths = buf[8 * P:12 * P].view(np.int32)
+        ops = buf[12 * P:]
+        out = []
+        for o, n in zip(offsets.tolist(), lengths.tolist()):
+            path = ops[o:o + n]
+            if n <= 0:
+                out.append("")
+                continue
+            ends = np.flatnonzero(np.diff(path)).tolist() + [n - 1]
+            begin, parts = 0, []
+            for e in ends:
+                parts.append(f"{e - begin + 1}{'MID'[path[e]]}")
+                begin = e + 1
+            out.append("".join(parts))
+        return out
+
+
+def align_paths(queries, targets, pairs, *, offset: float, gap_open: float,
+                gap_extend: float, device=None) -> tuple:
+    """`align_pairs` and the aligned path of every pair: (Alignments,
+    AlignmentPaths).  Arguments, validation and errors are those of
+    `align_pairs`, and the Alignments are the same bits.
+
+    The path is the one the tie rules of `align_pairs` define: followed back
+    from the end cell, H takes the first of diagonal, E, F that attains it, E
+    and F prefer opening to extending, and a diagonal step from H = 0 is the
+    start.  It starts and ends with M; #M + #I = query_end - query_begin and
+    #M + #D = target_end - target_begin.  A pair with score 0 has an empty
+    path.  Rescoring the path in fp32 gives the score bit for bit: v = 0 + s
+    at the first M, then + s per M, - gap_open per gap opened (after M or
+    after the other gap kind), - gap_extend per gap extended.
+
+    How: after the score pass the coordinates come back to the host (16 bytes
+    per pair, one synchronisation).  The DP then runs again over each pair's
+    box [query_begin, query_end) x [target_begin, target_end) only, recording
+    4 bits per cell, and a walk follows them back from the box's corner.
+    Inside the box every value is at most its value in the whole segments and
+    equal along the path, so the box pass must return the same score at
+    (0, h, 0, w); a pair where it does not raises RuntimeError (a library
+    bug, never a wrong path).  Boxes run in calls of at most CODE_BUDGET
+    bytes of pointer record.
+    """
+    pr = _prepare(queries, targets, pairs, offset, gap_open, gap_extend, device)
+    score, coords = _score_pass(pr)
+    dev, P = pr.dev, len(pr.pairs)
+    lengths = torch.zeros(P, dtype=torch.int32, device=dev)
+    if P == 0:
+        return (Alignments(score, *coords.unbind(1)),
+                AlignmentPaths(torch.empty(0, dtype=torch.uint8, device=dev),
+                               torch.empty(0, dtype=torch.int64, device=dev), lengths))
+    qb, qe, tb, te = coords.cpu().numpy().astype(np.int64).T
+    has = qb >= 0
+    h, w = np.where(has, qe - qb, 0), np.where(has, te - tb, 0)
+    boxes = np.stack([pr.pairs[:, 0] + np.maximum(qb, 0), h, pr.pairs[:, 2] + np.maximum(tb, 0), w], 1)
+    want = np.where(has[:, None], np.stack([np.zeros(P, np.int64), h, np.zeros(P, np.int64), w], 1), -1)
+    cap = np.maximum(h + w - 1, 0)
+    offsets = np.concatenate([[0], np.cumsum(cap)[:-1]]).astype(np.int64)
+    total = int(cap.sum())
+    code_end = np.cumsum(h * ((w + 31) // 32) * 16)
+    boxes_dev = torch.from_numpy(boxes.astype(np.int64)).to(dev, non_blocking=True)
+    want_dev = torch.from_numpy(want.astype(np.int32)).to(dev, non_blocking=True)
+    offsets_dev = torch.from_numpy(offsets).to(dev, non_blocking=True)
+    ops = torch.empty(max(total, 1), dtype=torch.uint8, device=dev)
+    box_score = torch.empty(P, dtype=torch.float32, device=dev)
+    box_coords = torch.empty((P, 4), dtype=torch.int32, device=dev)
+    go, ge, th = pr.params
+    q, t = pr.q, pr.t
+    with torch.cuda.device(dev):
+        stream = torch.cuda.current_stream().cuda_stream
+        a = 0
+        while a < P:
+            done = int(code_end[a - 1]) if a else 0
+            b = max(int(np.searchsorted(code_end, done + CODE_BUDGET, side="right")), a + 1)
+            need = nat.lib.gfx_align_trace_workspace_bytes(b - a, int(code_end[b - 1]) - done)
+            ws = torch.empty(need, dtype=torch.uint8, device=dev)
+            nat.check(nat.lib.gfx_align_trace(
+                q.data_ptr() if len(q) else None, len(q), t.data_ptr() if len(t) else None, len(t),
+                boxes_dev[a:].data_ptr(), b - a, th, go, ge, box_score[a:].data_ptr(),
+                box_coords[a:].data_ptr(), ops.data_ptr(), offsets_dev[a:].data_ptr(),
+                lengths[a:].data_ptr(), ws.data_ptr(), need, stream))
+            a = b
+    bad = ((box_score.view(torch.int32) != score.view(torch.int32)) | (box_coords != want_dev).any(1)
+           | (lengths < 0))
+    if bool(bad.any()):
+        p = int(torch.nonzero(bad)[0])
+        raise RuntimeError(
+            f"align_paths: pair {p}: the pass over its box [{int(boxes[p, 0])}, +{int(h[p])}) x "
+            f"[{int(boxes[p, 2])}, +{int(w[p])}) gave score {float(box_score[p])} at "
+            f"{tuple(int(v) for v in box_coords[p].tolist())}, path length {int(lengths[p])}; the score "
+            f"pass gave {float(score[p])}")
+    return Alignments(score, *coords.unbind(1)), AlignmentPaths(ops[:total], offsets_dev, lengths)
+
+
+class _Problem(NamedTuple):
+    q: torch.Tensor
+    t: torch.Tensor
+    pairs: np.ndarray            # int64 [P, 4], host
+    pairs_dev: torch.Tensor
+    max_t: int
+    params: list                 # gap_open, gap_extend, offset as float32 values
+    dev: torch.device
+
+
+def _prepare(queries, targets, pairs, offset, gap_open, gap_extend, device) -> _Problem:
     go, ge, th = _parameters(offset, gap_open, gap_extend)
     q = _table(queries, "queries")
     t = q if targets is queries else _table(targets, "targets")
@@ -96,22 +226,29 @@ def align_pairs(queries, targets, pairs, *, offset: float, gap_open: float,
     dev = _device(device, queries, targets)
     q = q.to(dev, non_blocking=True).contiguous()
     t = q if targets is queries else t.to(dev, non_blocking=True).contiguous()
-    P = len(pairs_host)
-    score = torch.empty(P, dtype=torch.float32, device=dev)
-    coords = torch.empty((P, 4), dtype=torch.int32, device=dev)
-    if P:
+    pairs_dev = None
+    if len(pairs_host):
         if isinstance(pairs, torch.Tensor) and pairs.device == dev:
             pairs_dev = pairs.to(torch.int64).contiguous()
         else:
             pairs_dev = torch.from_numpy(pairs_host).to(dev, non_blocking=True)
+    return _Problem(q, t, pairs_host, pairs_dev, max_t, [go, ge, th], dev)
+
+
+def _score_pass(pr: _Problem):
+    q, t, P, dev = pr.q, pr.t, len(pr.pairs), pr.dev
+    go, ge, th = pr.params
+    score = torch.empty(P, dtype=torch.float32, device=dev)
+    coords = torch.empty((P, 4), dtype=torch.int32, device=dev)
+    if P:
         with torch.cuda.device(dev):
-            need = nat.lib.gfx_align_workspace_bytes(P, max_t)
+            need = nat.lib.gfx_align_workspace_bytes(P, pr.max_t)
             ws = torch.empty(need, dtype=torch.uint8, device=dev)
             nat.check(nat.lib.gfx_align(
                 q.data_ptr() if len(q) else None, len(q), t.data_ptr() if len(t) else None, len(t),
-                pairs_dev.data_ptr(), P, th, go, ge, score.data_ptr(), coords.data_ptr(),
+                pr.pairs_dev.data_ptr(), P, th, go, ge, score.data_ptr(), coords.data_ptr(),
                 ws.data_ptr(), need, torch.cuda.current_stream().cuda_stream))
-    return Alignments(score, *coords.unbind(1))
+    return score, coords
 
 
 def _parameters(offset, gap_open, gap_extend):

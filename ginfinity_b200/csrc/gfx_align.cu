@@ -24,6 +24,13 @@
 // Each DP warp reduces its rows' best cell per pair into `parts`; a second
 // kernel picks the end cell of each pair by the tie rule.
 //
+// Traceback (gfx_align_trace) runs the same kernel with kTrace: each lane also records a
+// 4-bit code per cell of its row (kCode* below), 32 columns to a uint4, stored every 32
+// steps into the pair's pointer block (q_len rows x ceil(t_len/32) uint4, row-major).  In
+// the last block of a row of t_len % 32 = r != 0 columns, column j sits at nibble
+// 32 - r + (j & 31): the codes are shifted in from the top and the block is stored as it is.
+// A walk kernel then follows the codes back from the end cell, one warp per pair.
+//
 // Arithmetic per cell, fp32 round-to-nearest in this order (gfx.h):
 //   s = S - theta;  E = max(H_left - go, E_left - ge);  F = max(H_up - go, F_up - ge)
 //   H = max(0, H_diag + s, E, F)
@@ -79,7 +86,15 @@ struct Args {
   unsigned long long *counter;
   float4 *rowbuf;         // [gridDim.x][row_cap]: (H, F, start H, start F) of warp 3's bottom row
   int row_cap;            // columns of rowbuf per CTA: the longest target of a multi-stripe pair
+  // kTrace only
+  uint8_t *codes;         // pointer blocks
+  const int64_t *code_off;  // [P] byte offset of each pair's block in `codes`; -1: it did not fit
 };
+
+// Cell codes of the traceback: bits 0-1 where H came from, bit 2 E opened (else extended),
+// bit 3 F opened.  H's source follows the tie rule: zero when H = 0, else the first of
+// diagonal, E, F that attains it.
+enum Code : uint32_t { kCodeZero = 0, kCodeDiag = 1, kCodeE = 2, kCodeF = 3, kCodeEOpen = 4, kCodeFOpen = 8 };
 
 // Accuracy of S, relative: |S - q.t| <= kAlignRel |q| |t|.  The tensor-core sum is the same
 // fp16-product, fp32-accumulate dot product as the top-k scan, so the argument of kCertRel in
@@ -90,10 +105,22 @@ struct Args {
 // roundings of 2^-24 relative.  This rests on that argument, not on a measurement.
 [[maybe_unused]] constexpr float kAlignRel = 1.f / 16384.f;
 
-// Workspace: the pair counter, then parts, then the per-CTA rows.
+// Workspace: the pair counter, then parts, then the per-CTA rows.  gfx_align_trace puts the
+// pointer-block offsets after parts, then per-CTA rows of kMaxLen columns, then the blocks.
 constexpr size_t kHeaderBytes = 256;
 inline size_t parts_bytes(int64_t P) { return align256(size_t(P) * 4 * 16); }
 inline int grid_for(int64_t P) { return int(P < kNumSMs ? (P > 0 ? P : 1) : kNumSMs); }
+inline size_t trace_fixed_bytes(int64_t P) {
+  return kHeaderBytes + parts_bytes(P) + align256(size_t(P) * 8) + size_t(grid_for(P)) * kMaxLen * 16;
+}
+
+// the limits of gfx.h, and a per-CTA row for a multi-stripe pair (the producer writes the same
+// test out in full: as a call it changes the score instance's predicate allocation)
+__device__ __forceinline__ bool pair_valid(int64_t qs, int64_t ql, int64_t ts, int64_t tl, const Args &a) {
+  return qs >= 0 && ql >= 0 && ql <= kMaxLen && qs <= a.q_rows - ql && ts >= 0 && tl >= 0 &&
+         tl <= kMaxLen && ts <= a.t_rows - tl && (ql <= kTile || tl <= a.row_cap);
+}
+__device__ __forceinline__ int64_t code_bytes(int64_t ql, int64_t tl) { return ql * ((tl + 31) / 32) * 16; }
 
 __device__ __forceinline__ float max3(float a, float b, float c) {
   float r;
@@ -121,11 +148,14 @@ struct Dp {
   uint32_t sH, sE, sF, sHd;        // their starts, (i << 16) | j
   float cur;                       // best H of the row so far (+inf: row outside the segment)
   uint32_t best_end, best_start, ibase;
+  uint32_t c0, c1, c2, c3;         // kTrace: codes of the last 32 cells, the newest in c3's top nibble
+  uint4 *crow;                     // kTrace: this row's codes
+  int clast;                       // kTrace: last column stored (t_len - 1; -1 past the segment)
 };
 
 // Anti-diagonal steps k0 .. k1-1: lane computes cell (row, k - lane).  FILL: some lanes are
 // left of column 0 (k < 31); DRAIN: some are right of the last column (k >= t_len).
-template <bool FILL, bool DRAIN>
+template <bool TRACE, bool FILL, bool DRAIN>
 __device__ __forceinline__ void dp_steps(Dp &d, int k0, int k1, int lane, const float *srow,
                                          const float4 *top, float4 *out, int t_len, float theta,
                                          float go, float ge) {
@@ -165,6 +195,16 @@ __device__ __forceinline__ void dp_steps(Dp &d, int k0, int k1, int lane, const 
     d.sH = sHn;
     d.sE = sEn;
     d.sF = sFn;
+    if constexpr (TRACE) {
+      const uint32_t src = Hn == 0.f ? kCodeZero : dg == Hn ? kCodeDiag : En == Hn ? kCodeE : kCodeF;
+      const uint32_t c = src | (eo >= ee ? kCodeEOpen : 0u) | (fo >= fe ? kCodeFOpen : 0u);
+      d.c0 = __funnelshift_r(d.c0, d.c1, 4);
+      d.c1 = __funnelshift_r(d.c1, d.c2, 4);
+      d.c2 = __funnelshift_r(d.c2, d.c3, 4);
+      d.c3 = __funnelshift_r(d.c3, c, 4);
+      // the last column of a 32-column block, or of the row
+      if (j == min(j | 31, d.clast) && (!FILL || j >= 0)) d.crow[j >> 5] = make_uint4(d.c0, d.c1, d.c2, d.c3);
+    }
     if (Hn > d.cur && (!DRAIN || unsigned(j) < unsigned(t_len))) {
       d.cur = Hn;
       d.best_end = d.ibase | uint32_t(j);
@@ -174,6 +214,7 @@ __device__ __forceinline__ void dp_steps(Dp &d, int k0, int k1, int lane, const 
   }
 }
 
+template <bool kTrace>
 __global__ void __launch_bounds__(kThreads, 1)
 align_kernel(const __grid_constant__ Maps maps, const Args a) {
   using L = Smem;
@@ -225,7 +266,8 @@ align_kernel(const __grid_constant__ Maps maps, const Args a) {
       const int64_t qs = __shfl_sync(0xffffffffu, v, 0), ql = __shfl_sync(0xffffffffu, v, 1);
       const int64_t ts = __shfl_sync(0xffffffffu, v, 2), tl = __shfl_sync(0xffffffffu, v, 3);
       const bool valid = qs >= 0 && ql >= 0 && ql <= kMaxLen && qs <= a.q_rows - ql && ts >= 0 && tl >= 0 &&
-                         tl <= kMaxLen && ts <= a.t_rows - tl && (ql <= kTile || tl <= a.row_cap);
+                         tl <= kMaxLen && ts <= a.t_rows - tl && (ql <= kTile || tl <= a.row_cap) &&
+                         (!kTrace || a.code_off[p] >= 0);
       if (!valid || ql == 0 || tl == 0) {
         // nothing to align: score 0 (or NaN for a pair the caller should not have passed)
         if (lane < kDpWarps)
@@ -296,6 +338,8 @@ align_kernel(const __grid_constant__ Maps maps, const Args a) {
       const int q_len = reinterpret_cast<const volatile int *>(dsc)[1];
       const int t_len = reinterpret_cast<const volatile int *>(dsc)[2];
       const int stripes = (q_len + kTile - 1) / kTile, tiles = (t_len + kTile - 1) / kTile;
+      uint4 *cblock = nullptr;
+      if constexpr (kTrace) cblock = reinterpret_cast<uint4 *>(a.codes + a.code_off[p]);
       float best = 0.f;                       // best H of this lane's rows, strictly positive to count
       uint32_t best_end = ~0u, best_start = 0;
       for (int s = 0; s < stripes; ++s) {
@@ -323,6 +367,11 @@ align_kernel(const __grid_constant__ Maps maps, const Args a) {
         st.E = st.F = ninf;
         st.Hd = 0.f;
         st.sH = st.sE = st.sF = st.sHd = 0;
+        if constexpr (kTrace) {
+          st.c0 = st.c1 = st.c2 = st.c3 = 0;
+          st.crow = cblock + size_t(row) * ((t_len + 31) / 32);
+          st.clast = row < q_len ? t_len - 1 : -1;
+        }
         const float *srow = slab + lane * kSlabRow;
         const float4 *in_cur = in_ring;
         float4 *out_even = nullptr, *out_odd = nullptr;   // lane 31's destination for even / odd tiles
@@ -396,11 +445,11 @@ align_kernel(const __grid_constant__ Maps maps, const Args a) {
           if (k < t_len && t_len < next) next = t_len;
           if (kend < next) next = kend;
           if (k < 31) {
-            if (k < t_len) dp_steps<true, false>(st, k, next, lane, srow, in_cur, out, t_len, theta, go, ge);
-            else dp_steps<true, true>(st, k, next, lane, srow, in_cur, out, t_len, theta, go, ge);
+            if (k < t_len) dp_steps<kTrace, true, false>(st, k, next, lane, srow, in_cur, out, t_len, theta, go, ge);
+            else dp_steps<kTrace, true, true>(st, k, next, lane, srow, in_cur, out, t_len, theta, go, ge);
           } else {
-            if (k < t_len) dp_steps<false, false>(st, k, next, lane, srow, in_cur, out, t_len, theta, go, ge);
-            else dp_steps<false, true>(st, k, next, lane, srow, in_cur, out, t_len, theta, go, ge);
+            if (k < t_len) dp_steps<kTrace, false, false>(st, k, next, lane, srow, in_cur, out, t_len, theta, go, ge);
+            else dp_steps<kTrace, false, true>(st, k, next, lane, srow, in_cur, out, t_len, theta, go, ge);
           }
           k = next;
         }
@@ -454,6 +503,135 @@ align_finish_kernel(const float4 *__restrict__ parts, int64_t P, float *__restri
   }
 }
 
+// kTrace: byte offset of each pair's pointer block, in pair order (one block of 1024 threads,
+// an exclusive scan 1024 pairs at a time).  A block that ends past `capacity` gets -1.
+__global__ void __launch_bounds__(1024) align_code_offsets_kernel(const Args a, int64_t capacity) {
+  __shared__ int64_t warp_sum[32];
+  __shared__ int64_t carry;
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  int64_t *off = const_cast<int64_t *>(a.code_off);
+  if (tid == 0) carry = 0;
+  __syncthreads();
+  for (int64_t base = 0; base < a.num_pairs; base += 1024) {
+    const int64_t p = base + tid;
+    int64_t bytes = 0;
+    if (p < a.num_pairs) {
+      const int64_t qs = a.pairs[p * 4], ql = a.pairs[p * 4 + 1], ts = a.pairs[p * 4 + 2], tl = a.pairs[p * 4 + 3];
+      if (pair_valid(qs, ql, ts, tl, a)) bytes = code_bytes(ql, tl);
+    }
+    int64_t x = bytes;                     // inclusive scan over the warp
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const int64_t y = __shfl_up_sync(0xffffffffu, x, o);
+      if (lane >= o) x += y;
+    }
+    if (lane == 31) warp_sum[warp] = x;
+    __syncthreads();
+    if (warp == 0) {
+      int64_t v = warp_sum[lane];
+#pragma unroll
+      for (int o = 1; o < 32; o <<= 1) {
+        const int64_t y = __shfl_up_sync(0xffffffffu, v, o);
+        if (lane >= o) v += y;
+      }
+      warp_sum[lane] = v;
+    }
+    __syncthreads();
+    const int64_t end = carry + (warp > 0 ? warp_sum[warp - 1] : 0) + x;
+    if (p < a.num_pairs) off[p] = end <= capacity ? end - bytes : -1;
+    __syncthreads();
+    if (tid == 1023) carry = end;
+    __syncthreads();
+  }
+}
+
+// The traceback: one warp per pair, from the end cell the finish kernel picked.  The lanes
+// stage the 32 rows x 32 columns of codes that end at the current cell (one uint4 each);
+// lane 0 walks them until the path leaves that block, collecting ops in reverse.  A walk
+// that does not end at the reported start (or leaves the segments) gets length -1.
+constexpr int kWalkWarps = 4;
+constexpr int kMaxPath = 2 * kMaxLen - 1;
+
+__global__ void __launch_bounds__(kWalkWarps * 32)
+align_walk_kernel(const int64_t *__restrict__ pairs, int64_t P, const int64_t *__restrict__ code_off,
+                  const uint8_t *__restrict__ codes, const float *__restrict__ score,
+                  const int4 *__restrict__ coords, const int64_t *__restrict__ op_off,
+                  uint8_t *__restrict__ ops, int32_t *__restrict__ out_len) {
+  __shared__ uint4 stage_all[kWalkWarps][32];
+  __shared__ uint8_t rev_all[kWalkWarps][kMaxPath + 1];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int64_t p = int64_t(blockIdx.x) * kWalkWarps + warp;
+  if (p >= P) return;
+  if (!(score[p] > 0.f)) {
+    if (lane == 0) out_len[p] = 0;
+    return;
+  }
+  const int4 c = coords[p];
+  const int t_len = int(pairs[p * 4 + 3]);
+  const int stride = (t_len + 31) / 32, rem = t_len & 31;
+  const uint4 *blk = reinterpret_cast<const uint4 *>(codes + code_off[p]);
+  uint4 *stage = stage_all[warp];
+  uint8_t *rev = rev_all[warp];
+  int i = c.y - 1, j = c.w - 1, state = kCodeDiag, n = 0, status = 0;   // status: 1 done, 2 failed
+  for (;;) {
+    i = __shfl_sync(0xffffffffu, i, 0);
+    j = __shfl_sync(0xffffffffu, j, 0);
+    status = __shfl_sync(0xffffffffu, status, 0);
+    if (status) break;
+    const int r = i - 31 + lane;
+    stage[lane] = r >= 0 ? blk[size_t(r) * stride + (j >> 5)] : make_uint4(0u, 0u, 0u, 0u);
+    __syncwarp();
+    if (lane == 0) {
+      const int i0 = i - 31, cb = j >> 5;
+      const int shift = rem != 0 && cb == stride - 1 ? 32 - rem : 0;
+      const uint32_t *words = reinterpret_cast<const uint32_t *>(stage);
+      for (;;) {
+        if (i < 0 || j < 0) {
+          // only a diagonal step may leave the segments, and only from the reported start
+          status = state == kCodeDiag && n > 0 && rev[n - 1] == 0 && i + 1 == c.x && j + 1 == c.z ? 1 : 2;
+          break;
+        }
+        if (i < i0 || (j >> 5) != cb) break;
+        if (n == kMaxPath) {
+          status = 2;
+          break;
+        }
+        const int nib = (j & 31) + shift;
+        const uint32_t code = (words[(i - i0) * 4 + (nib >> 3)] >> ((nib & 7) * 4)) & 15u;
+        if (state == kCodeDiag) {
+          const uint32_t src = code & 3u;
+          if (src == kCodeZero) {
+            // H = 0 here: the diagonal step into the previous cell started the alignment
+            status = n > 0 && rev[n - 1] == 0 && i + 1 == c.x && j + 1 == c.z ? 1 : 2;
+            break;
+          }
+          if (src == kCodeDiag) {
+            rev[n++] = 0;
+            --i;
+            --j;
+          } else {
+            state = int(src);
+          }
+        } else if (state == kCodeE) {
+          rev[n++] = 2;
+          state = code & kCodeEOpen ? kCodeDiag : kCodeE;
+          --j;
+        } else {
+          rev[n++] = 1;
+          state = code & kCodeFOpen ? kCodeDiag : kCodeF;
+          --i;
+        }
+      }
+    }
+    __syncwarp();
+  }
+  n = __shfl_sync(0xffffffffu, n, 0);
+  uint8_t *dst = ops + op_off[p];
+  if (status == 1)
+    for (int k = lane; k < n; k += 32) dst[k] = rev[n - 1 - k];
+  if (lane == 0) out_len[p] = status == 1 ? n : -1;
+}
+
 }  // namespace align
 }  // namespace gfx
 
@@ -467,26 +645,45 @@ extern "C" size_t gfx_align_workspace_bytes(int64_t num_pairs, int64_t max_t_len
   return align::kHeaderBytes + align::parts_bytes(num_pairs) + size_t(align::grid_for(num_pairs)) * cols * 16;
 }
 
-extern "C" int gfx_align(const void *queries, int64_t q_rows, const void *targets, int64_t t_rows,
-                         const int64_t *pairs, int64_t num_pairs, float offset, float gap_open,
-                         float gap_extend, float *out_score, int32_t *out_coords, void *workspace,
-                         size_t workspace_bytes, void *stream) {
+extern "C" size_t gfx_align_trace_workspace_bytes(int64_t num_pairs, int64_t code_bytes) {
+  if (num_pairs < 0) num_pairs = 0;
+  if (code_bytes < 0) code_bytes = 0;
+  return align::trace_fixed_bytes(num_pairs) + size_t(code_bytes);
+}
+
+namespace {
+
+// gfx_align and gfx_align_trace: the same checks and launches; `trace` adds the pointer
+// blocks, the code pass and the walk.
+struct TraceOut {
+  uint8_t *ops;
+  const int64_t *op_offsets;
+  int32_t *len;
+};
+
+int run_align(const char *name, const void *queries, int64_t q_rows, const void *targets, int64_t t_rows,
+              const int64_t *pairs, int64_t num_pairs, float offset, float gap_open, float gap_extend,
+              float *out_score, int32_t *out_coords, const TraceOut *trace, void *workspace,
+              size_t workspace_bytes, void *stream) {
+  const std::string fn(name);
   if (num_pairs < 0 || q_rows < 0 || t_rows < 0 || q_rows > int64_t(INT_MAX) - 256 ||
       t_rows > int64_t(INT_MAX) - 256)
-    return fail(GFX_ERR_ARGUMENT, "gfx_align: bad sizes (table rows must fit int32)");
+    return fail(GFX_ERR_ARGUMENT, fn + ": bad sizes (table rows must fit int32)");
   if (!std::isfinite(offset) || !std::isfinite(gap_open) || !std::isfinite(gap_extend))
-    return fail(GFX_ERR_ARGUMENT, "gfx_align: offset, gap_open and gap_extend must be finite");
+    return fail(GFX_ERR_ARGUMENT, fn + ": offset, gap_open and gap_extend must be finite");
   if (!(gap_open > 0.f) || !(gap_extend > 0.f))
-    return fail(GFX_ERR_ARGUMENT, "gfx_align: gap_open and gap_extend must be positive");
+    return fail(GFX_ERR_ARGUMENT, fn + ": gap_open and gap_extend must be positive");
   if (num_pairs == 0) return GFX_OK;
-  if (!pairs || !out_score || !out_coords || !workspace || (q_rows > 0 && !queries) || (t_rows > 0 && !targets))
-    return fail(GFX_ERR_ARGUMENT, "gfx_align: null pointer");
+  if (!pairs || !out_score || !out_coords || !workspace || (q_rows > 0 && !queries) || (t_rows > 0 && !targets) ||
+      (trace && (!trace->ops || !trace->op_offsets || !trace->len)))
+    return fail(GFX_ERR_ARGUMENT, fn + ": null pointer");
   if ((reinterpret_cast<uintptr_t>(queries) | reinterpret_cast<uintptr_t>(targets) |
        reinterpret_cast<uintptr_t>(out_coords) | reinterpret_cast<uintptr_t>(workspace)) & 15)
-    return fail(GFX_ERR_ARGUMENT, "gfx_align: tables, out_coords and workspace must be 16-byte aligned");
+    return fail(GFX_ERR_ARGUMENT, fn + ": tables, out_coords and workspace must be 16-byte aligned");
   const int grid = align::grid_for(num_pairs);
-  const size_t fixed = align::kHeaderBytes + align::parts_bytes(num_pairs);
-  if (workspace_bytes < fixed) return fail(GFX_ERR_WORKSPACE, "gfx_align: workspace too small");
+  const size_t fixed = trace ? align::trace_fixed_bytes(num_pairs)
+                             : align::kHeaderBytes + align::parts_bytes(num_pairs);
+  if (workspace_bytes < fixed) return fail(GFX_ERR_WORKSPACE, fn + ": workspace too small");
   int64_t row_cap = int64_t((workspace_bytes - fixed) / (size_t(grid) * 16));
   row_cap = row_cap > align::kMaxLen ? align::kMaxLen : row_cap / align::kTile * align::kTile;
   cudaStream_t st = as_stream(stream);
@@ -503,20 +700,63 @@ extern "C" int gfx_align(const void *queries, int64_t q_rows, const void *target
   a.parts = reinterpret_cast<float4 *>(ws + align::kHeaderBytes);
   a.rowbuf = reinterpret_cast<float4 *>(ws + fixed);
   a.row_cap = int(row_cap);
+  if (trace) {
+    // offsets, then per-CTA rows of kMaxLen columns, then the pointer blocks
+    const size_t off_at = align::kHeaderBytes + align::parts_bytes(num_pairs);
+    a.code_off = reinterpret_cast<const int64_t *>(ws + off_at);
+    a.rowbuf = reinterpret_cast<float4 *>(ws + off_at + align256(size_t(num_pairs) * 8));
+    a.row_cap = align::kMaxLen;
+    a.codes = reinterpret_cast<uint8_t *>(ws + fixed);
+  }
   // An empty table is described as one row of the workspace; no pair can read it
   // (a segment inside it has length 0).
   align::Maps maps;
   int rc = tma::make_rows128_map(&maps.q, q_rows ? queries : workspace, q_rows ? q_rows : 1, 128);
   if (!rc) rc = tma::make_rows128_map(&maps.t, t_rows ? targets : workspace, t_rows ? t_rows : 1, 128);
   if (rc) return rc;
-  StageScope scope(GFX_STAGE_ALIGN, st, 2);
+  StageScope scope(GFX_STAGE_ALIGN, st, trace ? 4 : 2);
   GFX_CUDA(cudaMemsetAsync(ws, 0, align::kHeaderBytes, st));
-  GFX_CUDA(cudaFuncSetAttribute(align::align_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                align::Smem::total));
-  align::align_kernel<<<grid, align::kThreads, align::Smem::total, st>>>(maps, a);
+  if (trace) {
+    align::align_code_offsets_kernel<<<1, 1024, 0, st>>>(a, int64_t(workspace_bytes - fixed));
+    GFX_LAUNCH_CHECK();
+    GFX_CUDA(cudaFuncSetAttribute(align::align_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                  align::Smem::total));
+    align::align_kernel<true><<<grid, align::kThreads, align::Smem::total, st>>>(maps, a);
+  } else {
+    GFX_CUDA(cudaFuncSetAttribute(align::align_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                  align::Smem::total));
+    align::align_kernel<false><<<grid, align::kThreads, align::Smem::total, st>>>(maps, a);
+  }
   GFX_LAUNCH_CHECK();
   align::align_finish_kernel<<<int((num_pairs + 255) / 256), 256, 0, st>>>(
       a.parts, num_pairs, out_score, reinterpret_cast<int4 *>(out_coords));
   GFX_LAUNCH_CHECK();
+  if (trace) {
+    align::align_walk_kernel<<<int((num_pairs + align::kWalkWarps - 1) / align::kWalkWarps),
+                               align::kWalkWarps * 32, 0, st>>>(
+        pairs, num_pairs, a.code_off, a.codes, out_score, reinterpret_cast<const int4 *>(out_coords),
+        trace->op_offsets, trace->ops, trace->len);
+    GFX_LAUNCH_CHECK();
+  }
   return GFX_OK;
+}
+
+}  // namespace
+
+extern "C" int gfx_align(const void *queries, int64_t q_rows, const void *targets, int64_t t_rows,
+                         const int64_t *pairs, int64_t num_pairs, float offset, float gap_open,
+                         float gap_extend, float *out_score, int32_t *out_coords, void *workspace,
+                         size_t workspace_bytes, void *stream) {
+  return run_align("gfx_align", queries, q_rows, targets, t_rows, pairs, num_pairs, offset, gap_open,
+                   gap_extend, out_score, out_coords, nullptr, workspace, workspace_bytes, stream);
+}
+
+extern "C" int gfx_align_trace(const void *queries, int64_t q_rows, const void *targets, int64_t t_rows,
+                               const int64_t *pairs, int64_t num_pairs, float offset, float gap_open,
+                               float gap_extend, float *out_score, int32_t *out_coords, uint8_t *out_ops,
+                               const int64_t *op_offsets, int32_t *out_len, void *workspace,
+                               size_t workspace_bytes, void *stream) {
+  const TraceOut trace{out_ops, op_offsets, out_len};
+  return run_align("gfx_align_trace", queries, q_rows, targets, t_rows, pairs, num_pairs, offset, gap_open,
+                   gap_extend, out_score, out_coords, &trace, workspace, workspace_bytes, stream);
 }

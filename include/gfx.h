@@ -445,6 +445,41 @@ int gfx_align(const void *queries, int64_t q_rows, const void *targets,
               int32_t *out_coords, void *workspace, size_t workspace_bytes,
               void *stream);
 
+/* Traceback: gfx_align plus the aligned path of each pair.  Arguments,
+ * argument errors and out_score / out_coords are those of gfx_align (the
+ * messages name gfx_align_trace).
+ * Ops, one byte per step in forward order (query_begin -> query_end):
+ *   0 = M  query row i aligned with target row j (a diagonal step)
+ *   1 = I  a query row against a gap (an F step, gap in the target)
+ *   2 = D  a target row against a gap (an E step, gap in the query)
+ * The path is the one the tie rules above define: from the end cell back,
+ * H takes the first of diagonal, E, F that attains it, E and F prefer
+ * opening to extending, and a diagonal step from H = 0 is the start.  It
+ * starts and ends with M; #M + #I = query_end - query_begin and #M + #D =
+ * target_end - target_begin, so it has at most (q_len + t_len - 1) ops.  A
+ * pair with score 0 (or NaN) has an empty path.  Rescoring the path in fp32
+ * reproduces the score bit for bit: v = 0 + s at the first M, then each M
+ * adds its s, a gap opening (after M or after the other gap kind) subtracts
+ * gap_open and an extension subtracts gap_extend.
+ * out_ops uint8: pair p's path goes to out_ops[op_offsets[p] ...], a slot
+ * the caller sizes to at least q_len + t_len - 1 bytes; op_offsets int64
+ * [P]; out_len int32 [P] its length, or -1 if the walk did not end at the
+ * reported start (a library bug; the path is then not written).
+ * Workspace: gfx_align_trace_workspace_bytes(P, code_bytes), where
+ * code_bytes >= sum over the pairs of q_len * ceil(t_len / 32) * 16 (4 bits
+ * per cell of the DP's pointer record).  The per-CTA rows take every target
+ * length, so no other property of the pairs enters the size.  Pointer
+ * blocks are laid out in pair order; a pair whose block does not fit in the
+ * workspace gets score NaN, like a pair outside the limits.
+ * ------------------------------------------------------------------------ */
+size_t gfx_align_trace_workspace_bytes(int64_t num_pairs, int64_t code_bytes);
+int gfx_align_trace(const void *queries, int64_t q_rows, const void *targets,
+                    int64_t t_rows, const int64_t *pairs, int64_t num_pairs,
+                    float offset, float gap_open, float gap_extend,
+                    float *out_score, int32_t *out_coords, uint8_t *out_ops,
+                    const int64_t *op_offsets, int32_t *out_len,
+                    void *workspace, size_t workspace_bytes, void *stream);
+
 /* ------------------------------------------------------------------------
  * Instrumentation (used by bench.py; no effect on results).
  * Every kernel launch made by this library is counted per stage.  When a
